@@ -15,6 +15,7 @@ One "step" = one wifi_b200_rx_batch_dev pass over the whole resident capture (al
 gr-ieee802-11 flowgraph cannot be built here) on a bounded sample with all host threads.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -68,7 +69,41 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--viterbi-form", type=int, default=0, help="pin the Viterbi kernel form of the main handle (WIFI_P_VITERBI_FORM: 1 warp, 2 four lanes, 3 thread per trellis; 0 = by frame count)")
     ap.add_argument("--cpu-frames", type=int, default=8192, help="frames of the cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (frame table, "
+                    "decoded PSDU bytes; a fixed, seeded sample beyond %d frames / %d PSDUs) as DIR/<name>.npy in float64 / float32; "
+                    "rank 0 only" % (DUMP_FRAMES, DUMP_PSDUS))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_FRAMES, DUMP_PSDUS, PSDU_MAX = 65536, 8192, 1528     # PSDU_MAX: the largest PSDU the receiver decodes
+# --dump-outputs writes at most 65536 x 20 x 8 B (frame table) + 8192 x 1528 x 4 B (PSDU bytes) + 8192 x 8 B = 61 MB
+
+
+def dump_outputs(path, frames, psdu):
+    """--dump-outputs: the results of the last timed step as a caller receives them -- every field of the frame table and
+    the decoded PSDU bytes -- so that two builds can be compared output for output on the same inputs.  Integer and float
+    fields go out as float64 (exact), bytes as float32 with -1 where a frame has no decoded byte.  Beyond DUMP_FRAMES frames
+    the table is a sample drawn with a fixed seed (frame_index.npy says which rows), and the PSDU bytes are those of at
+    most DUMP_PSDUS of its rows (psdu_index.npy)."""
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(0)
+    n = len(frames)
+    rows = np.arange(n) if n <= DUMP_FRAMES else np.sort(rng.choice(n, DUMP_FRAMES, replace=False))
+    sel = rows if len(rows) <= DUMP_PSDUS else np.sort(rng.choice(rows, DUMP_PSDUS, replace=False))
+    out = {"frame_index": rows, "psdu_index": sel}
+    for k in frames.dtype.names:
+        out["frame_" + k] = frames[k][rows]
+    b = np.full((len(sel), PSDU_MAX), -1.0, np.float32)
+    for j, i in enumerate(sel):
+        p = psdu(int(i))
+        if p is not None:
+            b[j, :len(p)] = np.frombuffer(p, np.uint8)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v.astype(np.float64))
+    np.save(os.path.join(path, "psdu_bytes.npy"), b)
 
 
 def frame_samples():
@@ -242,6 +277,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", "-i", str(index), "--query-gpu=" + self.Q, "--format=csv,noheader,nounits", "-lms", "20"],
                                       stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)        # the sampler must not outlive bench.py, even when a section fails before stop()
         except Exception:
             self.p = None
 
@@ -348,6 +384,8 @@ def run_reference(args, out_fd):
         if it >= args.warmup:
             times.append(dt)
             ok = int(r.frames["crc_ok"].sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r.frames, r.psdu)
     t = float(np.sum(times))
     msps = x.size * len(times) / t / 1e6
     cfg = config_dict(args, n_links, fpl)
@@ -451,6 +489,8 @@ def main():
     sent = {p[:-4] for p in psdus}
     pd = res.pdus()
     assert all(p in sent for p in pd[:2000]), "decoded PDU not among the transmitted ones"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res.frames, res.psdu)
     tvec = torch.tensor([elapsed], dtype=torch.float64, device="cuda")
     cnt = torch.tensor([n_samples, st_frames, st_ok, st_ok * (PSDU_LEN - 4)], dtype=torch.int64, device="cuda")
     if world > 1:
@@ -747,4 +787,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the tree it runs from may be read-only: no __pycache__ beside the sources
     main()
