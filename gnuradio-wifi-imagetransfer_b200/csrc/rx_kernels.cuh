@@ -993,11 +993,14 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
 }
 
 // ------------------------------------------------------------------ R5f SIGNAL field
-// One thread per frame: deinterleave 48 hard bits, 62-step Viterbi (ntb 5), parse_signal.
+// One thread per frame: deinterleave 48 hard bits, 62-step Viterbi (ntb 5) on VitCoreH, parse_signal.
 __global__ void __launch_bounds__(VIT_BLOCK) k_signal(wifi_b200_frame *frames, int f0, int n_frames, const EqState *states)
 {
     __shared__ uint32_t ring[5 * 16 * VIT_BLOCK];
+    __shared__ uint4 s_bm[8 * 4 * 16];
     const int tid = threadIdx.x;
+    for (int i = tid; i < 512; i += VIT_BLOCK) s_bm[i] = VitCoreH::table_entry(i >> 6, (i >> 4) & 3, (uint32_t)(i & 15));
+    __syncthreads();
     int f = f0 + blockIdx.x * VIT_BLOCK + tid;
     if (f >= n_frames) return;
     if (frames[f].n_syms < 3) return;
@@ -1010,20 +1013,28 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_signal(wifi_b200_frame *frames, i
         uint64_t nib = s0 | (s1 << 2);
         if (tstep < 16) lo |= nib << (4 * tstep); else hi |= nib << (4 * (tstep - 16));
     }
-    VitCore v;
+    // k_viterbi's decoder, chunk for chunk; (lo, hi) is a 128-bit shift register of nibbles, zeros after step 24.
+    // Chunk 0 has 6 steps: two erased steps in front of them leave the all-zero metrics as they are and set bits 0, 1
+    // of every path byte, which trace_begin masks off (keep = 0xfc)
+    VitCoreH v;
     v.init();
+    const uint32_t first = (uint32_t)lo;
+    v.step4<0>(s_bm, 0xau, 0xau, first & 0xfu, (first >> 4) & 0xfu);
+    v.step4<4>(s_bm, (first >> 8) & 0xfu, (first >> 12) & 0xfu, (first >> 16) & 0xfu, (first >> 20) & 0xfu);
+    v.trace_begin(ring, 1, 5, tid, true, 0xfcu);
     uint32_t dec = 0;   // decoded bit i at bit i
-    int step = 0;
-    for (int chunk = 0; chunk < 8; ++chunk) {
-        int ns = chunk == 0 ? 6 : 8;
-        for (int k = 0; k < ns; ++k, ++step) {
-            uint32_t nib = step < 16 ? (uint32_t)(lo >> (4 * step)) & 0xfu : (step < 24 ? (uint32_t)(hi >> (4 * (step - 16))) & 0xfu : 0u);
-            v.step(nib);
-        }
-        uint32_t c = v.end_chunk(ring, (chunk + 1) % 5, 5, tid);
+#pragma unroll 1
+    for (int chunk = 1; chunk < 8; ++chunk) {
+        const uint32_t bits = (uint32_t)(lo >> 24);   // steps 8 * chunk - 2 .. 8 * chunk + 5
+        lo = (lo >> 32) | (hi << 32);
+        hi >>= 32;
+        v.step4<0>(s_bm, bits & 0xfu, (bits >> 4) & 0xfu, (bits >> 8) & 0xfu, (bits >> 12) & 0xfu);
+        v.step4<4>(s_bm, (bits >> 16) & 0xfu, (bits >> 20) & 0xfu, (bits >> 24) & 0xfu, bits >> 28);
+        VitTrace tr = v.trace_begin(ring, (chunk + 1) % 5, 5, tid, (chunk & 3) == 0);
         if (chunk >= 5) {
-            int m = chunk - 5;
-            dec |= (__brev(c) >> 24) << (8 * m);
+            // the ring byte holds the decisions in ascending bit order, as dec does
+            VitCoreH::trace_hops<4>(tr, ring, 5, tid);
+            dec |= vit_ring_byte(ring, tr.sl, tr.bs, tid) << (8 * (chunk - 5));
         }
     }
     int r = 0, len = 0;
@@ -1282,7 +1293,7 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict
     sink.init(out, L, s_crc, s_scr);
     uint32_t next = 1 < nw ? in[1] : 0u;
     // software pipeline: the traceback of chunk j-1 runs interleaved with the trellis steps of chunk j
-    VitCore::Trace tr;
+    VitTrace tr;
     tr.bs = 0; tr.sl = slot; tr.left = 0;
     bool pending = false;
 #pragma unroll 1
@@ -1324,7 +1335,7 @@ __global__ void __launch_bounds__(VQ_BLOCK) k_viterbi_quad(const JobDesc *__rest
     const int tid = threadIdx.x;
     for (int i = tid; i < 256; i += VQ_BLOCK) s_crc[i] = c_tab.crc_tab[i];
     for (int i = tid; i < 128; i += VQ_BLOCK) s_scr[i] = c_tab.scr_tab[i];
-    if (tid < 16) { uint32_t T, E; VitCore::branch((uint32_t)tid, T, E); s_bm[tid] = make_uint2(T, E); }
+    if (tid < 16) { uint32_t T, E; VitQuad::branch((uint32_t)tid, T, E); s_bm[tid] = make_uint2(T, E); }
     __syncthreads();
     const int job = f0 + blockIdx.x * VQ_FRAMES + (tid >> 2);
     // the quads of a warp stay together (full-mask shuffles): a quad without a frame, or with a shorter one, runs along
@@ -1356,7 +1367,7 @@ __global__ void __launch_bounds__(VQ_BLOCK) k_viterbi_quad(const JobDesc *__rest
     sink.init(psdu + (int64_t)(active ? job : f0) * (PSDU_STRIDE / 4), L, s_crc, s_scr);
     sink.writer = active && (tid & 3) == 0;
     uint32_t next = 1 < nw ? in[1] : 0u;
-    VitCore::Trace tr;
+    VitTrace tr;
     tr.bs = 0; tr.sl = slot; tr.left = 0;
 #pragma unroll 1
     for (int chunk = 1; chunk <= trips; ++chunk) {
@@ -1538,16 +1549,17 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi_soft(const JobDesc *__res
     v.init();
     PsduSink sink;
     sink.init(psdu + (int64_t)job * (PSDU_STRIDE / 4), L, s_crc, s_scr);
-    int wi = 0;
-    auto two_steps = [&](uint32_t word) {
-        v.step((int)(int8_t)(word & 0xffu), (int)(int8_t)((word >> 8) & 0xffu));
-        v.step((int)(int8_t)((word >> 16) & 0xffu), (int)(int8_t)(word >> 24));
-    };
-#pragma unroll 1
-    for (int k = 0; k < 3; ++k, ++wi) two_steps(wi < nw ? in[wi] : 0u);
+    // chunk 0 has 6 steps: two erased steps (soft value 0: every branch metric 254, so every candidate ties) in front of
+    // them leave every metric equal and set bits 7, 6 of every path byte, which are masked off; the renormalisation
+    // removes the uniform +508
+    v.step4<0>(0u, 0 < nw ? in[0] : 0u);
+    v.step4<4>(1 < nw ? in[1] : 0u, 2 < nw ? in[2] : 0u);
+#pragma unroll
+    for (int i = 0; i < 32; ++i) v.P[i] &= 0x003f003fu;
     int slot = 1 % ntb;
-    v.end_chunk(ring, slot, ntb, tid, true);
-    VitCore::Trace tr;
+    v.trace_begin(ring, slot, ntb, tid, true);
+    int wi = 3;
+    VitTrace tr;
     tr.bs = 0; tr.sl = slot; tr.left = 0;
     bool pending = false;
 #pragma unroll 1
@@ -1556,19 +1568,19 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi_soft(const JobDesc *__res
 #pragma unroll
         for (int k = 0; k < 4; ++k) w4[k] = (wi + k < nw) ? in[wi + k] : 0u;
         wi += 4;
-        VitCore::trace_hops<3>(tr, ring, ntb, tid);
+        VitCoreSoft::trace_hops<3>(tr, ring, ntb, tid);
         v.step4<0>(w4[0], w4[1]);
-        VitCore::trace_hops<3>(tr, ring, ntb, tid);
+        VitCoreSoft::trace_hops<3>(tr, ring, ntb, tid);
         v.step4<4>(w4[2], w4[3]);
-        VitCore::trace_hops<3>(tr, ring, ntb, tid);
-        if (pending && chunk - 1 >= ntb) sink.push(VitCore::trace_finish(tr, ring, tid), chunk - 1 - ntb);
+        VitCoreSoft::trace_hops<3>(tr, ring, ntb, tid);
+        if (pending && chunk - 1 >= ntb) sink.push(vit_ring_byte(ring, tr.sl, tr.bs, tid), chunk - 1 - ntb);
         slot = (slot + 1 == ntb) ? 0 : slot + 1;
         tr = v.trace_begin(ring, slot, ntb, tid, (chunk & 1) == 0);
         pending = true;
     }
     if (pending && last_chunk >= ntb) {
-        VitCore::trace_hops<9>(tr, ring, ntb, tid);
-        sink.push(VitCore::trace_finish(tr, ring, tid), last_chunk - ntb);
+        VitCoreSoft::trace_hops<9>(tr, ring, ntb, tid);
+        sink.push(vit_ring_byte(ring, tr.sl, tr.bs, tid), last_chunk - ntb);
     }
     frames[J.frame].crc_ok = sink.crc_ok();
 }

@@ -1,20 +1,28 @@
-// viterbi.cuh -- K=7 (133,171) hard-decision Viterbi decoder.
+// viterbi.cuh -- K=7 (133,171) Viterbi decoders, hard and soft decision.
 //
 // Restates [UPSTREAM] gr-ieee802-11 lib/viterbi_decoder/{base,viterbi_decoder_generic}.cc
 // (instance wifi_phy_hier.grc:533-549 decode_mac, and :550-569 frame_equalizer for SIGNAL):
 // 8-bit agreement metrics, tie -> predecessor k+32, per-state 8-bit path registers, a
 // traceback over `ntb` stored path snapshots every 8 trellis steps (first after 6).
 //
-// Three forms of the same decoder, chosen by the number of frames in a call (wifi_b200.cu):
-//   VitCoreH  one trellis per THREAD (k_viterbi), metric and path byte of a state in one halfword, two states per
-//             register: the add-compare-select of four new states is two VIADDMNMX.U16x2 + two adds (round 2);
-//   VitQuad   one trellis per FOUR lanes (k_viterbi_quad), byte-packed metrics as VitCore, two quad exchanges per 4 steps;
+// Three forms of the hard-decision decoder, chosen by the number of frames in a call (wifi_b200.cu):
+//   VitCoreH  one trellis per THREAD (k_viterbi, and k_signal for the SIGNAL field), metric and path byte of a state in
+//             one halfword, two states per register: the add-compare-select of four new states is two VIADDMNMX.U16x2
+//             + two adds;
+//   VitQuad   one trellis per FOUR lanes (k_viterbi_quad), byte-packed metrics and path bytes (4 states per register),
+//             two quad exchanges per 4 steps;
 //   (k_viterbi_warp, rx_kernels.cuh: one trellis per warp.)
-// VitCore is the byte-packed per-thread form of round 1 -- 64 path metrics in 16 registers (4 states per register, one
-// byte each), 64 path bytes in 16 more; IADD for the candidate metrics, IADD3 + PRMT (sign-replicate) for the byte-wise
-// "m0 > m1" masks, LOP3 selects -- which k_signal and VitQuad still use.  Metrics never exceed 12 + 4 * 16 (spread
-// bound of the code + growth between renormalisations), so bytes cannot carry into each other.  Path snapshots go to
-// shared memory, word-interleaved across the block's threads (bank = thread id, conflict free).
+// VitCoreSoft is the soft-decision decoder (k_viterbi_soft): 16-bit metrics and path halfwords, two states per register.
+//
+// VitCoreH, VitQuad and VitCoreSoft run the trellis four steps at a time (step4) with one re-layout instead of four.
+// A butterfly leaves its survivors split into "new even states" and "new odd states" words; instead of interleaving
+// them back to natural order after every step, the next steps pair the split words directly -- the state stride inside
+// a word doubles each step: 1 (natural) -> 2 -> 4 -> 8 -> 16 -- and one transpose restores natural order after the
+// fourth step.  Chunks are 8 steps, so snapshots and the best-state search always see the natural layout.  The path
+// bytes are never shifted: step s of a chunk sets its own decision bit.  Chunk 0 has 6 steps; it runs as two erased
+// steps + 6, whose two extra decision bits are masked off before the snapshot (see the kernels).
+// Path snapshots of the per-thread forms go to shared memory, word-interleaved across the block's threads (bank =
+// thread id, conflict free).
 #pragma once
 #include "wifi_common.cuh"
 
@@ -28,31 +36,8 @@ __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
     return d;
 }
 
-// branch selector for butterfly word j: byte b <- T byte (2*A_k + B_k), k = 4j + b
+// parity of a 7-bit word; butterfly k's expected code bits are A = par(2k & 0x6d), B = par(2k & 0x4f)
 __host__ __device__ constexpr uint32_t vit_par(uint32_t v) { return (v ^ (v >> 1) ^ (v >> 2) ^ (v >> 3) ^ (v >> 4) ^ (v >> 5) ^ (v >> 6)) & 1u; }
-__host__ __device__ constexpr uint32_t vit_sel(int j)
-{
-    uint32_t s = 0;
-    for (int b = 0; b < 4; ++b) {
-        uint32_t k = 4 * j + b;
-        uint32_t A = vit_par((2 * k) & 0x6d), B = vit_par((2 * k) & 0x4f);
-        s |= (2 * A + B) << (4 * b);
-    }
-    return s;
-}
-
-// selector for a packed butterfly whose byte lanes hold butterflies k0..k3
-__host__ __device__ constexpr uint32_t vit_sel4(int k0, int k1, int k2, int k3)
-{
-    const int k[4] = {k0, k1, k2, k3};
-    uint32_t s = 0;
-    for (int b = 0; b < 4; ++b) {
-        uint32_t A = vit_par((2 * k[b]) & 0x6d), B = vit_par((2 * k[b]) & 0x4f);
-        s |= (2 * A + B) << (4 * b);
-    }
-    return s;
-}
-
 // selector picking, for two butterflies k0 (low halfword) and k1 (high), halfword (2A+B) of a (Tlo, Thi) register pair
 __host__ __device__ constexpr uint32_t vit_sel2(int k0, int k1)
 {
@@ -65,257 +50,20 @@ __host__ __device__ constexpr uint32_t vit_sel2(int k0, int k1)
     return s;
 }
 
-struct VitCore {
-    uint32_t M[16], P[16];
-
-    __device__ __forceinline__ void init()
-    {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) { M[i] = 0; P[i] = 0; }
-    }
-
-    // one trellis step; nib = s0 | s1 << 2 with s in {0,1,2 = erasure}
-    __device__ __forceinline__ void step(uint32_t nib)
-    {
-        const uint32_t s0 = nib & 3u, s1 = (nib >> 2) & 3u;
-        const uint32_t t0 = (s0 == 2u) ? 0u : (s0 ? 0x00000101u : 0x01010000u);
-        const uint32_t t1 = (s1 == 2u) ? 0u : (s1 ? 0x00010001u : 0x01000100u);
-        const uint32_t T = t0 + t1;                                     // disagreements per (A,B)
-        const uint32_t E = ((s0 != 2u) ? 0x01010101u : 0u) + ((s1 != 2u) ? 0x01010101u : 0u);
-        uint32_t Mn[16], Pn[16];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const uint32_t sel = vit_sel(j);
-            const uint32_t svm = prmt(T, 0u, sel), sv = E - svm;   // agreements = available symbols - disagreements
-            const uint32_t lo = M[j], hi = M[j + 8];
-            const uint32_t m0 = lo + sv, m1 = hi + svm, m2 = lo + svm, m3 = hi + sv;
-            const uint32_t k0 = prmt(m0 + 0x7f7f7f7fu - m1, 0u, 0xba98u); // 0xff where m0 > m1
-            const uint32_t k1 = prmt(m2 + 0x7f7f7f7fu - m3, 0u, 0xba98u);
-            const uint32_t v0 = (m0 & k0) | (m1 & ~k0);
-            const uint32_t v1 = (m2 & k1) | (m3 & ~k1);
-            const uint32_t sh0 = P[j] << 1, sh1 = (P[j + 8] << 1) | 0x01010101u;
-            const uint32_t q0 = (sh0 & k0) | (sh1 & ~k0);
-            const uint32_t q1 = (sh0 & k1) | (sh1 & ~k1);
-            Mn[2 * j] = prmt(v0, v1, 0x5140u);
-            Mn[2 * j + 1] = prmt(v0, v1, 0x7362u);
-            Pn[2 * j] = prmt(q0, q1, 0x5140u);
-            Pn[2 * j + 1] = prmt(q0, q1, 0x7362u);
-        }
-#pragma unroll
-        for (int i = 0; i < 16; ++i) { M[i] = Mn[i]; P[i] = Pn[i]; }
-    }
-
-    // per-step branch words: T = disagreements per (A,B) pattern, E = symbols present (not erased)
-    static __device__ __forceinline__ void branch(uint32_t nib, uint32_t &T, uint32_t &E)
-    {
-        const uint32_t s0 = nib & 3u, s1 = (nib >> 2) & 3u;
-        const uint32_t t0 = (s0 == 2u) ? 0u : (s0 ? 0x00000101u : 0x01010000u);
-        const uint32_t t1 = (s1 == 2u) ? 0u : (s1 ? 0x00010001u : 0x01000100u);
-        T = t0 + t1;
-        E = ((s0 != 2u) ? 0x01010101u : 0u) + ((s1 != 2u) ? 0x01010101u : 0u);
-    }
-    // four packed butterflies: lo = old states k_b, hi = old states k_b + 32 (same byte lanes);
-    // v0/q0 = survivors of new states 2k_b, v1/q1 of 2k_b + 1
-    // BIT: the decision bit of this step inside the path byte.  The bytes are never shifted: step s of a
-    // chunk ORs its decision in at bit 7 - s (earliest decision = MSB, as upstream's shift register leaves it).
-    template <uint32_t BIT>
-    static __device__ __forceinline__ void bfly(uint32_t T, uint32_t E, uint32_t sel, uint32_t lo, uint32_t hi, uint32_t plo, uint32_t phi,
-                                                uint32_t &v0, uint32_t &v1, uint32_t &q0, uint32_t &q1)
-    {
-        // the selectors of a step come in complementary pairs (pattern p <-> 3 - p, i.e. sel ^ 0x3333), and
-        // T[3 - p] = E - T[p]: one permute serves both, with the two branch words swapped
-        const uint32_t selc = sel < (sel ^ 0x3333u) ? sel : (sel ^ 0x3333u);
-        const uint32_t ta = prmt(T, 0u, selc), tb = E - ta;
-        const uint32_t svm = (sel == selc) ? ta : tb, sv = (sel == selc) ? tb : ta;
-        const uint32_t m0 = lo + sv, m1 = hi + svm, m2 = lo + svm, m3 = hi + sv;
-        const uint32_t k0 = prmt(m0 + 0x7f7f7f7fu - m1, 0u, 0xba98u);
-        const uint32_t k1 = prmt(m2 + 0x7f7f7f7fu - m3, 0u, 0xba98u);
-        v0 = (m0 & k0) | (m1 & ~k0);
-        v1 = (m2 & k1) | (m3 & ~k1);
-        const uint32_t pb = phi + BIT;
-        q0 = (plo & k0) | (pb & ~k0);
-        q1 = (plo & k1) | (pb & ~k1);
-    }
-    // Four trellis steps with one re-layout instead of four.  A butterfly leaves its survivors split
-    // into "new even states" and "new odd states" words; instead of interleaving them back to natural
-    // order after every step (4 PRMT per word pair), the next steps pair the split words directly --
-    // the state stride inside a word doubles each step: 1 (natural) -> 2 -> 4 -> 8 -> 16 -- and one 4x4
-    // byte transpose per four words (2 PRMT per word) restores natural order after the fourth step.
-    // Chunks are 8 steps, so snapshots and the best-state search always see the natural layout.
-    // bm: 16-entry shared-memory table of branch() results indexed by the 4-bit symbol pair
-    // S0: index of the first of the four steps inside its 8-step chunk (0 or 4)
-    template <int S0>
-    __device__ __forceinline__ void step4(const uint2 *bm, uint32_t n0, uint32_t n1, uint32_t n2, uint32_t n3)
-    {
-        constexpr uint32_t B0 = 0x01010101u << (7 - S0), B1 = B0 >> 1, B2 = B0 >> 2, B3 = B0 >> 3;
-        uint32_t T, E;
-        uint32_t S[16], SP[16], Q[16], QP[16];
-        // A: natural.  pair j: k = 4j + b  ->  S[j] = states 8j + 2b (even), S[8 + j] = 8j + 2b + 1 (odd)
-        { const uint2 te = bm[n0]; T = te.x; E = te.y; }
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-            bfly<B0>(T, E, vit_sel4(4 * j, 4 * j + 1, 4 * j + 2, 4 * j + 3), M[j], M[j + 8], P[j], P[j + 8], S[j], S[8 + j], SP[j], SP[8 + j]);
-        // B: stride 2.  even pair j: k = 8j + 2b, odd pair j: k = 8j + 2b + 1  ->  Q[4j + o] = states 16j + 4b + o
-        { const uint2 te = bm[n1]; T = te.x; E = te.y; }
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            bfly<B1>(T, E, vit_sel4(8 * j, 8 * j + 2, 8 * j + 4, 8 * j + 6), S[j], S[j + 4], SP[j], SP[j + 4], Q[4 * j], Q[4 * j + 1], QP[4 * j], QP[4 * j + 1]);
-            bfly<B1>(T, E, vit_sel4(8 * j + 1, 8 * j + 3, 8 * j + 5, 8 * j + 7), S[8 + j], S[12 + j], SP[8 + j], SP[12 + j], Q[4 * j + 2], Q[4 * j + 3],
-                 QP[4 * j + 2], QP[4 * j + 3]);
-        }
-        // C: stride 4.  pair (j, o): k = 16j + 4b + o  ->  S[8j + o'] = states 32j + 8b + o', o' = 2o, 2o + 1
-        { const uint2 te = bm[n2]; T = te.x; E = te.y; }
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int o = 0; o < 4; ++o)
-                bfly<B2>(T, E, vit_sel4(16 * j + o, 16 * j + 4 + o, 16 * j + 8 + o, 16 * j + 12 + o), Q[4 * j + o], Q[4 * (j + 2) + o], QP[4 * j + o],
-                     QP[4 * (j + 2) + o], S[8 * j + 2 * o], S[8 * j + 2 * o + 1], SP[8 * j + 2 * o], SP[8 * j + 2 * o + 1]);
-        // D: stride 8.  pair o': k = 8b + o'  ->  Q[o''] = states 16b + o'', o'' = 2o', 2o' + 1
-        { const uint2 te = bm[n3]; T = te.x; E = te.y; }
-#pragma unroll
-        for (int o = 0; o < 8; ++o)
-            bfly<B3>(T, E, vit_sel4(o, 8 + o, 16 + o, 24 + o), S[o], S[8 + o], SP[o], SP[8 + o], Q[2 * o], Q[2 * o + 1], QP[2 * o], QP[2 * o + 1]);
-        // stride 16 -> natural: natural word w, byte i = Q[4 (w % 4) + i] byte (w / 4)
-#pragma unroll
-        for (int g = 0; g < 4; ++g) {
-            uint32_t t0 = prmt(Q[4 * g], Q[4 * g + 1], 0x5140u), t1 = prmt(Q[4 * g], Q[4 * g + 1], 0x7362u);
-            uint32_t t2 = prmt(Q[4 * g + 2], Q[4 * g + 3], 0x5140u), t3 = prmt(Q[4 * g + 2], Q[4 * g + 3], 0x7362u);
-            M[g] = prmt(t0, t2, 0x5410u); M[g + 4] = prmt(t0, t2, 0x7632u); M[g + 8] = prmt(t1, t3, 0x5410u); M[g + 12] = prmt(t1, t3, 0x7632u);
-            t0 = prmt(QP[4 * g], QP[4 * g + 1], 0x5140u); t1 = prmt(QP[4 * g], QP[4 * g + 1], 0x7362u);
-            t2 = prmt(QP[4 * g + 2], QP[4 * g + 3], 0x5140u); t3 = prmt(QP[4 * g + 2], QP[4 * g + 3], 0x7362u);
-            P[g] = prmt(t0, t2, 0x5410u); P[g + 4] = prmt(t0, t2, 0x7632u); P[g + 8] = prmt(t1, t3, 0x5410u); P[g + 12] = prmt(t1, t3, 0x7632u);
-        }
-    }
-
-    // byte-wise unsigned max / min of packed words (bytes < 0x80)
-    static __device__ __forceinline__ uint32_t vmax4(uint32_t a, uint32_t b)
-    {
-        uint32_t k = prmt((a | 0x80808080u) - b, 0u, 0xba98u); // 0xff where a >= b
-        return (a & k) | (b & ~k);
-    }
-    static __device__ __forceinline__ uint32_t vmin4(uint32_t a, uint32_t b)
-    {
-        uint32_t k = prmt((a | 0x80808080u) - b, 0u, 0xba98u);
-        return (b & k) | (a & ~k);
-    }
-
-    // The traceback of one chunk is a chain of dependent shared-memory reads.  trace_begin() stores the
-    // snapshot and finds the first best state; trace_hops() advances a few hops (branch-free, so the
-    // scheduler can interleave the chain with the next chunk's add-compare-select work);
-    // trace_finish() reads the output byte.  It must run before the next snapshot is stored (the byte
-    // it reads lives in the slot that snapshot overwrites).
-    struct Trace { int bs, sl, left; };
-    __device__ __forceinline__ Trace trace_begin(uint32_t *ring, int slot, int ntb, int tid, bool renorm)
-    {
-#pragma unroll
-        for (int w = 0; w < 16; ++w) ring[(slot * 16 + w) * VIT_BLOCK + tid] = P[w];
-        // first best state from 16-bit keys (metric << 8) | (63 - state): the largest key is the largest
-        // metric at the smallest state; two keys per word, reduced with the packed-halfword maximum
-        // (VIMNMX.U16x2 / VIMNMX3 on sm_100a)
-        uint32_t key[32];
-#pragma unroll
-        for (int w = 0; w < 16; ++w) {
-            const uint32_t c = (uint32_t)(63 - 4 * w) | ((uint32_t)(62 - 4 * w) << 8) | ((uint32_t)(61 - 4 * w) << 16) | ((uint32_t)(60 - 4 * w) << 24);
-            key[2 * w] = prmt(M[w], c, 0x1504u);
-            key[2 * w + 1] = prmt(M[w], c, 0x3726u);
-        }
-#pragma unroll
-        for (int n = 16; n >= 1; n >>= 1)
-#pragma unroll
-            for (int i = 0; i < n; ++i) key[i] = __vmaxu2(key[i], key[i + n]);
-        const uint32_t kbest = max(key[0] & 0xffffu, key[0] >> 16);
-        Trace t;
-        t.bs = 63 - (int)(kbest & 0xffu);
-        t.sl = slot;
-        t.left = ntb - 1;
-        if (renorm) {
-            // Only metric differences matter (upstream subtracts the minimum after every chunk).  Any state
-            // is reached from any other in K - 1 = 6 steps of at most 2 agreements each, so min >= max - 12:
-            // subtracting max - 12 keeps every byte non-negative without a search for the minimum.
-            const uint32_t mx = kbest >> 8;
-            const uint32_t minw = (mx > 12u ? mx - 12u : 0u) * 0x01010101u;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) M[i] -= minw;
-        }
-#pragma unroll
-        for (int i = 0; i < 16; ++i) P[i] = 0;
-        return t;
-    }
-    // byte (slot, state) of this thread's ring: the ring is word-interleaved across the block's threads,
-    // word (slot * 16 + state / 4) * VIT_BLOCK + tid, so the path byte is a single byte load
-    static __device__ __forceinline__ uint32_t ring_byte(const uint32_t *ring, int sl, int bs, int tid)
-    {
-        const uint8_t *rb = reinterpret_cast<const uint8_t *>(ring) + tid * 4;
-        return rb[sl * (16 * VIT_BLOCK * 4) + (bs >> 2) * (VIT_BLOCK * 4) + (bs & 3)];
-    }
-    template <int N>
-    static __device__ __forceinline__ void trace_hops(Trace &t, const uint32_t *ring, int ntb, int tid)
-    {
-#pragma unroll
-        for (int i = 0; i < N; ++i) {
-            // Branch-free on purpose: the chain of dependent loads interleaves with the add-compare-select
-            // work.  (Measured: a variant without the three selects, for warps whose frames all trace back
-            // nine snapshots, is slower -- the kernel is bound by its schedule, not by these few ops.)
-            const bool go = t.left > 0;
-            const int nb = (int)(ring_byte(ring, t.sl, t.bs, tid) >> 2);
-            const int ns = (t.sl == 0) ? ntb - 1 : t.sl - 1;
-            t.bs = go ? nb : t.bs;
-            t.sl = go ? ns : t.sl;
-            t.left -= go ? 1 : 0;
-        }
-    }
-    static __device__ __forceinline__ uint32_t trace_finish(const Trace &t, const uint32_t *ring, int tid)
-    {
-        return ring_byte(ring, t.sl, t.bs, tid);
-    }
-
-    // viterbi_get_output_generic: snapshot the paths into ring slot `slot`, find the first
-    // best state, trace back ntb-1 snapshots, return that snapshot's path byte, renormalise
-    // the metrics by their minimum and clear the path registers.
-    __device__ __forceinline__ uint32_t end_chunk(uint32_t *ring, int slot, int ntb, int tid, bool renorm = true)
-    {
-#pragma unroll
-        for (int w = 0; w < 16; ++w) ring[(slot * 16 + w) * VIT_BLOCK + tid] = P[w];
-        uint32_t mx = M[0];
-#pragma unroll
-        for (int w = 1; w < 16; ++w) mx = vmax4(mx, M[w]);
-        mx = vmax4(mx, mx >> 16); mx = vmax4(mx, mx >> 8);
-        const uint32_t bestw = (mx & 0xffu) * 0x01010101u;
-        // first state whose metric equals the maximum
-        int wsel = 0;
-        uint32_t zsel = 0;
-#pragma unroll
-        for (int w = 15; w >= 0; --w) {
-            uint32_t x = M[w] ^ bestw;
-            uint32_t z = ((x + 0x7f7f7f7fu) & 0x80808080u) ^ 0x80808080u; // bit7 set where equal
-            if (z) { wsel = w; zsel = z; }
-        }
-        int bs = wsel * 4 + ((__ffs((int)zsel) - 8) >> 3);
-        int sl = slot;
-        for (int i = 0; i < ntb - 1; ++i) {
-            uint32_t w = ring[(sl * 16 + (bs >> 2)) * VIT_BLOCK + tid];
-            bs = (int)((w >> (8 * (bs & 3))) & 0xffu) >> 2;
-            sl = (sl == 0) ? ntb - 1 : sl - 1;
-        }
-        uint32_t w = ring[(sl * 16 + (bs >> 2)) * VIT_BLOCK + tid];
-        uint32_t c = (w >> (8 * (bs & 3))) & 0xffu;
-        // upstream subtracts the minimum after every chunk; only metric differences matter, so the
-        // subtraction may be skipped as long as bytes stay below 0x80 (spread <= 12, +16 per chunk)
-        if (renorm) {
-            uint32_t mn = M[0];
-#pragma unroll
-            for (int w = 1; w < 16; ++w) mn = vmin4(mn, M[w]);
-            mn = vmin4(mn, mn >> 16); mn = vmin4(mn, mn >> 8);
-            const uint32_t minw = (mn & 0xffu) * 0x01010101u;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) M[i] -= minw;
-        }
-#pragma unroll
-        for (int i = 0; i < 16; ++i) P[i] = 0;
-        return c;
-    }
-};
+// The traceback of one chunk is a chain of dependent shared-memory reads.  trace_begin() stores the snapshot and finds
+// the first best state; trace_hops() advances a few hops (branch-free, so the scheduler can interleave the chain with
+// the next chunk's add-compare-select work; measured: a variant without the three selects, for warps whose frames all
+// trace back nine snapshots, is slower -- the kernel is bound by its schedule, not by these few ops); then the output
+// byte is read.  That read must come before the next snapshot is stored: the byte lives in the slot it overwrites.
+// VitTrace is the cursor: state, ring slot, hops left.
+struct VitTrace { int bs, sl, left; };
+// byte (slot, state) of this thread's ring: the ring is word-interleaved across the block's threads,
+// word (slot * 16 + state / 4) * VIT_BLOCK + tid, so the path byte is a single byte load
+__device__ __forceinline__ uint32_t vit_ring_byte(const uint32_t *ring, int sl, int bs, int tid)
+{
+    const uint8_t *rb = reinterpret_cast<const uint8_t *>(ring) + tid * 4;
+    return rb[sl * (16 * VIT_BLOCK * 4) + (bs >> 2) * (VIT_BLOCK * 4) + (bs & 3)];
+}
 
 // ---------------------------------------------------------------------------------------------------------------
 // VitCoreH: the per-thread decoder with metric and path byte of a state in ONE halfword, two states per register:
@@ -325,7 +73,8 @@ struct VitCore {
 // compare, upstream's tie rule (-> k + 32) and the selection of metric and path together -- VIADDMNMX.U16x2 even adds
 // one candidate's branch metric on the way.  An add-compare-select of two butterflies (four new states) is two
 // alu-pipe instructions + two adds (which ptxas places on the fma pipe), against 8.5 + 5 for four butterflies in the
-// byte-packed form (compare word, sign-replicating permute, two selects per output word).  Same 32 registers of state.
+// byte-packed form of VitQuad::bfly (compare word, sign-replicating permute, two selects per output word), for the
+// same 32 registers of state a whole trellis takes in bytes (16 metric words + 16 path words).
 // Path bytes are therefore bit-reversed with respect to upstream's shift register (decision of step s at bit 7 - s):
 // the traceback reverses the byte it follows (one BREV per hop), and the output byte is reversed once.
 // Metrics stay below 12 + 4 * 16 = 76 between renormalisations (every fourth chunk), so 8 bits hold them.
@@ -421,10 +170,10 @@ struct VitCoreH {
                 X[(32 * j + 16 + e2) >> 1] = prmt(Q[16 * j + e2], Q[16 * j + e2 + 1], 0x7632u);
             }
     }
-    // end of a chunk: snapshot the path bytes (ring slot `slot`, byte = state, as VitCore's ring), first best state,
-    // optional renormalisation, path bytes cleared.  keep: mask applied to the path bytes first (0xff; 0xfc after the
-    // 6-step first chunk, which runs as two erased steps + 6).
-    __device__ __forceinline__ VitCore::Trace trace_begin(uint32_t *ring, int slot, int ntb, int tid, bool renorm, uint32_t keep = 0xffu)
+    // end of a chunk: snapshot the path bytes (ring slot `slot`, one byte per state, see vit_ring_byte), first best
+    // state, optional renormalisation, path bytes cleared.  keep: mask applied to the path bytes first (0xff; 0xfc after
+    // the 6-step first chunk, which runs as two erased steps + 6).
+    __device__ __forceinline__ VitTrace trace_begin(uint32_t *ring, int slot, int ntb, int tid, bool renorm, uint32_t keep = 0xffu)
     {
         const uint32_t keepw = 0xff00ff00u | keep | (keep << 16);
 #pragma unroll
@@ -442,11 +191,14 @@ struct VitCoreH {
 #pragma unroll
             for (int i = 0; i < n; ++i) key[i] = __vmaxu2(key[i], key[i + n]);
         const uint32_t kbest = max(key[0] & 0xffffu, key[0] >> 16);
-        VitCore::Trace t;
+        VitTrace t;
         t.bs = 63 - (int)(kbest & 0xffu);
         t.sl = slot;
         t.left = ntb - 1;
         if (renorm) {
+            // Only metric differences matter (upstream subtracts the minimum after every chunk).  Any state is reached
+            // from any other in K - 1 = 6 steps of at most 2 agreements each, so min >= max - 12: subtracting max - 12
+            // keeps every metric non-negative without a search for the minimum.
             const uint32_t mx = kbest >> 8;
             const uint32_t nminw = 0u - (mx > 12u ? ((mx - 12u) << 8) * 0x00010001u : 0u);
 #pragma unroll
@@ -456,12 +208,12 @@ struct VitCoreH {
     }
     // ring bytes hold the decisions in ascending bit order: the state eight steps back is the byte reversed, >> 2
     template <int N>
-    static __device__ __forceinline__ void trace_hops(VitCore::Trace &t, const uint32_t *ring, int ntb, int tid)
+    static __device__ __forceinline__ void trace_hops(VitTrace &t, const uint32_t *ring, int ntb, int tid)
     {
 #pragma unroll
         for (int i = 0; i < N; ++i) {
             const bool go = t.left > 0;
-            const int nb = (int)(__brev(VitCore::ring_byte(ring, t.sl, t.bs, tid)) >> 26);
+            const int nb = (int)(__brev(vit_ring_byte(ring, t.sl, t.bs, tid)) >> 26);
             const int ns = (t.sl == 0) ? ntb - 1 : t.sl - 1;
             t.bs = go ? nb : t.bs;
             t.sl = go ? ns : t.sl;
@@ -469,26 +221,38 @@ struct VitCoreH {
         }
     }
     // the chunk's output byte in upstream's bit order (MSB = earliest decision)
-    static __device__ __forceinline__ uint32_t trace_finish(const VitCore::Trace &t, const uint32_t *ring, int tid)
+    static __device__ __forceinline__ uint32_t trace_finish(const VitTrace &t, const uint32_t *ring, int tid)
     {
-        return __brev(VitCore::ring_byte(ring, t.sl, t.bs, tid)) >> 24;
+        return __brev(vit_ring_byte(ring, t.sl, t.bs, tid)) >> 24;
     }
 };
 
 // ---------------------------------------------------------------------------------------------------------------
 // The same decoder with one trellis spread over FOUR lanes (a "quad"), for calls that hold too few frames to fill the
 // machine with one thread per trellis (a 1528-byte frame is 12312 dependent trellis steps; one warp per scheduler runs
-// them in ~1.7 ms however idle the GPU is).  Lane g of a quad owns the natural metric words {g, g+4, g+8, g+12} (and
-// the path words), i.e. local word i <-> natural word g + 4i.  In VitCore::step4's schedule that ownership makes
-//   step A (natural, pairs word j with j+8)        local: j = g and j = g + 4
-//   step B (stride 2, pairs S[j] with S[j+4])      local
-//   step C (stride 4, pairs Q[4j+o], Q[4(j+2)+o])  one exchange with lane g ^ 2 (two metric + two path words each way)
-//   step D (stride 8, pairs S[o], S[8+o])          one exchange with lane g ^ 1
-//   the 4x4 byte transpose back to natural order   local, and lands on the ownership step A needs
+// them in ~1.7 ms however idle the GPU is).
+// Metrics and path bytes are byte-packed: natural word w holds states 4w .. 4w + 3, 16 metric and 16 path words per
+// trellis.  Metrics never exceed 12 + 4 * 16 (spread bound of the code + growth between renormalisations, every fourth
+// chunk), so bytes cannot carry into each other.  The four-step schedule of the 16 words (b = byte lane, k = butterfly,
+// which pairs old states k and k + 32; S and Q are the split layouts between steps):
+//   step A  natural: words j, j + 8, k = 4j + b                  -> S[j] = states 8j + 2b, S[8 + j] = states 8j + 2b + 1
+//   step B  stride 2: S[j], S[j + 4], k = 8j + 2b (o = 0, 1); S[8 + j], S[12 + j], k = 8j + 2b + 1 (o = 2, 3)
+//                                                                -> Q[4j + o] = states 16j + 4b + o
+//   step C  stride 4: Q[4j + o], Q[4(j + 2) + o], k = 16j + 4b + o -> S[8j + o'] = states 32j + 8b + o', o' = 2o, 2o + 1
+//   step D  stride 8: S[o], S[8 + o], k = 8b + o                  -> Q[o'] = states 16b + o', o' = 2o, 2o + 1
+//   stride 16 -> natural: a 4x4 byte transpose per four words, natural word w byte i = Q[4 (w % 4) + i] byte (w / 4)
+// Lane g of a quad owns the natural metric words {g, g+4, g+8, g+12} (and the path words), i.e. local word i <-> natural
+// word g + 4i.  That ownership makes
+//   step A           local: j = g and j = g + 4
+//   step B           local
+//   step C           one exchange with lane g ^ 2 (two metric + two path words each way)
+//   step D           one exchange with lane g ^ 1
+//   the transpose    local, and lands on the ownership step A needs
 // so four trellis steps cost a quarter of the butterflies plus 8 shuffles per lane.  Which butterflies a lane computes
 // depends on g, so the branch selectors are per-lane registers (set up once) instead of immediates.  The eight quads of
 // a warp run in lock step (full-mask shuffles): the kernel gives them one trip count.
-// Results are those of VitCore bit for bit: same metrics, same tie rule, same path bytes, same first-best-state search.
+// Decoded bytes are those of VitCoreH bit for bit: same metrics, same tie rule, same first-best-state search.  The path
+// bytes are in upstream's bit order (earliest decision = MSB), VitCoreH's reversed.
 #define VQ_BLOCK 64                      // threads per block: 16 quads
 #define VQ_FRAMES (VQ_BLOCK / 4)
 #define VQ_RSTRIDE (VIT_NTB_MAX * 16 + 4) // ring words per frame; 164 = 4 (mod 32): the 8 quads x 4 lanes of a warp hit 32 banks
@@ -500,6 +264,15 @@ struct VitQuad {
     int g;
     bool hiC, hiD;
 
+    // per-step branch words: T = disagreements per (A,B) pattern, E = symbols present (not erased)
+    static __device__ __forceinline__ void branch(uint32_t nib, uint32_t &T, uint32_t &E)
+    {
+        const uint32_t s0 = nib & 3u, s1 = (nib >> 2) & 3u;
+        const uint32_t t0 = (s0 == 2u) ? 0u : (s0 ? 0x00000101u : 0x01010000u);
+        const uint32_t t1 = (s1 == 2u) ? 0u : (s1 ? 0x00010001u : 0x01000100u);
+        T = t0 + t1;
+        E = ((s0 != 2u) ? 0x01010101u : 0u) + ((s1 != 2u) ? 0x01010101u : 0u);
+    }
     static __device__ __forceinline__ uint32_t sel4(int k0, int k1, int k2, int k3)
     {
         const int k[4] = {k0, k1, k2, k3};
@@ -531,11 +304,15 @@ struct VitQuad {
           selD1 = sel4(o + 1, 9 + o, 17 + o, 25 + o); }
     }
 
+    // four packed butterflies: lo = old states k_b, hi = old states k_b + 32 (same byte lanes);
+    // v0/q0 = survivors of new states 2k_b, v1/q1 of 2k_b + 1
+    // BIT: the decision bit of this step inside the path byte.  The bytes are never shifted: step s of a
+    // chunk ORs its decision in at bit 7 - s (earliest decision = MSB, as upstream's shift register leaves it).
     template <uint32_t BIT>
     static __device__ __forceinline__ void bfly(uint32_t T, uint32_t E, uint32_t sel, uint32_t lo, uint32_t hi, uint32_t plo, uint32_t phi,
                                                 uint32_t &v0, uint32_t &v1, uint32_t &q0, uint32_t &q1)
     {
-        const uint32_t svm = prmt(T, 0u, sel), sv = E - svm;
+        const uint32_t svm = prmt(T, 0u, sel), sv = E - svm;   // agreements = available symbols - disagreements
         const uint32_t m0 = lo + sv, m1 = hi + svm, m2 = lo + svm, m3 = hi + sv;
         const uint32_t k0 = prmt(m0 + 0x7f7f7f7fu - m1, 0u, 0xba98u);
         const uint32_t k1 = prmt(m2 + 0x7f7f7f7fu - m3, 0u, 0xba98u);
@@ -588,7 +365,7 @@ struct VitQuad {
             bfly<B3>(T, E, selD0, la, ha, pla, pha, q[0], q[1], qp[0], qp[1]);
             bfly<B3>(T, E, selD1, lb, hb, plb, phb, q[2], q[3], qp[2], qp[3]);
         }
-        // lane g holds Q[4g .. 4g+3]: the transpose of VitCore::step4, group g -> natural words g, g+4, g+8, g+12
+        // lane g holds Q[4g .. 4g+3]: the byte transpose of group g -> natural words g, g+4, g+8, g+12
         uint32_t t0 = prmt(q[0], q[1], 0x5140u), t1 = prmt(q[0], q[1], 0x7362u);
         uint32_t t2 = prmt(q[2], q[3], 0x5140u), t3 = prmt(q[2], q[3], 0x7362u);
         m[0] = prmt(t0, t2, 0x5410u); m[1] = prmt(t0, t2, 0x7632u); m[2] = prmt(t1, t3, 0x5410u); m[3] = prmt(t1, t3, 0x7632u);
@@ -599,7 +376,7 @@ struct VitQuad {
 
     // ring: this frame's VIT_NTB_MAX x 16 words (natural order).  All four lanes follow the traceback (same addresses:
     // broadcast reads), so no lane waits for another's result.
-    __device__ __forceinline__ VitCore::Trace trace_begin(uint32_t *ring, int slot, int ntb, bool renorm)
+    __device__ __forceinline__ VitTrace trace_begin(uint32_t *ring, int slot, int ntb, bool renorm)
     {
         __syncwarp();                                        // the quad is done reading the slot this snapshot replaces
 #pragma unroll
@@ -618,11 +395,11 @@ struct VitQuad {
         kbest = max(kbest, __shfl_xor_sync(0xffffffffu, kbest, 1));
         kbest = max(kbest, __shfl_xor_sync(0xffffffffu, kbest, 2));  // (also orders the snapshot stores before the quad's reads)
         __syncwarp();
-        VitCore::Trace t;
+        VitTrace t;
         t.bs = 63 - (int)(kbest & 0xffu);
         t.sl = slot;
         t.left = ntb - 1;
-        if (renorm) {
+        if (renorm) {                                        // by max - 12, as VitCoreH::trace_begin
             const uint32_t mx = kbest >> 8;
             const uint32_t minw = (mx > 12u ? mx - 12u : 0u) * 0x01010101u;
 #pragma unroll
@@ -637,7 +414,7 @@ struct VitQuad {
         return reinterpret_cast<const uint8_t *>(ring)[sl * 64 + bs];
     }
     template <int N>
-    static __device__ __forceinline__ void trace_hops(VitCore::Trace &t, const uint32_t *ring, int ntb)
+    static __device__ __forceinline__ void trace_hops(VitTrace &t, const uint32_t *ring, int ntb)
     {
 #pragma unroll
         for (int i = 0; i < N; ++i) {
@@ -697,55 +474,7 @@ struct VitCoreSoft {
 #pragma unroll
         for (int i = 0; i < 32; ++i) { M[i] = 0; P[i] = 0; }
     }
-    // selector picking halfword (2A+B) of the (Tlo, Thi) pair for butterflies 2j (low lane), 2j+1 (high lane)
-    static __host__ __device__ constexpr uint32_t selx(int j)
-    {
-        uint32_t s = 0;
-        for (int b = 0; b < 2; ++b) {
-            uint32_t k = 2 * j + b;
-            uint32_t idx = 2 * vit_par((2 * k) & 0x6d) + vit_par((2 * k) & 0x4f);
-            s |= ((2 * idx) | ((2 * idx + 1) << 4)) << (8 * b);
-        }
-        return s;
-    }
-    __device__ __forceinline__ void step(int q0, int q1)
-    {
-        const uint32_t t11 = (uint32_t)(q0 + q1 + 254), t00 = 508u - t11;
-        const uint32_t t10 = (uint32_t)(q0 - q1 + 254), t01 = 508u - t10;
-        const uint32_t Tlo = t00 | (t01 << 16), Thi = t10 | (t11 << 16);
-        uint32_t Mn[32], Pn[32];
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-            const uint32_t x = prmt(Tlo, Thi, selx(j)), y = 0x01fc01fcu - x;
-            const uint32_t lo = M[j], hi = M[j + 16];
-            const uint32_t m0 = lo + x, m1 = hi + y, m2 = lo + y, m3 = hi + x;
-            const uint32_t k0 = prmt(m0 + 0x7fff7fffu - m1, 0u, 0xbb99u);   // 0xffff where m0 > m1
-            const uint32_t k1 = prmt(m2 + 0x7fff7fffu - m3, 0u, 0xbb99u);
-            const uint32_t v0 = (m0 & k0) | (m1 & ~k0);
-            const uint32_t v1 = (m2 & k1) | (m3 & ~k1);
-            const uint32_t sh0 = P[j] << 1, sh1 = (P[j + 16] << 1) | 0x00010001u;
-            const uint32_t p0 = (sh0 & k0) | (sh1 & ~k0);
-            const uint32_t p1 = (sh0 & k1) | (sh1 & ~k1);
-            Mn[2 * j] = prmt(v0, v1, 0x5410u);
-            Mn[2 * j + 1] = prmt(v0, v1, 0x7632u);
-            Pn[2 * j] = prmt(p0, p1, 0x5410u);
-            Pn[2 * j + 1] = prmt(p0, p1, 0x7632u);
-        }
-#pragma unroll
-        for (int i = 0; i < 32; ++i) { M[i] = Mn[i]; P[i] = Pn[i]; }
-    }
-    // selector picking, for two butterflies k0 (low lane) and k1 (high lane), halfword (2A+B) of (Tlo, Thi)
-    static __host__ __device__ constexpr uint32_t sel2(int k0, int k1)
-    {
-        const int k[2] = {k0, k1};
-        uint32_t s = 0;
-        for (int b = 0; b < 2; ++b) {
-            uint32_t idx = 2 * vit_par((2 * k[b]) & 0x6d) + vit_par((2 * k[b]) & 0x4f);
-            s |= ((2 * idx) | ((2 * idx + 1) << 4)) << (8 * b);
-        }
-        return s;
-    }
-    // BIT: position of this step's decision in the path halfword (never shifted, see VitCore::bfly)
+    // BIT: position of this step's decision in the path halfword (never shifted, see VitQuad::bfly)
     template <uint32_t BIT>
     static __device__ __forceinline__ void bfly(uint32_t Tlo, uint32_t Thi, uint32_t sel, uint32_t lo, uint32_t hi, uint32_t plo, uint32_t phi,
                                                 uint32_t &v0, uint32_t &v1, uint32_t &p0, uint32_t &p1)
@@ -767,7 +496,7 @@ struct VitCoreSoft {
         Tlo = t00 | (t01 << 16);
         Thi = t10 | (t11 << 16);
     }
-    // Four steps with one re-layout (see VitCore::step4): with two states per word the stride inside a
+    // Four steps with one re-layout (see the top of this file): with two states per word the stride inside a
     // word goes 1 -> 2 -> 4 -> 8 -> 16 and one halfword transpose per word pair restores natural order.
     // w0 / w1: the two input words (2 steps x 2 int8 each).
     template <int S0>
@@ -779,13 +508,13 @@ struct VitCoreSoft {
         // A: natural, pair j: k = 2j + b -> S[j] = {4j, 4j+2}, S[16+j] = {4j+1, 4j+3}
         branch((int)(int8_t)(w0 & 0xffu), (int)(int8_t)((w0 >> 8) & 0xffu), Tlo, Thi);
 #pragma unroll
-        for (int j = 0; j < 16; ++j) bfly<B0>(Tlo, Thi, sel2(2 * j, 2 * j + 1), M[j], M[j + 16], P[j], P[j + 16], S[j], S[16 + j], SP[j], SP[16 + j]);
+        for (int j = 0; j < 16; ++j) bfly<B0>(Tlo, Thi, vit_sel2(2 * j, 2 * j + 1), M[j], M[j + 16], P[j], P[j + 16], S[j], S[16 + j], SP[j], SP[16 + j]);
         // B: stride 2.  even pair j: k = 4j + 2b ; odd pair j: k = 4j + 2b + 1 -> Q[4j + o] = {8j + o, 8j + 4 + o}
         branch((int)(int8_t)((w0 >> 16) & 0xffu), (int)(int8_t)(w0 >> 24), Tlo, Thi);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
-            bfly<B1>(Tlo, Thi, sel2(4 * j, 4 * j + 2), S[j], S[j + 8], SP[j], SP[j + 8], Q[4 * j], Q[4 * j + 1], QP[4 * j], QP[4 * j + 1]);
-            bfly<B1>(Tlo, Thi, sel2(4 * j + 1, 4 * j + 3), S[16 + j], S[24 + j], SP[16 + j], SP[24 + j], Q[4 * j + 2], Q[4 * j + 3], QP[4 * j + 2], QP[4 * j + 3]);
+            bfly<B1>(Tlo, Thi, vit_sel2(4 * j, 4 * j + 2), S[j], S[j + 8], SP[j], SP[j + 8], Q[4 * j], Q[4 * j + 1], QP[4 * j], QP[4 * j + 1]);
+            bfly<B1>(Tlo, Thi, vit_sel2(4 * j + 1, 4 * j + 3), S[16 + j], S[24 + j], SP[16 + j], SP[24 + j], Q[4 * j + 2], Q[4 * j + 3], QP[4 * j + 2], QP[4 * j + 3]);
         }
         // C: stride 4.  pair (j, o): k = 8j + 4b + o -> S[8j + o'] = {16j + o', 16j + 8 + o'}, o' = 2o, 2o+1
         branch((int)(int8_t)(w1 & 0xffu), (int)(int8_t)((w1 >> 8) & 0xffu), Tlo, Thi);
@@ -793,7 +522,7 @@ struct VitCoreSoft {
         for (int j = 0; j < 4; ++j)
 #pragma unroll
             for (int o = 0; o < 4; ++o)
-                bfly<B2>(Tlo, Thi, sel2(8 * j + o, 8 * j + 4 + o), Q[4 * j + o], Q[4 * (j + 4) + o], QP[4 * j + o], QP[4 * (j + 4) + o],
+                bfly<B2>(Tlo, Thi, vit_sel2(8 * j + o, 8 * j + 4 + o), Q[4 * j + o], Q[4 * (j + 4) + o], QP[4 * j + o], QP[4 * (j + 4) + o],
                      S[8 * j + 2 * o], S[8 * j + 2 * o + 1], SP[8 * j + 2 * o], SP[8 * j + 2 * o + 1]);
         // D: stride 8.  pair (j, o'): k = 16j + 8b + o' -> Q[16j + o''] = {32j + o'', 32j + 16 + o''}, o'' = 2o', 2o'+1
         branch((int)(int8_t)((w1 >> 16) & 0xffu), (int)(int8_t)(w1 >> 24), Tlo, Thi);
@@ -801,7 +530,7 @@ struct VitCoreSoft {
         for (int j = 0; j < 2; ++j)
 #pragma unroll
             for (int o = 0; o < 8; ++o)
-                bfly<B3>(Tlo, Thi, sel2(16 * j + o, 16 * j + 8 + o), S[8 * j + o], S[8 * (j + 2) + o], SP[8 * j + o], SP[8 * (j + 2) + o],
+                bfly<B3>(Tlo, Thi, vit_sel2(16 * j + o, 16 * j + 8 + o), S[8 * j + o], S[8 * (j + 2) + o], SP[8 * j + o], SP[8 * (j + 2) + o],
                      Q[16 * j + 2 * o], Q[16 * j + 2 * o + 1], QP[16 * j + 2 * o], QP[16 * j + 2 * o + 1]);
         // stride 16 -> natural: natural word w = {2w, 2w+1}; Q[16j + e], Q[16j + e + 1] (e even) hold them in the same lane
 #pragma unroll
@@ -815,7 +544,7 @@ struct VitCoreSoft {
             }
     }
     // snapshot + first best state (index-carrying tournament over adjacent words) + optional renormalisation
-    __device__ __forceinline__ VitCore::Trace trace_begin(uint32_t *ring, int slot, int ntb, int tid, bool renorm)
+    __device__ __forceinline__ VitTrace trace_begin(uint32_t *ring, int slot, int ntb, int tid, bool renorm)
     {
 #pragma unroll
         for (int w = 0; w < 16; ++w) ring[(slot * 16 + w) * VIT_BLOCK + tid] = prmt(P[2 * w], P[2 * w + 1], 0x6420u);
@@ -838,7 +567,7 @@ struct VitCoreSoft {
             }
         const int v0 = (int)(tv[0] & 0xffffu), s0 = (int)(ti[0] & 0xffffu) * 2;
         const int v1 = (int)(tv[0] >> 16), s1 = (int)(ti[0] >> 16) * 2 + 1;
-        VitCore::Trace t;
+        VitTrace t;
         t.bs = (v1 > v0 || (v1 == v0 && s1 < s0)) ? s1 : s0;
         t.sl = slot;
         t.left = ntb - 1;
@@ -855,53 +584,23 @@ struct VitCoreSoft {
         for (int i = 0; i < 32; ++i) P[i] = 0;
         return t;
     }
-    static __device__ __forceinline__ uint32_t vmax2(uint32_t a, uint32_t b)
-    {
-        uint32_t k = prmt((a | 0x80008000u) - b, 0u, 0xbb99u);
-        return (a & k) | (b & ~k);
-    }
     static __device__ __forceinline__ uint32_t vmin2(uint32_t a, uint32_t b)
     {
         uint32_t k = prmt((a | 0x80008000u) - b, 0u, 0xbb99u);
         return (b & k) | (a & ~k);
     }
-    __device__ __forceinline__ uint32_t end_chunk(uint32_t *ring, int slot, int ntb, int tid, bool renorm)
+    // ring bytes hold the decisions MSB first (upstream's order): the state eight steps back is the byte >> 2
+    template <int N>
+    static __device__ __forceinline__ void trace_hops(VitTrace &t, const uint32_t *ring, int ntb, int tid)
     {
 #pragma unroll
-        for (int w = 0; w < 16; ++w) ring[(slot * 16 + w) * VIT_BLOCK + tid] = prmt(P[2 * w], P[2 * w + 1], 0x6420u);
-        uint32_t mx = M[0];
-#pragma unroll
-        for (int w = 1; w < 32; ++w) mx = vmax2(mx, M[w]);
-        mx = vmax2(mx, mx >> 16);
-        const uint32_t bestw = (mx & 0xffffu) * 0x00010001u;
-        int wsel = 0;
-        uint32_t zsel = 0;
-#pragma unroll
-        for (int w = 31; w >= 0; --w) {
-            uint32_t x = M[w] ^ bestw;
-            uint32_t z = ((x + 0x7fff7fffu) & 0x80008000u) ^ 0x80008000u;   // bit 15 / 31 set where equal
-            if (z) { wsel = w; zsel = z; }
+        for (int i = 0; i < N; ++i) {
+            const bool go = t.left > 0;
+            const int nb = (int)(vit_ring_byte(ring, t.sl, t.bs, tid) >> 2);
+            const int ns = (t.sl == 0) ? ntb - 1 : t.sl - 1;
+            t.bs = go ? nb : t.bs;
+            t.sl = go ? ns : t.sl;
+            t.left -= go ? 1 : 0;
         }
-        int bs = wsel * 2 + ((__ffs((int)zsel) - 16) >> 4);
-        int sl = slot;
-        for (int i = 0; i < ntb - 1; ++i) {
-            uint32_t w = ring[(sl * 16 + (bs >> 2)) * VIT_BLOCK + tid];
-            bs = (int)((w >> (8 * (bs & 3))) & 0xffu) >> 2;
-            sl = (sl == 0) ? ntb - 1 : sl - 1;
-        }
-        uint32_t w = ring[(sl * 16 + (bs >> 2)) * VIT_BLOCK + tid];
-        uint32_t c = (w >> (8 * (bs & 3))) & 0xffu;
-        if (renorm) {
-            uint32_t mn = M[0];
-#pragma unroll
-            for (int i = 1; i < 32; ++i) mn = vmin2(mn, M[i]);
-            mn = vmin2(mn, mn >> 16);
-            const uint32_t minw = (mn & 0xffffu) * 0x00010001u;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) M[i] -= minw;
-        }
-#pragma unroll
-        for (int i = 0; i < 32; ++i) P[i] = 0;
-        return c;
     }
 };

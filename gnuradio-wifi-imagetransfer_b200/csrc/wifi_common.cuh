@@ -119,31 +119,9 @@ __device__ __forceinline__ int64_t job_row(const JobDesc &J, const wifi_b200_fra
     return frames[J.last_frame].row_off + left;
 }
 
-__device__ __forceinline__ int dev_decide(int nb, cf s)
-{
-    if (nb == 1) return s.re > 0;
-    if (nb == 2) return (s.re > 0) | ((s.im > 0) << 1);
-    if (nb == 4) {
-        const float level = sqrtf(0.1f);
-        int r = s.re > 0;
-        r |= (fabsf(s.re) < (2 * level)) << 1;
-        r |= (s.im > 0) << 2;
-        r |= (fabsf(s.im) < (2 * level)) << 3;
-        return r;
-    }
-    const float level = sqrtf(1.0f / 42.0f);
-    float ar = fabsf(s.re), ai = fabsf(s.im);
-    int r = s.re > 0;
-    r |= (ar < (4 * level)) << 1;
-    r |= ((ar < (6 * level)) && (ar > (2 * level))) << 2;
-    r |= (s.im > 0) << 3;
-    r |= (ai < (4 * level)) << 4;
-    r |= ((ai < (6 * level)) && (ai > (2 * level))) << 5;
-    return r;
-}
-
-// One axis of a decision and of the decided constellation point.  The comparisons are dev_decide()'s, the
-// point is the table value (float)(+-magnitude) * level picked by selects instead of rebuilt from the bits.
+// One axis of a decision and of the decided constellation point.  The comparisons are those of upstream's
+// decision_maker (the oracle's decide()), the point is the table value (float)(+-magnitude) * level picked by
+// selects instead of rebuilt from the bits.
 template <int H>   // bits per axis: 1, 2, 3
 __device__ __forceinline__ void dev_axis(float v, int &bits, float &pt)
 {
@@ -266,25 +244,4 @@ __device__ __forceinline__ SoftQ dev_soft_demap(int nb, cf s, float w)
         }
     }
     return r;
-}
-
-// constellation point of a decided index, computed exactly as the table is built
-// ((float)(+-magnitude) * level), so no lane-divergent constant-memory lookup is needed
-__device__ __forceinline__ cf dev_point(int nb, int v)
-{
-    if (nb == 1) return {v ? 1.f : -1.f, 0.f};
-    const int h = nb >> 1;
-    const float level = (h == 1) ? sqrtf(0.5f) : (h == 2) ? sqrtf(0.1f) : sqrtf(1.0f / 42.0f);
-    const int top = (1 << h) - 1;                  // 1, 3, 7: outermost magnitude
-    float o[2];
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-        const int ax = u ? (v >> h) : (v & top);
-        // magnitude bits b1 (b2) are a Gray code of the distance from the outermost level
-        const int b1 = (ax >> 1) & 1, b2 = (ax >> 2) & 1;
-        const int g = (h == 3) ? ((b1 << 1) | (b1 ^ b2)) : b1;      // h == 1: b1 = 0
-        const int mag = top - 2 * g;
-        o[u] = (float)((ax & 1) ? mag : -mag) * level;
-    }
-    return {o[0], o[1]};
 }
