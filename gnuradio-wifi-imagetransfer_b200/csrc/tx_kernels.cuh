@@ -154,3 +154,49 @@ __global__ void __launch_bounds__(256) k_channel(const cf *__restrict__ in, cf *
         out[S.out_off + i] = y;
     }
 }
+
+// time-varying fading channel (wifi_b200_channel_fading_dev), mirrors tests/fading_oracle.cpp: the taps of k_channel become
+// h_t(t0 + i) of include/wifi_detmath.h; gain, CFO rotation and Philox AWGN are k_channel's.  The block first draws its
+// segment's terms into shared memory (tap t at slots t * FADE_SLOTS ..; tap 0's line-of-sight term follows its n_sin
+// sinusoids), then every sample evaluates one NCO sincos and one complex multiply-accumulate per term.
+#define FADE_SLOTS 17
+__global__ void __launch_bounds__(256) k_channel_fading(const cf *__restrict__ in, cf *__restrict__ out, const wifi_b200_chan_seg *__restrict__ segs,
+                                                        const wifi_b200_fading *__restrict__ fades, int n_segs)
+{
+    __shared__ wdm_fade_ent ent[8 * FADE_SLOTS];
+    const int sidx = blockIdx.y;
+    if (sidx >= n_segs) return;
+    const wifi_b200_chan_seg S = segs[sidx];
+    const wifi_b200_fading F = fades[sidx];
+    const int cnt0 = F.n_sin + (F.k_factor > 0.f ? 1 : 0);
+    for (int k = threadIdx.x; k < F.n_taps * FADE_SLOTS; k += blockDim.x) {
+        const int t = k / FADE_SLOTS, m = k - t * FADE_SLOTS;
+        if (m < (t == 0 ? cnt0 : F.n_sin))
+            ent[k] = wdm_fading_entry(F.seed, F.stream, t, m, F.n_sin, F.power[t], F.k_factor, F.doppler, F.los_doppler);
+    }
+    __syncthreads();
+    const float ns = S.noise_sigma * 0.70710678f;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < S.n; i += (int64_t)gridDim.x * blockDim.x) {
+        const uint32_t n = (uint32_t)(F.t0 + i);
+        cf acc = {0.f, 0.f};
+        for (int t = 0; t < F.n_taps; ++t) {
+            int64_t j = i - F.delay[t];
+            if (j < 0 || j >= S.in_len) continue;
+            acc = wdm_cmac(acc, wdm_fading_tap(ent + t * FADE_SLOTS, t == 0 ? cnt0 : F.n_sin, n), in[S.in_off + j]);
+        }
+        acc = cscale(acc, S.gain);
+        cf w = crot(S.cfo * (float)i + S.phase0);
+        cf y = cmul(acc, w);
+        if (S.noise_sigma > 0.f) {
+            uint64_t idx = (uint64_t)(S.n0 + i);
+            uint32_t r[4];
+            wdm_philox4x32((uint32_t)idx, (uint32_t)(idx >> 32), (uint32_t)S.stream, (uint32_t)(S.stream >> 32),
+                           (uint32_t)S.seed, (uint32_t)(S.seed >> 32), r);
+            float z0, z1;
+            wdm_box_muller(r[0], r[1], &z0, &z1);
+            y.re = y.re + ns * z0;
+            y.im = y.im + ns * z1;
+        }
+        out[S.out_off + i] = y;
+    }
+}

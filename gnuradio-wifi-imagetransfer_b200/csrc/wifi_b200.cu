@@ -3,6 +3,7 @@
 // No CPU fallback anywhere in this file: every entry point that computes launches CUDA kernels.
 #include <sched.h>
 
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -215,6 +216,8 @@ struct wifi_b200 {
     int tx_seed = 1;               // [UPSTREAM] mapper.cc d_scrambler: 1, ++ per frame, wraps after 127
     wifi_b200_chan_seg *d_segs = nullptr;
     int segs_cap = 0;
+    wifi_b200_fading *d_fades = nullptr;
+    int fades_cap = 0;
     // last rx call
     const cf *cur_iq = nullptr;
     std::vector<LinkDesc> h_links;
@@ -305,7 +308,7 @@ void free_all(wifi_b200 *h)
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     for (int k = 0; k < A_SLOTS; ++k) if (h->a_ev[k]) cudaEventDestroy(h->a_ev[k]);
     void *ptrs[] = {h->d_stage[0], h->d_stage[1], h->d_stage[2], h->d_stream, h->d_moves, h->d_sc16, h->d_iq, h->d_flags, h->d_links, h->d_frames, h->d_states, h->d_rows, h->d_carrier, h->d_jobs, h->d_vit_in,
-                    h->d_psdu, h->d_depunct, h->d_counters, h->d_summary, h->d_trig_tmp, h->d_pack_list, h->d_link_dirty, h->d_spec_trig, h->d_spec_cnt, h->d_spec_trig2, h->d_spec_cnt2, h->d_soft, h->d_vit_soft_in, h->d_txblob, h->d_txdesc, h->d_txsym, h->d_txiq, h->d_segs};
+                    h->d_psdu, h->d_depunct, h->d_counters, h->d_summary, h->d_trig_tmp, h->d_pack_list, h->d_link_dirty, h->d_spec_trig, h->d_spec_cnt, h->d_spec_trig2, h->d_spec_cnt2, h->d_soft, h->d_vit_soft_in, h->d_txblob, h->d_txdesc, h->d_txsym, h->d_txiq, h->d_segs, h->d_fades};
     for (void *p : ptrs) if (p) cudaFree(p);
     if (h->h_counters) cudaFreeHost(h->h_counters);
     if (h->h_frames) cudaFreeHost(h->h_frames);
@@ -811,7 +814,7 @@ int wifi_b200_create(const wifi_b200_cfg *cfg_in, wifi_b200_t **out)
         const void *kernels[] = {(const void *)k_detect, (const void *)k_select_spec, (const void *)k_select_fix, (const void *)k_select, (const void *)k_reserve,
                                  (const void *)k_frames_init, (const void *)k_sync_long, (const void *)k_signal, (const void *)k_plan_fast,
                                  (const void *)k_plan, (const void *)k_pack, (const void *)k_viterbi, (const void *)k_viterbi_warp,
-                                 (const void *)k_move_segments, (const void *)k_viterbi_quad, (const void *)k_append_sc16, (const void *)k_sc16_to_fc32, (const void *)k_tx, (const void *)k_channel,
+                                 (const void *)k_move_segments, (const void *)k_viterbi_quad, (const void *)k_append_sc16, (const void *)k_sc16_to_fc32, (const void *)k_tx, (const void *)k_channel, (const void *)k_channel_fading,
                                  (const void *)k_demod<false, WIFI_EQ_LS, 0>, (const void *)k_demod<false, WIFI_EQ_LS, 1>,
                                  (const void *)k_demod<false, WIFI_EQ_LMS, 0>, (const void *)k_demod<false, WIFI_EQ_LMS, 1>,
                                  (const void *)k_demod<false, WIFI_EQ_COMB, 0>, (const void *)k_demod<false, WIFI_EQ_COMB, 1>,
@@ -1067,6 +1070,85 @@ int wifi_b200_channel(wifi_b200_t *h, const float *in_host, int64_t in_len, floa
             return WIFI_E_ARG;
         }
     int rc = wifi_b200_channel_dev(h, (const float *)d_in, (float *)d_out, segs, n_segs);
+    if (rc == WIFI_OK) {
+        std::lock_guard<std::mutex> g(h->mu);
+        if (cudaMemcpy(out_host, d_out, (size_t)out_len * sizeof(cf), cudaMemcpyDeviceToHost) != cudaSuccess) rc = WIFI_E_CUDA;
+    }
+    cudaFree(d_in);
+    cudaFree(d_out);
+    return rc;
+}
+
+static bool fading_ok(const wifi_b200_chan_seg &s, const wifi_b200_fading &f)
+{
+    if (s.n_taps != 0 || s.n < 0 || f.n_taps < 1 || f.n_taps > 8 || f.n_sin < 1 || f.n_sin > 16) return false;
+    if (!(f.k_factor >= 0.f && f.k_factor <= FLT_MAX) || !(f.doppler >= 0.f && f.doppler <= 0.25f) || !(fabsf(f.los_doppler) <= 0.25f)) return false;
+    for (int t = 0; t < f.n_taps; ++t)
+        if (f.delay[t] < 0 || !(f.power[t] >= 0.f && f.power[t] <= FLT_MAX)) return false;
+    return true;
+}
+
+int wifi_b200_channel_fading_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, const wifi_b200_chan_seg *segs,
+                                 const wifi_b200_fading *fades, int n_segs)
+{
+    if (!h || !in_dev || !out_dev || !segs || !fades || n_segs <= 0) return WIFI_E_ARG;
+    std::lock_guard<std::mutex> g(h->mu);
+    cudaSetDevice(h->device);
+    int64_t maxn = 0;
+    for (int i = 0; i < n_segs; ++i) {
+        if (!fading_ok(segs[i], fades[i])) { h->err = "bad fading channel segment"; return WIFI_E_ARG; }
+        maxn = std::max(maxn, segs[i].n);
+    }
+    if (n_segs > h->segs_cap) {
+        if (h->d_segs) cudaFree(h->d_segs);
+        h->d_segs = nullptr;
+        CK(cudaMalloc(&h->d_segs, (size_t)(n_segs + 64) * sizeof(wifi_b200_chan_seg)));
+        h->segs_cap = n_segs + 64;
+    }
+    if (n_segs > h->fades_cap) {
+        if (h->d_fades) cudaFree(h->d_fades);
+        h->d_fades = nullptr;
+        CK(cudaMalloc(&h->d_fades, (size_t)(n_segs + 64) * sizeof(wifi_b200_fading)));
+        h->fades_cap = n_segs + 64;
+    }
+    CK(cudaMemcpyAsync(h->d_segs, segs, (size_t)n_segs * sizeof(wifi_b200_chan_seg), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_fades, fades, (size_t)n_segs * sizeof(wifi_b200_fading), cudaMemcpyHostToDevice, h->stream));
+    for (int base = 0; base < n_segs; base += 65535) {
+        int cnt = std::min(65535, n_segs - base);
+        dim3 grid((unsigned)std::min<int64_t>((maxn + 255) / 256, 4096), cnt);
+        if (grid.x == 0) grid.x = 1;
+        k_channel_fading<<<grid, 256, 0, h->stream>>>((const cf *)in_dev, (cf *)out_dev, h->d_segs + base, h->d_fades + base, cnt);
+    }
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(h->stream));
+    return WIFI_OK;
+}
+
+// host-buffer form of the fading channel, staged as wifi_b200_channel stages
+int wifi_b200_channel_fading(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
+                             const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs)
+{
+    if (!h || !in_host || !out_host || !segs || !fades || in_len <= 0 || out_len <= 0 || n_segs <= 0) return WIFI_E_ARG;
+    for (int i = 0; i < n_segs; ++i)
+        if (segs[i].in_off < 0 || segs[i].in_len < 0 || segs[i].in_off + segs[i].in_len > in_len || segs[i].out_off < 0 ||
+            segs[i].n < 0 || segs[i].out_off + segs[i].n > out_len) {
+            h->err = "channel segment outside the buffers";
+            return WIFI_E_ARG;
+        }
+    cf *d_in = nullptr, *d_out = nullptr;
+    {
+        std::lock_guard<std::mutex> g(h->mu);
+        cudaSetDevice(h->device);
+        CK(cudaMalloc(&d_in, (size_t)in_len * sizeof(cf)));
+        if (cudaMalloc(&d_out, (size_t)out_len * sizeof(cf)) != cudaSuccess) { cudaFree(d_in); h->err = "cudaMalloc"; return WIFI_E_NOMEM; }
+        if (cudaMemcpy(d_in, in_host, (size_t)in_len * sizeof(cf), cudaMemcpyHostToDevice) != cudaSuccess ||
+            cudaMemset(d_out, 0, (size_t)out_len * sizeof(cf)) != cudaSuccess) {
+            cudaFree(d_in); cudaFree(d_out);
+            h->err = "channel staging copy";
+            return WIFI_E_CUDA;
+        }
+    }
+    int rc = wifi_b200_channel_fading_dev(h, (const float *)d_in, (float *)d_out, segs, fades, n_segs);
     if (rc == WIFI_OK) {
         std::lock_guard<std::mutex> g(h->mu);
         if (cudaMemcpy(out_host, d_out, (size_t)out_len * sizeof(cf), cudaMemcpyDeviceToHost) != cudaSuccess) rc = WIFI_E_CUDA;
@@ -1675,10 +1757,9 @@ int wifi_b200_host_alloc(wifi_b200_t *h, size_t bytes, void **out)
     }
     void *p = nullptr;
     const cudaError_t e = cudaHostAlloc(&p, bytes, cudaHostAllocPortable);
-    if (e == cudaSuccess) {
-        volatile char *c = (volatile char *)p;                        // first touch from the GPU's side of the machine
-        for (size_t i = 0; i < bytes; i += 4096) c[i] = 0;
-    }
+    // first touch from the GPU's side of the machine; the whole buffer, because the driver may hand back pinned pages a
+    // previous allocation of this process left data in
+    if (e == cudaSuccess) memset(p, 0, bytes);
     if (moved) sched_setaffinity(0, sizeof old_set, &old_set);
     if (e != cudaSuccess) { cudaGetLastError(); h->err = "cudaHostAlloc failed"; return WIFI_E_NOMEM; }
     *out = p;

@@ -27,8 +27,13 @@ class IrsTransceiver:
     """Defaults are the flowgraph's variables (IRS_tranceiver.py:80-92)."""
 
     def __init__(self, in_port=50010, out_addr=("localhost", 10010), snr=22.0, epsilon=0.0, encoding=3, chan_est=0,
-                 freq=5.89e9, samp_rate=20e6, device=0, mtu=1024, idle_flush_s=0.2, seed=0):
+                 freq=5.89e9, samp_rate=20e6, device=0, mtu=1024, idle_flush_s=0.2, seed=0, doppler_hz=None, k_factor=None):
         self.snr, self.epsilon, self.freq, self.samp_rate = float(snr), float(epsilon), float(freq), float(samp_rate)
+        # doppler_hz / k_factor (either one) replace the flowgraph's fixed tap [1] with one flat Rayleigh/Rician tap of unit
+        # power that fades continuously across datagrams: one realisation, sample n of the link at time n
+        self.fading = None
+        if doppler_hz is not None or k_factor is not None:
+            self.fading = dict(taps=((0, 1.0),), doppler=float(doppler_hz or 0.0) / self.samp_rate, k_factor=float(k_factor or 0.0), seed=seed)
         self.mtu, self.idle_flush_s, self.seed = mtu, idle_flush_s, seed
         self.phy = wifi_phy_hier(bandwidth=samp_rate, chan_est=chan_est, encoding=encoding, frequency=freq, sensitivity=0.56,
                                  device=device, max_samples=1 << 20)
@@ -66,7 +71,9 @@ class IrsTransceiver:
         # channel_model(frequency_offset = epsilon * freq / 10e6) (IRS_tranceiver.py:284,425,434): GNU Radio reads that
         # value as normalised cycles per sample, i.e. a phase step of 2 pi frequency_offset; the library's cfo is rad/sample
         cfo = 2 * math.pi * self.epsilon * self.freq / 10e6
-        y = self.phy.handle.channel(x, n_out=n_out, n0=self._n0, gain=gain, cfo=cfo, noise_sigma=math.sqrt(2.0), seed=self.seed)
+        fading = None if self.fading is None else dict(self.fading, t0=self._n0)
+        y = self.phy.handle.channel(x, n_out=n_out, n0=self._n0, gain=gain, cfo=cfo, noise_sigma=math.sqrt(2.0), seed=self.seed,
+                                    fading=fading)
         self._n0 += n_out
         return y
 
@@ -118,8 +125,11 @@ def main():
     ap.add_argument("--encoding", type=int, default=3)
     ap.add_argument("--chan-est", type=int, default=0)
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--doppler-hz", type=float, default=None, help="maximum Doppler shift of a flat fading channel (Hz)")
+    ap.add_argument("--k-factor", type=float, default=None, help="Rician K of the flat fading channel (linear, 0: Rayleigh)")
     a = ap.parse_args()
-    t = IrsTransceiver(a.in_port, (a.out_host, a.out_port), a.snr, a.epsilon, a.encoding, a.chan_est, device=a.device)
+    t = IrsTransceiver(a.in_port, (a.out_host, a.out_port), a.snr, a.epsilon, a.encoding, a.chan_est, device=a.device,
+                       doppler_hz=a.doppler_hz, k_factor=a.k_factor)
     print("listening on UDP :%d, forwarding decoded patches to %s:%d" % (t.in_port, a.out_host, a.out_port))
     try:
         t.serve()

@@ -42,6 +42,18 @@ CHANSEG_DTYPE = np.dtype([
 assert CHANSEG_DTYPE.itemsize == C.sizeof(ChanSeg), (CHANSEG_DTYPE.itemsize, C.sizeof(ChanSeg))
 
 
+class Fading(C.Structure):
+    _fields_ = [("n_taps", C.c_int32), ("n_sin", C.c_int32), ("delay", C.c_int32 * 8), ("power", C.c_float * 8),
+                ("k_factor", C.c_float), ("doppler", C.c_float), ("los_doppler", C.c_float), ("reserved", C.c_int32),
+                ("t0", C.c_int64), ("seed", C.c_uint64), ("stream", C.c_uint64)]
+
+
+FADING_DTYPE = np.dtype([
+    ("n_taps", "<i4"), ("n_sin", "<i4"), ("delay", "<i4", (8,)), ("power", "<f4", (8,)), ("k_factor", "<f4"), ("doppler", "<f4"),
+    ("los_doppler", "<f4"), ("reserved", "<i4"), ("t0", "<i8"), ("seed", "<u8"), ("stream", "<u8")], align=True)
+assert FADING_DTYPE.itemsize == C.sizeof(Fading) == 112, (FADING_DTYPE.itemsize, C.sizeof(Fading))
+
+
 LINK_STATE_DTYPE = np.dtype([("min_pos", "<i8"), ("fo_carry", "<f4"), ("hist", "<i4")], align=True)
 
 
@@ -60,7 +72,7 @@ EXPORTS = [
     "wifi_b200_abi_version", "wifi_b200_device_count", "wifi_b200_create", "wifi_b200_destroy", "wifi_b200_set_param",
     "wifi_b200_get_param", "wifi_b200_last_error", "wifi_b200_strerror", "wifi_b200_stream", "wifi_b200_sync",
     "wifi_b200_mac_frame", "wifi_b200_n_sym", "wifi_b200_frame_samples", "wifi_b200_tx", "wifi_b200_tx_dev",
-    "wifi_b200_tx_symbols", "wifi_b200_channel_dev", "wifi_b200_channel", "wifi_b200_rx_batch", "wifi_b200_rx_batch_dev", "wifi_b200_rx_batch_dev_state", "wifi_b200_rx_batch_sc16", "wifi_b200_rx_counts",
+    "wifi_b200_tx_symbols", "wifi_b200_channel_dev", "wifi_b200_channel", "wifi_b200_channel_fading_dev", "wifi_b200_channel_fading", "wifi_b200_rx_batch", "wifi_b200_rx_batch_dev", "wifi_b200_rx_batch_dev_state", "wifi_b200_rx_batch_sc16", "wifi_b200_rx_counts",
     "wifi_b200_rx_frames", "wifi_b200_rx_rows", "wifi_b200_rx_psdus", "wifi_b200_rx_soft", "wifi_b200_rx_flags", "wifi_b200_rx_push",
     "wifi_b200_rx_pop", "wifi_b200_rx_reset", "wifi_b200_rx_push_links", "wifi_b200_get_stats", "wifi_b200_stage_times", "wifi_b200_stage_name",
     "wifi_b200_selftest_detmath", "wifi_b200_alu_peak", "wifi_b200_rx_push_links_async", "wifi_b200_rx_push_links_sc16_async", "wifi_b200_rx_push_wait", "wifi_b200_rx_pop_view",
@@ -97,6 +109,8 @@ def lib():
         L.wifi_b200_tx_symbols.restype = i64
         L.wifi_b200_channel_dev.argtypes = [vp, vp, vp, vp, C.c_int]
         L.wifi_b200_channel.argtypes = [vp, vp, i64, vp, i64, vp, C.c_int]
+        L.wifi_b200_channel_fading_dev.argtypes = [vp, vp, vp, vp, vp, C.c_int]
+        L.wifi_b200_channel_fading.argtypes = [vp, vp, i64, vp, i64, vp, vp, C.c_int]
         for f in ("wifi_b200_rx_batch", "wifi_b200_rx_batch_dev"):
             getattr(L, f).argtypes = [vp, vp, vp, C.c_int, C.c_int]
         L.wifi_b200_rx_batch_dev_state.argtypes = [vp, vp, vp, C.c_int, C.c_int, vp]
@@ -162,6 +176,21 @@ def chan_seg(in_off=0, in_len=0, out_off=0, n=0, n0=0, gain=1.0, cfo=0.0, phase0
         s["delay"][0, i], s["tap_re"][0, i], s["tap_im"][0, i] = d, np.float32(complex(hh).real), np.float32(complex(hh).imag)
     s["seed"], s["stream"] = seed, stream
     return s
+
+
+def fading(taps=((0, 1.0),), n_sin=8, k_factor=0.0, doppler=0.0, los_doppler=0.0, t0=0, seed=0, stream=0):
+    """One wifi_b200_fading record: taps = ((delay, power), ...) with power = E|h_t|^2; doppler and los_doppler in
+    cycles/sample; the realisation is (seed, stream), placed in time by t0."""
+    f = np.zeros(1, FADING_DTYPE)
+    f["n_taps"], f["n_sin"] = len(taps), n_sin
+    for i, (d, p) in enumerate(taps):
+        f["delay"][0, i], f["power"][0, i] = d, p
+    f["k_factor"], f["doppler"], f["los_doppler"] = k_factor, doppler, los_doppler
+    f["t0"], f["seed"], f["stream"] = t0, seed, stream
+    return f
+
+
+_fading = fading     # Handle.channel's keyword of the same name hides it there
 
 
 class RxResult:
@@ -262,13 +291,27 @@ class Handle:
         segs = np.ascontiguousarray(segs, CHANSEG_DTYPE)
         self._ck(self._L.wifi_b200_channel_dev(self._h, C.c_void_p(in_ptr), C.c_void_p(out_ptr), _p(segs), segs.size))
 
-    def channel(self, x, n_out=None, **kw):
-        """One-segment convenience form of the test channel on host arrays (keywords as chan_seg())."""
+    def channel_fading_dev(self, in_ptr, out_ptr, segs, fades):
+        """Fading channel on device buffers: one FADING_DTYPE record per CHANSEG_DTYPE segment (whose n_taps is 0)."""
+        segs = np.ascontiguousarray(segs, CHANSEG_DTYPE)
+        fades = np.ascontiguousarray(fades, FADING_DTYPE)
+        if fades.size != segs.size:
+            raise ValueError("one fading record per segment")
+        self._ck(self._L.wifi_b200_channel_fading_dev(self._h, C.c_void_p(in_ptr), C.c_void_p(out_ptr), _p(segs), _p(fades), segs.size))
+
+    def channel(self, x, n_out=None, fading=None, **kw):
+        """One-segment convenience form of the test channel on host arrays (keywords as chan_seg()).  fading: None for the
+        fixed taps, or a FADING_DTYPE record / a dict of fading() keywords for time-varying taps (then `taps` is not given)."""
         a = np.ascontiguousarray(x, np.complex64)
         n_out = a.size if n_out is None else int(n_out)
         out = np.empty(n_out, np.complex64)
-        seg = chan_seg(in_len=a.size, n=n_out, **kw)
-        self._ck(self._L.wifi_b200_channel(self._h, _p(a), a.size, _p(out), n_out, _p(seg), 1))
+        if fading is None:
+            seg = chan_seg(in_len=a.size, n=n_out, **kw)
+            self._ck(self._L.wifi_b200_channel(self._h, _p(a), a.size, _p(out), n_out, _p(seg), 1))
+            return out
+        seg = chan_seg(in_len=a.size, n=n_out, taps=(), **kw)
+        f = np.ascontiguousarray(fading if isinstance(fading, np.ndarray) else _fading(**fading), FADING_DTYPE)
+        self._ck(self._L.wifi_b200_channel_fading(self._h, _p(a), a.size, _p(out), n_out, _p(seg), _p(f), 1))
         return out
 
     # ---- RX ----

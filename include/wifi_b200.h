@@ -120,6 +120,26 @@ typedef struct wifi_b200_chan_seg {
     uint64_t seed, stream;
 } wifi_b200_chan_seg;
 
+/* Time-varying multipath fading for one segment of wifi_b200_channel_fading_dev (DESIGN.md "fading channel"):
+ *     y(i) = gain * sum_t h_t(t0 + i) * x(i - delay[t]),  then the segment's CFO rotation and AWGN as in wifi_b200_channel_dev.
+ * Every tap is a sum of n_sin sinusoids with complex Gaussian weights and Clarke-spread frequencies (|f| <= doppler); tap 0
+ * adds a line-of-sight term of Rician factor k_factor.  doppler = 0 gives block fading, one CN(0, power[t]) value per tap.
+ * The realisation depends only on (seed, stream); t0 places the segment in time, so segments that share (seed, stream)
+ * and set t0 to their position form one continuous channel.  Phases are 32-bit NCOs: the process repeats every 2^32
+ * samples.  112 bytes, no implicit padding. */
+typedef struct wifi_b200_fading {
+    int32_t n_taps;           /* 1..8                                                              */
+    int32_t n_sin;            /* sinusoids per tap, 1..16                                           */
+    int32_t delay[8];         /* samples, >= 0                                                     */
+    float power[8];           /* E|h_t|^2, linear, >= 0                                            */
+    float k_factor;           /* Rician K of tap 0, linear, >= 0 (0: Rayleigh)                     */
+    float doppler;            /* maximum Doppler f_d / f_s, cycles/sample, 0 .. 0.25               */
+    float los_doppler;        /* Doppler of the line-of-sight term, cycles/sample, -0.25 .. 0.25    */
+    int32_t reserved;         /* 0                                                                 */
+    int64_t t0;               /* time index of output sample 0                                     */
+    uint64_t seed, stream;    /* Philox key and counter words of the realisation                    */
+} wifi_b200_fading;
+
 typedef struct wifi_b200 wifi_b200_t;
 
 int  wifi_b200_abi_version(void);
@@ -158,6 +178,12 @@ int  wifi_b200_channel_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, 
 /* same with host buffers (in: in_len complex samples, out: out_len, zero where no segment writes) */
 int  wifi_b200_channel(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
                        const wifi_b200_chan_seg *segs, int n_segs);
+/* the same with fading taps: segment i takes its taps from fades[i] (segs[i].n_taps must be 0); everything else in segs[i]
+ * keeps its meaning.  Out-of-range fields give WIFI_E_ARG before anything is written. */
+int  wifi_b200_channel_fading_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, const wifi_b200_chan_seg *segs,
+                                  const wifi_b200_fading *fades, int n_segs);
+int  wifi_b200_channel_fading(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
+                              const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs);
 
 /* ---- RX, batch form: n_links independent streams; link l is iq[link_off[l] .. link_off[l+1]) complex
  * samples.  final != 0: the streams end here (flush).  Results stay in the handle until the next rx call. */
@@ -228,7 +254,7 @@ int  wifi_b200_stage_times(wifi_b200_t *h, float *ms, int cap);
 const char *wifi_b200_stage_name(int i);
 
 /* ---- page-locked host memory for the host-buffer entry points (rx_batch, rx_push*, tx) ----
- * cudaHostAlloc'd, so copies are plain DMA, and first touched from the host cores on the GPU's side of the machine
+ * cudaHostAlloc'd, so copies are plain DMA, and zero-filled from the host cores on the GPU's side of the machine
  * (/sys/bus/pci/devices/<gpu>/local_cpulist): on a multi-socket box the pages land on the NUMA node of the GPU's PCIe root. */
 int  wifi_b200_host_alloc(wifi_b200_t *h, size_t bytes, void **out);
 int  wifi_b200_host_free(wifi_b200_t *h, void *p);

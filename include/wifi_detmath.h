@@ -126,6 +126,30 @@ WDM_FN void wdm_sincosf(float x, float *s, float *c)
     *c = co;
 }
 
+/* sin and cos of 2*pi*p/2^32: a phase in turns held as an unsigned 32-bit integer (the accumulator of a numerically
+ * controlled oscillator).  The quadrant comes from the top bits and the remainder is a signed offset in [-pi/4, pi/4),
+ * so no Cody-Waite step is needed and the error is below 3e-7 absolute for every phase.  The polynomials and the
+ * quadrant swap are wdm_sincosf's; they are written out again because sharing them through a helper reschedules the
+ * receiver kernels that call wdm_sincosf. */
+WDM_FN void wdm_sincos_turn(uint32_t p, float *s, float *c)
+{
+    const uint32_t q = (p + 0x20000000u) >> 30;                                  /* nearest quarter turn, 0..3 */
+    const float r = (float)(int32_t)(p - (q << 30)) * 1.46291807926715968e-9f;   /* x 2 pi / 2^32 */
+    float z = r * r;
+    float ps = fmaf(z, -1.9515295891e-4f, 8.3321608736e-3f);
+    ps = fmaf(ps, z, -1.6666654611e-1f);
+    float sr = fmaf(ps * z, r, r);
+    float pc = fmaf(z, 2.443315711809948e-5f, -1.388731625493765e-3f);
+    pc = fmaf(pc, z, 4.166664568298827e-2f);
+    float cr = fmaf(pc * z, z, fmaf(z, -0.5f, 1.0f));
+    float so = (q & 1) ? cr : sr;
+    float co = (q & 1) ? sr : cr;
+    if (q & 2) so = -so;
+    if ((q + 1) & 2) co = -co;
+    *s = so;
+    *c = co;
+}
+
 /* atan2(y, x) in (-pi, pi].  atan2(0,0) = 0.  NaN inputs give NaN.
  * One division and no branches: with mn = min(|x|,|y|), mx = max(|x|,|y|) the angle of (mx, mn) lies in [0, pi/4];
  * above tan(pi/8) it is pi/4 + atan((mn - mx)/(mn + mx)), so the argument of the polynomial is formed as a quotient of
@@ -214,10 +238,76 @@ WDM_FN void wdm_box_muller(uint32_t w0, uint32_t w1, float *z0, float *z1)
     *z1 = rad * s;
 }
 
+/* ---- time-varying multipath fading: a sum of sinusoids per tap (DESIGN.md "fading channel") ----
+ * Tap t of a realisation is  h_t(n) = sum_{m < n_sin} w_{t,m} exp(j 2 pi f_{t,m} n)  (+ the line-of-sight term on tap 0)
+ * with w ~ CN(0, P_t / n_sin) and f_{t,m} = doppler cos(2 pi (m + u_{t,m}) / n_sin), u ~ U[0,1): given the frequencies the
+ * tap is complex Gaussian at every n, and over realisations its autocorrelation is Clarke's J0(2 pi doppler tau).  Phases
+ * are 32-bit NCO phases fq * n (mod 2^32), exact for every n, so the process is periodic in 2^32 samples.
+ * The draws come from Philox with key = seed and counter (16 t + m, 0xFFFFFFFF, stream): word 1 of an AWGN counter is the
+ * high half of a non-negative sample index and never 0xFFFFFFFF, so the fading and the noise of one key are independent. */
+typedef struct wdm_fade_ent { float re, im; uint32_t fq, pad; } wdm_fade_ent;   /* weight w and NCO increment of one term */
+
+/* cycles/sample -> NCO phase increment per sample; |f| <= 0.25 keeps rintf(f 2^32) inside int32 */
+WDM_FN uint32_t wdm_nco_freq(float f) { return (uint32_t)(int32_t)rintf(f * 4294967296.0f); }
+
+/* Term m of tap t of the realisation (seed, stream).  m < n_sin: scatter sinusoid m, with power E|w|^2 = P / n_sin, or
+ * on tap 0 P / (n_sin (k + 1)) (Rician K = k).  m == n_sin, tap 0, k > 0 only: the line-of-sight term
+ * sqrt(P k / (k + 1)) exp(j (2 pi los_doppler n + phi)), phi from its own counter (128, 0xFFFFFFFF, stream). */
+WDM_FN wdm_fade_ent wdm_fading_entry(uint64_t seed, uint64_t stream, int t, int m, int n_sin, float power, float k,
+                                     float doppler, float los_doppler)
+{
+    wdm_fade_ent e;
+    uint32_t r[4];
+    float s, c;
+    wdm_philox4x32(m < n_sin ? (uint32_t)(16 * t + m) : 128u, 0xFFFFFFFFu, (uint32_t)stream, (uint32_t)(stream >> 32),
+                   (uint32_t)seed, (uint32_t)(seed >> 32), r);
+    if (m < n_sin) {
+        const float kk = t == 0 ? k : 0.0f;
+        const float amp = sqrtf(power / ((float)n_sin * (kk + 1.0f))) * 0.70710678f;   /* per component of CN(0, 1) */
+        float z0, z1;
+        wdm_box_muller(r[0], r[1], &z0, &z1);
+        e.re = amp * z0;
+        e.im = amp * z1;
+        /* angle (m + u) / n_sin turns with u = (r2 >> 8) / 2^24, as a 32-bit phase: an exact integer division */
+        const uint32_t p = (uint32_t)((((uint64_t)m << 32) | (r[2] & 0xFFFFFF00u)) / (uint64_t)n_sin);
+        wdm_sincos_turn(p, &s, &c);
+        e.fq = wdm_nco_freq(doppler * c);
+    } else {
+        const float amp = sqrtf(power * k / (k + 1.0f));
+        wdm_sincos_turn(r[0], &s, &c);
+        e.re = amp * c;
+        e.im = amp * s;
+        e.fq = wdm_nco_freq(los_doppler);
+    }
+    e.pad = 0u;
+    return e;
+}
+
+/* acc + w exp(j 2 pi fq n / 2^32): one term of a tap at sample n */
+WDM_FN wdm_cf wdm_fading_step(wdm_cf acc, wdm_fade_ent e, uint32_t n)
+{
+    wdm_cf w, g;
+    wdm_sincos_turn(e.fq * n, &w.im, &w.re);
+    g.re = e.re;
+    g.im = e.im;
+    return wdm_cmac(acc, g, w);
+}
+
+/* h_t(n): the terms of one tap summed in ascending order */
+WDM_FN wdm_cf wdm_fading_tap(const wdm_fade_ent *e, int cnt, uint32_t n)
+{
+    wdm_cf h;
+    h.re = 0.0f;
+    h.im = 0.0f;
+    for (int k = 0; k < cnt; ++k) h = wdm_fading_step(h, e[k], n);
+    return h;
+}
+
 /* ---- self-test dispatch: one element of tests/test_detmath.py (host: orc_detmath, device: wifi_b200_selftest_detmath).
  * o0/o1 are in-out (the accumulator of the multiply-accumulate forms). ---- */
 enum { WDM_T_SINCOS = 0, WDM_T_ATAN2, WDM_T_LOG, WDM_T_CMUL, WDM_T_CMULC, WDM_T_CDIV, WDM_T_BOX_MULLER, WDM_T_CMAC,
-       WDM_T_CMACC, WDM_T_CMSUBC, WDM_T_NORM_ADD, WDM_T_NORM_SUB, WDM_T_PHILOX, WDM_T_COUNT };
+       WDM_T_CMACC, WDM_T_CMSUBC, WDM_T_NORM_ADD, WDM_T_NORM_SUB, WDM_T_PHILOX, WDM_T_SINCOS_TURN, WDM_T_FADING_ENTRY,
+       WDM_T_FADING_FREQ, WDM_T_FADING_STEP, WDM_T_COUNT };
 WDM_FN void wdm_selftest(int fn, float a, float b, float c, float d, float *o0, float *o1)
 {
     wdm_cf x, y, acc, r;
@@ -242,6 +332,28 @@ WDM_FN void wdm_selftest(int fn, float a, float b, float c, float d, float *o0, 
         wdm_philox4x32(ua.u, ub.u, 0u, 0u, uc.u, ud.u, w);
         ua.u = w[0] ^ w[2]; ub.u = w[1] ^ w[3];
         *o0 = ua.f; *o1 = ub.f;
+        break;
+    }
+    case WDM_T_SINCOS_TURN: wdm_sincos_turn(ua.u, o0, o1); break;                /* a carries the phase */
+    case WDM_T_FADING_ENTRY:     /* a, b: bits of seed, stream; c: doppler (-c: LoS doppler); d: bits t | m << 4 | (n_sin - 1) << 12;  */
+    case WDM_T_FADING_FREQ: {    /* in: o0 = power, o1 = k.  ENTRY: o0, o1 = weight; FREQ: o0 = bits of fq, o1 = 0               */
+        const wdm_fade_ent e = wdm_fading_entry(ua.u, ub.u, (int)(ud.u & 7u), (int)((ud.u >> 4) & 31u), (int)((ud.u >> 12) & 15u) + 1,
+                                                *o0, *o1, c, -c);
+        if (fn == WDM_T_FADING_ENTRY) {
+            *o0 = e.re;
+            *o1 = e.im;
+        } else {
+            ua.u = e.fq;
+            *o0 = ua.f;
+            *o1 = 0.0f;
+        }
+        break;
+    }
+    case WDM_T_FADING_STEP: {    /* a, b: weight; c, d: bits of fq and n; o0, o1: accumulator */
+        wdm_fade_ent e;
+        e.re = a; e.im = b; e.fq = uc.u; e.pad = 0u;
+        r = wdm_fading_step(acc, e, ud.u);
+        *o0 = r.re; *o1 = r.im;
         break;
     }
     default: break;
