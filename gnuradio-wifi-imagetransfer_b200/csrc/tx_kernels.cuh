@@ -124,19 +124,21 @@ __global__ void __launch_bounds__(128) k_tx(const uint8_t *__restrict__ psdu_blo
     }
 }
 
-// synthetic channel, mirrors oracle channel(): taps, gain, CFO rotation, Philox AWGN
-__global__ void __launch_bounds__(256) k_channel(const cf *__restrict__ in, cf *__restrict__ out, const wifi_b200_chan_seg *__restrict__ segs, int n_segs)
+// synthetic channel, mirrors the oracle's channel(): y(i) = gain * sum_t tap(t, t0 + i) * x(i - delay[t]), then the CFO
+// rotation and Philox AWGN at counter n0 + i.  One grid row per segment.  tap(t, n) is tap t's coefficient at time n
+// (a 32-bit NCO time, computed once per sample here; the fixed taps ignore it).
+template <class Tap>
+__device__ __forceinline__ void channel_body(const cf *__restrict__ in, cf *__restrict__ out, const wifi_b200_chan_seg &S, int n_taps,
+                                             const int32_t *delay, int64_t t0, Tap tap)
 {
-    const int sidx = blockIdx.y;
-    if (sidx >= n_segs) return;
-    const wifi_b200_chan_seg S = segs[sidx];
     const float ns = S.noise_sigma * 0.70710678f;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < S.n; i += (int64_t)gridDim.x * blockDim.x) {
+        const uint32_t n = (uint32_t)(t0 + i);
         cf acc = {0.f, 0.f};
-        for (int t = 0; t < S.n_taps; ++t) {
-            int64_t j = i - S.delay[t];
+        for (int t = 0; t < n_taps; ++t) {
+            int64_t j = i - delay[t];
             if (j < 0 || j >= S.in_len) continue;
-            acc = wdm_cmac(acc, cf{S.tap_re[t], S.tap_im[t]}, in[S.in_off + j]);
+            acc = wdm_cmac(acc, tap(t, n), in[S.in_off + j]);
         }
         acc = cscale(acc, S.gain);
         cf w = crot(S.cfo * (float)i + S.phase0);
@@ -155,10 +157,18 @@ __global__ void __launch_bounds__(256) k_channel(const cf *__restrict__ in, cf *
     }
 }
 
-// time-varying fading channel (wifi_b200_channel_fading_dev), mirrors tests/fading_oracle.cpp: the taps of k_channel become
-// h_t(t0 + i) of include/wifi_detmath.h; gain, CFO rotation and Philox AWGN are k_channel's.  The block first draws its
-// segment's terms into shared memory (tap t at slots t * FADE_SLOTS ..; tap 0's line-of-sight term follows its n_sin
-// sinusoids), then every sample evaluates one NCO sincos and one complex multiply-accumulate per term.
+// fixed taps (wifi_b200_channel_dev)
+__global__ void __launch_bounds__(256) k_channel(const cf *__restrict__ in, cf *__restrict__ out, const wifi_b200_chan_seg *__restrict__ segs, int n_segs)
+{
+    const int sidx = blockIdx.y;
+    if (sidx >= n_segs) return;
+    const wifi_b200_chan_seg S = segs[sidx];
+    channel_body(in, out, S, S.n_taps, S.delay, 0, [&](int t, uint32_t) { return cf{S.tap_re[t], S.tap_im[t]}; });
+}
+
+// time-varying fading channel (wifi_b200_channel_fading_dev): the taps are h_t(t0 + i) of include/wifi_detmath.h.  The
+// block first draws its segment's terms into shared memory (tap t at slots t * FADE_SLOTS ..; tap 0's line-of-sight term
+// follows its n_sin sinusoids), then every sample evaluates one NCO sincos and one complex multiply-accumulate per term.
 #define FADE_SLOTS 17
 __global__ void __launch_bounds__(256) k_channel_fading(const cf *__restrict__ in, cf *__restrict__ out, const wifi_b200_chan_seg *__restrict__ segs,
                                                         const wifi_b200_fading *__restrict__ fades, int n_segs)
@@ -175,28 +185,6 @@ __global__ void __launch_bounds__(256) k_channel_fading(const cf *__restrict__ i
             ent[k] = wdm_fading_entry(F.seed, F.stream, t, m, F.n_sin, F.power[t], F.k_factor, F.doppler, F.los_doppler);
     }
     __syncthreads();
-    const float ns = S.noise_sigma * 0.70710678f;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < S.n; i += (int64_t)gridDim.x * blockDim.x) {
-        const uint32_t n = (uint32_t)(F.t0 + i);
-        cf acc = {0.f, 0.f};
-        for (int t = 0; t < F.n_taps; ++t) {
-            int64_t j = i - F.delay[t];
-            if (j < 0 || j >= S.in_len) continue;
-            acc = wdm_cmac(acc, wdm_fading_tap(ent + t * FADE_SLOTS, t == 0 ? cnt0 : F.n_sin, n), in[S.in_off + j]);
-        }
-        acc = cscale(acc, S.gain);
-        cf w = crot(S.cfo * (float)i + S.phase0);
-        cf y = cmul(acc, w);
-        if (S.noise_sigma > 0.f) {
-            uint64_t idx = (uint64_t)(S.n0 + i);
-            uint32_t r[4];
-            wdm_philox4x32((uint32_t)idx, (uint32_t)(idx >> 32), (uint32_t)S.stream, (uint32_t)(S.stream >> 32),
-                           (uint32_t)S.seed, (uint32_t)(S.seed >> 32), r);
-            float z0, z1;
-            wdm_box_muller(r[0], r[1], &z0, &z1);
-            y.re = y.re + ns * z0;
-            y.im = y.im + ns * z1;
-        }
-        out[S.out_off + i] = y;
-    }
+    channel_body(in, out, S, F.n_taps, F.delay, F.t0,
+                 [&](int t, uint32_t n) { return wdm_fading_tap(ent + t * FADE_SLOTS, t == 0 ? cnt0 : F.n_sin, n); });
 }

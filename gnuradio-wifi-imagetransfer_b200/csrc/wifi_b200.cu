@@ -211,13 +211,12 @@ struct wifi_b200 {
     TxFrameDesc *d_txdesc = nullptr;
     uint8_t *d_txsym = nullptr;
     cf *d_txiq = nullptr;
-    size_t txblob_cap = 0, txiq_cap = 0, txsym_cap = 0;
+    size_t txblob_cap = 0, txiq_cap = 0, txsym_cap = 0;   // bytes, as every capacity grow() keeps
     int64_t tx_sym_bytes = 0;
     int tx_seed = 1;               // [UPSTREAM] mapper.cc d_scrambler: 1, ++ per frame, wraps after 127
     wifi_b200_chan_seg *d_segs = nullptr;
-    int segs_cap = 0;
     wifi_b200_fading *d_fades = nullptr;
-    int fades_cap = 0;
+    size_t segs_cap = 0, fades_cap = 0;
     // last rx call
     const cf *cur_iq = nullptr;
     std::vector<LinkDesc> h_links;
@@ -322,6 +321,19 @@ void free_all(wifi_b200 *h)
     if (h->d2h_stream) cudaStreamDestroy(h->d2h_stream);
     if (h->aux_stream) cudaStreamDestroy(h->aux_stream);
     if (h->stream) cudaStreamDestroy(h->stream);
+}
+
+// Grows the handle buffer *p to hold need bytes, with slack bytes to spare; what it held is not kept.  A failed
+// allocation leaves *p null and *cap 0, so the next call allocates again.
+int grow(wifi_b200 *h, void **p, size_t *cap, size_t need, size_t slack)
+{
+    if (need <= *cap) return WIFI_OK;
+    if (*p) cudaFree(*p);
+    *p = nullptr;
+    *cap = 0;
+    CK(cudaMalloc(p, need + slack));
+    *cap = need + slack;
+    return WIFI_OK;
 }
 
 int ensure_soft(wifi_b200 *h)
@@ -967,29 +979,12 @@ static int64_t tx_common(wifi_b200_t *h, const uint8_t *blob, const uint32_t *of
     if (burst_off) burst_off[n] = pos;
     if (pos > cap) { h->err = "iq_out too small"; return WIFI_E_OVERFLOW; }
     if (!seed) h->tx_seed = seedc;
-    if (blob_bytes > h->txblob_cap) {
-        if (h->d_txblob) cudaFree(h->d_txblob);
-        h->d_txblob = nullptr;
-        CK(cudaMalloc(&h->d_txblob, blob_bytes + 1024));
-        h->txblob_cap = blob_bytes + 1024;
-    }
+    int rc = grow(h, (void **)&h->d_txblob, &h->txblob_cap, blob_bytes, 1024);
+    if (rc == WIFI_OK) rc = grow(h, (void **)&h->d_txsym, &h->txsym_cap, spos, 1024);
+    if (rc == WIFI_OK && !out_is_dev) rc = grow(h, (void **)&h->d_txiq, &h->txiq_cap, pos * sizeof(cf), 1024 * sizeof(cf));
+    if (rc != WIFI_OK) return rc;
     if (!h->d_txdesc) CK(cudaMalloc(&h->d_txdesc, (size_t)h->cfg.max_frames * sizeof(TxFrameDesc)));
-    if (spos > h->txsym_cap) {
-        if (h->d_txsym) cudaFree(h->d_txsym);
-        h->d_txsym = nullptr;
-        CK(cudaMalloc(&h->d_txsym, spos + 1024));
-        h->txsym_cap = spos + 1024;
-    }
-    cf *dst = (cf *)iq_out;
-    if (!out_is_dev) {
-        if (pos > h->txiq_cap) {
-            if (h->d_txiq) cudaFree(h->d_txiq);
-            h->d_txiq = nullptr;
-            CK(cudaMalloc(&h->d_txiq, (pos + 1024) * sizeof(cf)));
-            h->txiq_cap = pos + 1024;
-        }
-        dst = h->d_txiq;
-    }
+    cf *dst = out_is_dev ? (cf *)iq_out : h->d_txiq;
     cudaStream_t s = h->stream;
     CK(cudaMemcpyAsync(h->d_txblob, blob, blob_bytes, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(h->d_txdesc, descs.data(), n * sizeof(TxFrameDesc), cudaMemcpyHostToDevice, s));
@@ -1021,141 +1016,115 @@ int64_t wifi_b200_tx_symbols(wifi_b200_t *h, uint8_t *out, size_t cap)
     return h->tx_sym_bytes;
 }
 
-int wifi_b200_channel_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, const wifi_b200_chan_seg *segs, int n_segs)
-{
-    if (!h || !in_dev || !out_dev || !segs || n_segs <= 0) return WIFI_E_ARG;
-    std::lock_guard<std::mutex> g(h->mu);
-    cudaSetDevice(h->device);
-    int64_t maxn = 0;
-    for (int i = 0; i < n_segs; ++i) {
-        if (segs[i].n_taps < 0 || segs[i].n_taps > 8 || segs[i].n < 0) { h->err = "bad channel segment"; return WIFI_E_ARG; }
-        maxn = std::max(maxn, segs[i].n);
-    }
-    if (n_segs > h->segs_cap) {
-        if (h->d_segs) cudaFree(h->d_segs);
-        h->d_segs = nullptr;
-        CK(cudaMalloc(&h->d_segs, (size_t)(n_segs + 64) * sizeof(wifi_b200_chan_seg)));
-        h->segs_cap = n_segs + 64;
-    }
-    CK(cudaMemcpyAsync(h->d_segs, segs, (size_t)n_segs * sizeof(wifi_b200_chan_seg), cudaMemcpyHostToDevice, h->stream));
-    for (int base = 0; base < n_segs; base += 65535) {
-        int cnt = std::min(65535, n_segs - base);
-        dim3 grid((unsigned)std::min<int64_t>((maxn + 255) / 256, 4096), cnt);
-        if (grid.x == 0) grid.x = 1;
-        k_channel<<<grid, 256, 0, h->stream>>>((const cf *)in_dev, (cf *)out_dev, h->d_segs + base, cnt);
-    }
-    CK(cudaGetLastError());
-    CK(cudaStreamSynchronize(h->stream));
-    return WIFI_OK;
-}
-
-// host-buffer form of the test channel: stages in/out through the handle's device buffers
-int wifi_b200_channel(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
-                      const wifi_b200_chan_seg *segs, int n_segs)
-{
-    if (!h || !in_host || !out_host || in_len <= 0 || out_len <= 0) return WIFI_E_ARG;
-    cf *d_in = nullptr, *d_out = nullptr;
-    {
-        std::lock_guard<std::mutex> g(h->mu);
-        cudaSetDevice(h->device);
-        CK(cudaMalloc(&d_in, (size_t)in_len * sizeof(cf)));
-        if (cudaMalloc(&d_out, (size_t)out_len * sizeof(cf)) != cudaSuccess) { cudaFree(d_in); h->err = "cudaMalloc"; return WIFI_E_NOMEM; }
-        cudaMemcpy(d_in, in_host, (size_t)in_len * sizeof(cf), cudaMemcpyHostToDevice);
-        cudaMemset(d_out, 0, (size_t)out_len * sizeof(cf));
-    }
-    for (int i = 0; i < n_segs; ++i)
-        if (segs[i].in_off < 0 || segs[i].in_off + segs[i].in_len > in_len || segs[i].out_off < 0 || segs[i].out_off + segs[i].n > out_len) {
-            cudaFree(d_in); cudaFree(d_out);
-            h->err = "channel segment outside the buffers";
-            return WIFI_E_ARG;
-        }
-    int rc = wifi_b200_channel_dev(h, (const float *)d_in, (float *)d_out, segs, n_segs);
-    if (rc == WIFI_OK) {
-        std::lock_guard<std::mutex> g(h->mu);
-        if (cudaMemcpy(out_host, d_out, (size_t)out_len * sizeof(cf), cudaMemcpyDeviceToHost) != cudaSuccess) rc = WIFI_E_CUDA;
-    }
-    cudaFree(d_in);
-    cudaFree(d_out);
-    return rc;
-}
-
 static bool fading_ok(const wifi_b200_chan_seg &s, const wifi_b200_fading &f)
 {
-    if (s.n_taps != 0 || s.n < 0 || f.n_taps < 1 || f.n_taps > 8 || f.n_sin < 1 || f.n_sin > 16) return false;
+    if (s.n_taps != 0 || f.n_taps < 1 || f.n_taps > 8 || f.n_sin < 1 || f.n_sin > 16) return false;
     if (!(f.k_factor >= 0.f && f.k_factor <= FLT_MAX) || !(f.doppler >= 0.f && f.doppler <= 0.25f) || !(fabsf(f.los_doppler) <= 0.25f)) return false;
     for (int t = 0; t < f.n_taps; ++t)
         if (f.delay[t] < 0 || !(f.power[t] >= 0.f && f.power[t] <= FLT_MAX)) return false;
     return true;
 }
 
-int wifi_b200_channel_fading_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, const wifi_b200_chan_seg *segs,
-                                 const wifi_b200_fading *fades, int n_segs)
+// The argument check of the four channel entry points, made before anything is allocated or written.  fades == nullptr
+// selects the fixed taps.  in_len / out_len are the lengths of host buffers, which every segment must lie inside; device
+// buffers (in_len == 0) are the caller's to size.
+static int check_channel(wifi_b200 *h, const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs, int64_t in_len, int64_t out_len)
 {
-    if (!h || !in_dev || !out_dev || !segs || !fades || n_segs <= 0) return WIFI_E_ARG;
-    std::lock_guard<std::mutex> g(h->mu);
-    cudaSetDevice(h->device);
-    int64_t maxn = 0;
+    if (!segs || n_segs <= 0) { h->err = "no channel segments"; return WIFI_E_ARG; }
     for (int i = 0; i < n_segs; ++i) {
-        if (!fading_ok(segs[i], fades[i])) { h->err = "bad fading channel segment"; return WIFI_E_ARG; }
-        maxn = std::max(maxn, segs[i].n);
+        const wifi_b200_chan_seg &s = segs[i];
+        if (s.n < 0 || s.in_len < 0 || (fades ? !fading_ok(s, fades[i]) : (s.n_taps < 0 || s.n_taps > 8))) {
+            h->err = fades ? "bad fading channel segment" : "bad channel segment";
+            return WIFI_E_ARG;
+        }
+        if (in_len && (s.in_off < 0 || s.in_off + s.in_len > in_len || s.out_off < 0 || s.out_off + s.n > out_len)) {
+            h->err = "channel segment outside the buffers";
+            return WIFI_E_ARG;
+        }
     }
-    if (n_segs > h->segs_cap) {
-        if (h->d_segs) cudaFree(h->d_segs);
-        h->d_segs = nullptr;
-        CK(cudaMalloc(&h->d_segs, (size_t)(n_segs + 64) * sizeof(wifi_b200_chan_seg)));
-        h->segs_cap = n_segs + 64;
-    }
-    if (n_segs > h->fades_cap) {
-        if (h->d_fades) cudaFree(h->d_fades);
-        h->d_fades = nullptr;
-        CK(cudaMalloc(&h->d_fades, (size_t)(n_segs + 64) * sizeof(wifi_b200_fading)));
-        h->fades_cap = n_segs + 64;
-    }
+    return WIFI_OK;
+}
+
+// Runs checked segments through k_channel, or k_channel_fading when fades is given, in launches of at most 65535 grid
+// rows (one segment per row).  The caller holds h->mu and has made h->device current.
+static int run_channel(wifi_b200 *h, const cf *in_dev, cf *out_dev, const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs)
+{
+    int64_t maxn = 0;
+    for (int i = 0; i < n_segs; ++i) maxn = std::max(maxn, segs[i].n);
+    int rc = grow(h, (void **)&h->d_segs, &h->segs_cap, (size_t)n_segs * sizeof(wifi_b200_chan_seg), 64 * sizeof(wifi_b200_chan_seg));
+    if (rc == WIFI_OK && fades) rc = grow(h, (void **)&h->d_fades, &h->fades_cap, (size_t)n_segs * sizeof(wifi_b200_fading), 64 * sizeof(wifi_b200_fading));
+    if (rc != WIFI_OK) return rc;
     CK(cudaMemcpyAsync(h->d_segs, segs, (size_t)n_segs * sizeof(wifi_b200_chan_seg), cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(h->d_fades, fades, (size_t)n_segs * sizeof(wifi_b200_fading), cudaMemcpyHostToDevice, h->stream));
+    if (fades) CK(cudaMemcpyAsync(h->d_fades, fades, (size_t)n_segs * sizeof(wifi_b200_fading), cudaMemcpyHostToDevice, h->stream));
     for (int base = 0; base < n_segs; base += 65535) {
         int cnt = std::min(65535, n_segs - base);
         dim3 grid((unsigned)std::min<int64_t>((maxn + 255) / 256, 4096), cnt);
         if (grid.x == 0) grid.x = 1;
-        k_channel_fading<<<grid, 256, 0, h->stream>>>((const cf *)in_dev, (cf *)out_dev, h->d_segs + base, h->d_fades + base, cnt);
+        if (fades) k_channel_fading<<<grid, 256, 0, h->stream>>>(in_dev, out_dev, h->d_segs + base, h->d_fades + base, cnt);
+        else k_channel<<<grid, 256, 0, h->stream>>>(in_dev, out_dev, h->d_segs + base, cnt);
     }
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(h->stream));
     return WIFI_OK;
 }
 
-// host-buffer form of the fading channel, staged as wifi_b200_channel stages
-int wifi_b200_channel_fading(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
-                             const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs)
+static int channel_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs)
 {
-    if (!h || !in_host || !out_host || !segs || !fades || in_len <= 0 || out_len <= 0 || n_segs <= 0) return WIFI_E_ARG;
-    for (int i = 0; i < n_segs; ++i)
-        if (segs[i].in_off < 0 || segs[i].in_len < 0 || segs[i].in_off + segs[i].in_len > in_len || segs[i].out_off < 0 ||
-            segs[i].n < 0 || segs[i].out_off + segs[i].n > out_len) {
-            h->err = "channel segment outside the buffers";
-            return WIFI_E_ARG;
-        }
+    if (!h || !in_dev || !out_dev) return WIFI_E_ARG;
+    std::lock_guard<std::mutex> g(h->mu);
+    int rc = check_channel(h, segs, fades, n_segs, 0, 0);
+    if (rc != WIFI_OK) return rc;
+    cudaSetDevice(h->device);
+    return run_channel(h, (const cf *)in_dev, (cf *)out_dev, segs, fades, n_segs);
+}
+
+// host-buffer forms: stage in/out through temporary device buffers; out is zero where no segment writes
+static int channel_host(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
+                        const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs)
+{
+    if (!h || !in_host || !out_host || in_len <= 0 || out_len <= 0) return WIFI_E_ARG;
+    std::lock_guard<std::mutex> g(h->mu);
+    int rc = check_channel(h, segs, fades, n_segs, in_len, out_len);
+    if (rc != WIFI_OK) return rc;
+    cudaSetDevice(h->device);
     cf *d_in = nullptr, *d_out = nullptr;
-    {
-        std::lock_guard<std::mutex> g(h->mu);
-        cudaSetDevice(h->device);
-        CK(cudaMalloc(&d_in, (size_t)in_len * sizeof(cf)));
-        if (cudaMalloc(&d_out, (size_t)out_len * sizeof(cf)) != cudaSuccess) { cudaFree(d_in); h->err = "cudaMalloc"; return WIFI_E_NOMEM; }
-        if (cudaMemcpy(d_in, in_host, (size_t)in_len * sizeof(cf), cudaMemcpyHostToDevice) != cudaSuccess ||
-            cudaMemset(d_out, 0, (size_t)out_len * sizeof(cf)) != cudaSuccess) {
-            cudaFree(d_in); cudaFree(d_out);
-            h->err = "channel staging copy";
-            return WIFI_E_CUDA;
-        }
-    }
-    int rc = wifi_b200_channel_fading_dev(h, (const float *)d_in, (float *)d_out, segs, fades, n_segs);
-    if (rc == WIFI_OK) {
-        std::lock_guard<std::mutex> g(h->mu);
-        if (cudaMemcpy(out_host, d_out, (size_t)out_len * sizeof(cf), cudaMemcpyDeviceToHost) != cudaSuccess) rc = WIFI_E_CUDA;
+    CK(cudaMalloc(&d_in, (size_t)in_len * sizeof(cf)));
+    if (cudaMalloc(&d_out, (size_t)out_len * sizeof(cf)) != cudaSuccess) { cudaFree(d_in); h->err = "cudaMalloc"; return WIFI_E_NOMEM; }
+    if (cudaMemcpy(d_in, in_host, (size_t)in_len * sizeof(cf), cudaMemcpyHostToDevice) != cudaSuccess ||
+        cudaMemset(d_out, 0, (size_t)out_len * sizeof(cf)) != cudaSuccess) {
+        h->err = "channel staging copy";
+        rc = WIFI_E_CUDA;
+    } else if ((rc = run_channel(h, d_in, d_out, segs, fades, n_segs)) == WIFI_OK &&
+               cudaMemcpy(out_host, d_out, (size_t)out_len * sizeof(cf), cudaMemcpyDeviceToHost) != cudaSuccess) {
+        h->err = "channel staging copy";
+        rc = WIFI_E_CUDA;
     }
     cudaFree(d_in);
     cudaFree(d_out);
     return rc;
+}
+
+int wifi_b200_channel_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, const wifi_b200_chan_seg *segs, int n_segs)
+{
+    return channel_dev(h, in_dev, out_dev, segs, nullptr, n_segs);
+}
+
+int wifi_b200_channel(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
+                      const wifi_b200_chan_seg *segs, int n_segs)
+{
+    return channel_host(h, in_host, in_len, out_host, out_len, segs, nullptr, n_segs);
+}
+
+int wifi_b200_channel_fading_dev(wifi_b200_t *h, const float *in_dev, float *out_dev, const wifi_b200_chan_seg *segs,
+                                 const wifi_b200_fading *fades, int n_segs)
+{
+    return fades ? channel_dev(h, in_dev, out_dev, segs, fades, n_segs) : WIFI_E_ARG;
+}
+
+int wifi_b200_channel_fading(wifi_b200_t *h, const float *in_host, int64_t in_len, float *out_host, int64_t out_len,
+                             const wifi_b200_chan_seg *segs, const wifi_b200_fading *fades, int n_segs)
+{
+    return fades ? channel_host(h, in_host, in_len, out_host, out_len, segs, fades, n_segs) : WIFI_E_ARG;
 }
 
 int wifi_b200_rx_batch_dev(wifi_b200_t *h, const float *iq_dev, const uint64_t *link_off, int n_links, int final)
@@ -1541,13 +1510,9 @@ static int push_async(wifi_b200 *h, const void *iq, size_t bytes_per_sample, flo
     if (h->a_pending.size() >= A_SLOTS) { h->err = "three asynchronous pushes are already pending: call wifi_b200_rx_push_wait first"; return WIFI_E_OVERFLOW; }
     if (total > h->cfg.max_samples) { h->err = "push larger than max_samples"; return WIFI_E_OVERFLOW; }
     const int slot = h->a_next % A_SLOTS;
-    if ((int64_t)h->a_cap[slot] < total) {        // slots are sized in fc32 samples: either format fits
-        if (h->d_stage[slot]) cudaFree(h->d_stage[slot]);
-        h->d_stage[slot] = nullptr;
-        h->a_cap[slot] = 0;
-        CK(cudaMalloc(&h->d_stage[slot], (size_t)(total + 64) * sizeof(cf)));
-        h->a_cap[slot] = (size_t)total + 64;
-    }
+    // slots are sized in fc32 samples: either format fits
+    int rc = grow(h, (void **)&h->d_stage[slot], &h->a_cap[slot], (size_t)total * sizeof(cf), 64 * sizeof(cf));
+    if (rc != WIFI_OK) return rc;
     if (!h->a_ev[slot]) CK(cudaEventCreateWithFlags(&h->a_ev[slot], cudaEventDisableTiming));
     wifi_b200::AsyncPush job;
     job.slot = slot;

@@ -33,6 +33,13 @@ class ChanCfg(C.Structure):
                 ("seed", C.c_uint64), ("stream", C.c_uint64)]
 
 
+class FadingCfg(C.Structure):
+    """Same layout and meaning as wifi_b200_fading (include/wifi_b200.h)."""
+    _fields_ = [("n_taps", C.c_int32), ("n_sin", C.c_int32), ("delay", C.c_int32 * 8), ("power", C.c_float * 8),
+                ("k_factor", C.c_float), ("doppler", C.c_float), ("los_doppler", C.c_float), ("reserved", C.c_int32),
+                ("t0", C.c_int64), ("seed", C.c_uint64), ("stream", C.c_uint64)]
+
+
 def build(force=False):
     so = os.path.join(_HERE, "liboracle.so")
     srcs = [os.path.join(_HERE, "wifi_oracle.cpp"), os.path.join(_HERE, "wifi_oracle.h"),
@@ -222,11 +229,35 @@ def chan_cfg(gain=1.0, cfo=0.0, phase0=0.0, noise_sigma=0.0, taps=((0, 1.0 + 0j)
     return c
 
 
-def channel(x, n0=0, **kw):
+def fading_cfg(taps=((0, 1.0),), n_sin=8, k_factor=0.0, doppler=0.0, los_doppler=0.0, t0=0, seed=0, stream=0):
+    """taps = ((delay, power), ...); the rest as wifi_b200_fading."""
+    f = FadingCfg()
+    f.n_taps, f.n_sin = len(taps), n_sin
+    for i, (d, p) in enumerate(taps):
+        f.delay[i], f.power[i] = int(d), float(p)
+    f.k_factor, f.doppler, f.los_doppler = k_factor, doppler, los_doppler
+    f.t0, f.seed, f.stream = t0, seed, stream
+    return f
+
+
+def channel(x, n0=0, fading=None, **kw):
+    """Gain, taps, CFO rotation and Philox AWGN keyed by seed / stream at counter n0 + i (keywords of chan_cfg).
+    fading: the time-varying taps instead of the fixed ones, as a FadingCfg, a FADING_DTYPE record or a dict of
+    fading_cfg keywords; out-of-range parameters raise ValueError."""
     a = np.ascontiguousarray(x, np.complex64)
     o = np.empty_like(a)
-    cfg = kw.pop("cfg", None) or chan_cfg(**kw)
-    lib().orc_channel(_p(a), _p(o), C.c_int64(a.size), C.c_int64(n0), C.byref(cfg))
+    if fading is None:
+        cfg = kw.pop("cfg", None) or chan_cfg(**kw)
+        lib().orc_channel(_p(a), _p(o), C.c_int64(a.size), C.c_int64(n0), C.byref(cfg))
+        return o
+    if isinstance(fading, dict):
+        fading = fading_cfg(**fading)
+    elif isinstance(fading, np.ndarray):
+        fading = FadingCfg.from_buffer_copy(np.ascontiguousarray(fading).tobytes())
+    kw.setdefault("taps", ())
+    cfg = chan_cfg(**kw)
+    if lib().orc_channel_fading(_p(a), _p(o), C.c_int64(a.size), C.c_int64(n0), C.byref(cfg), C.byref(fading)):
+        raise ValueError("fading parameters out of range")
     return o
 
 

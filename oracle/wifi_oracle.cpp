@@ -525,15 +525,17 @@ static int depuncture(const uint8_t *in, int n_in, int enc, uint8_t *out)
 }
 
 /* ----------------------------------------------------------------- channel */
-static void channel(const cf *in, cf *out, int64_t n, int64_t n0, const orc_chan_cfg &c)
+/* y(i) = gain * sum_t tap(t, i) * x(i - delay[t]), then the CFO rotation and Philox AWGN at counter n0 + i */
+template <class Tap>
+static void channel(const cf *in, cf *out, int64_t n, int64_t n0, const orc_chan_cfg &c, int n_taps, const int32_t *delay, Tap tap)
 {
     const float ns = c.noise_sigma * 0.70710678f;
     for (int64_t i = 0; i < n; ++i) {
         cf acc = {0.f, 0.f};
-        for (int t = 0; t < c.n_taps; ++t) {
-            int64_t j = i - c.delay[t];
+        for (int t = 0; t < n_taps; ++t) {
+            int64_t j = i - delay[t];
             if (j < 0 || j >= n) continue;
-            acc = wdm_cmac(acc, cf{c.tap_re[t], c.tap_im[t]}, in[j]);
+            acc = wdm_cmac(acc, tap(t, i), in[j]);
         }
         acc = cscale(acc, c.gain);
         cf w = crot(c.cfo * (float)i + c.phase0);
@@ -550,6 +552,26 @@ static void channel(const cf *in, cf *out, int64_t n, int64_t n0, const orc_chan
         }
         out[i] = y;
     }
+}
+
+/* the fading taps h_t(t0 + i) of include/wifi_detmath.h; tap t's terms in ascending order, tap 0's line-of-sight term
+ * after its n_sin sinusoids */
+static_assert(sizeof(orc_fading_cfg) == 112, "orc_fading_cfg has the layout of wifi_b200_fading");
+static int channel_fading(const cf *in, cf *out, int64_t n, int64_t n0, const orc_chan_cfg &c, const orc_fading_cfg &f)
+{
+    if (c.n_taps != 0 || f.n_taps < 1 || f.n_taps > 8 || f.n_sin < 1 || f.n_sin > 16 || !(f.k_factor >= 0.f) ||
+        !(f.doppler >= 0.f && f.doppler <= 0.25f) || !(std::fabs(f.los_doppler) <= 0.25f))
+        return -1;
+    for (int t = 0; t < f.n_taps; ++t)
+        if (f.delay[t] < 0 || !(f.power[t] >= 0.f)) return -1;
+    wdm_fade_ent ent[8][17];
+    const int cnt0 = f.n_sin + (f.k_factor > 0.f ? 1 : 0);
+    for (int t = 0; t < f.n_taps; ++t)
+        for (int m = 0; m < (t == 0 ? cnt0 : f.n_sin); ++m)
+            ent[t][m] = wdm_fading_entry(f.seed, f.stream, t, m, f.n_sin, f.power[t], f.k_factor, f.doppler, f.los_doppler);
+    channel(in, out, n, n0, c, f.n_taps, f.delay,
+            [&](int t, int64_t i) { return wdm_fading_tap(ent[t], t == 0 ? cnt0 : f.n_sin, (uint32_t)(f.t0 + i)); });
+    return 0;
 }
 
 /* ------------------------------------------------------------------- RX */
@@ -1105,7 +1127,15 @@ int orc_mac_frame(const uint8_t *payload, int n, int seq, const uint8_t *src, co
 }
 int orc_tx_symbols(const uint8_t *psdu, int len, int enc, int seed, uint8_t *out) { return tx_symbols(psdu, len, enc, seed, out); }
 int orc_tx_frame(const uint8_t *psdu, int len, int enc, int seed, float *iq, int cap) { return tx_frame(psdu, len, enc, seed, (cf *)iq, cap); }
-void orc_channel(const float *in, float *out, int64_t n, int64_t n0, const orc_chan_cfg *cfg) { channel((const cf *)in, (cf *)out, n, n0, *cfg); }
+void orc_channel(const float *in, float *out, int64_t n, int64_t n0, const orc_chan_cfg *cfg)
+{
+    const orc_chan_cfg &c = *cfg;
+    channel((const cf *)in, (cf *)out, n, n0, c, c.n_taps, c.delay, [&](int t, int64_t) { return cf{c.tap_re[t], c.tap_im[t]}; });
+}
+int orc_channel_fading(const float *in, float *out, int64_t n, int64_t n0, const orc_chan_cfg *seg, const orc_fading_cfg *fad)
+{
+    return channel_fading((const cf *)in, (cf *)out, n, n0, *seg, *fad);
+}
 
 void orc_frontend(const float *x, int64_t n, float *a_out, float *p_out, float *c_out)
 {

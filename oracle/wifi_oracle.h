@@ -95,6 +95,21 @@ typedef struct orc_chan_cfg {
     uint64_t stream;       /* Philox counter high words (link id)                */
 } orc_chan_cfg;
 void orc_channel(const float *in, float *out, int64_t n, int64_t n0, const orc_chan_cfg *cfg);
+/* time-varying fading taps, same layout and meaning as wifi_b200_fading (include/wifi_b200.h, 112 bytes) */
+typedef struct orc_fading_cfg {
+    int32_t n_taps;        /* 1..8                                               */
+    int32_t n_sin;         /* sinusoids per tap, 1..16                           */
+    int32_t delay[8];      /* samples, >= 0                                      */
+    float power[8];        /* E|h_t|^2, >= 0                                     */
+    float k_factor;        /* Rician K of tap 0, >= 0                            */
+    float doppler;         /* cycles/sample, 0 .. 0.25                           */
+    float los_doppler;     /* cycles/sample, -0.25 .. 0.25                       */
+    int32_t reserved;
+    int64_t t0;            /* time index of output sample 0                      */
+    uint64_t seed, stream; /* Philox key and counter words of the realisation    */
+} orc_fading_cfg;
+/* orc_channel with the taps of fad (seg->n_taps must be 0); -1 for out-of-range parameters, else 0 */
+int  orc_channel_fading(const float *in, float *out, int64_t n, int64_t n0, const orc_chan_cfg *seg, const orc_fading_cfg *fad);
 
 /* ---- RX ---- */
 void orc_frontend(const float *x, int64_t n, float *a_out, float *p_out, float *c_out);

@@ -1,5 +1,5 @@
 """Time-varying Rayleigh/Rician multipath fading (wifi_b200_channel_fading[_dev]) and its CPU reference
-(tests/fading_oracle.cpp, the oracle's channel() loop with the fading taps).
+(the oracle's channel() with the fading taps).
 
 The CPU half checks the model through that reference and the oracle's contract self-test: the NCO sincos of include/wifi_detmath.h, the Rayleigh / Rician
 marginals, Clarke's autocorrelation, the power-delay profile and the determinism a user builds on (same realisation for the
@@ -10,15 +10,14 @@ capture that fades inside its frames."""
 import numpy as np
 import pytest
 
-import fading_oracle as F
 from util import assert_frames_equal
 
 SINCOS_TURN, FADING_ENTRY, FADING_FREQ, FADING_STEP = 13, 14, 15, 16
 
 
-def _h(n, **fad):
+def _h(O, n, **fad):
     """The realisation itself: all-ones input, one tap at delay 0, gain 1, no noise -> the output is h_0(t0 + i)."""
-    return F.channel(np.ones(n, np.complex64), fading=dict(taps=fad.pop("taps", ((0, 1.0),)), **fad))
+    return O.channel(np.ones(n, np.complex64), fading=dict(taps=fad.pop("taps", ((0, 1.0),)), **fad))
 
 
 # ---------------------------------------------------------------------------------------------------------- CPU (oracle)
@@ -33,37 +32,37 @@ def test_turn_sincos_accuracy(O):
     assert s[z] == 0.0 and c[z] == 1.0                       # zero phase is exactly (0, 1): a static tap stays exact
 
 
-def test_block_rayleigh():
+def test_block_rayleigh(O):
     from scipy import stats
-    h = _h(64, taps=((0, 2.0),), seed=5, stream=0)
+    h = _h(O, 64, taps=((0, 2.0),), seed=5, stream=0)
     assert np.all(h == h[0])                                   # doppler 0: one value per segment, exactly
-    h = np.array([_h(1, taps=((0, 2.0),), seed=5, stream=s)[0] for s in range(4000)])
+    h = np.array([_h(O, 1, taps=((0, 2.0),), seed=5, stream=s)[0] for s in range(4000)])
     e = np.abs(h.astype(np.complex128)) ** 2
     assert abs(e.mean() - 2.0) < 5 * 2.0 / np.sqrt(e.size)
     assert stats.kstest(e, "expon", args=(0, 2.0)).pvalue > 1e-3
 
 
-def test_rician_k_by_moments():
-    h = np.array([_h(1, k_factor=4.0, doppler=1e-3, los_doppler=2e-4, seed=9, stream=s)[0] for s in range(4000)])
+def test_rician_k_by_moments(O):
+    h = np.array([_h(O, 1, k_factor=4.0, doppler=1e-3, los_doppler=2e-4, seed=9, stream=s)[0] for s in range(4000)])
     e = np.abs(h.astype(np.complex128)) ** 2
     q = np.sqrt(2 - np.mean(e ** 2) / np.mean(e) ** 2)        # m4 / m2^2 = 2 - (K / (K + 1))^2
     assert abs(q / (1 - q) - 4.0) < 0.2 * 4.0
     assert abs(e.mean() - 1.0) < 0.05
 
 
-def test_strong_line_of_sight_without_doppler_keeps_its_phase():
-    h = _h(20000, k_factor=1e5, doppler=1e-3, los_doppler=0.0, seed=1, stream=7)
+def test_strong_line_of_sight_without_doppler_keeps_its_phase(O):
+    h = _h(O, 20000, k_factor=1e5, doppler=1e-3, los_doppler=0.0, seed=1, stream=7)
     d = np.angle(h * np.conj(h[0]))
     assert np.abs(d).max() < 0.05
-    g = _h(20000, k_factor=1e5, doppler=1e-3, los_doppler=1e-4, seed=1, stream=7)
+    g = _h(O, 20000, k_factor=1e5, doppler=1e-3, los_doppler=1e-4, seed=1, stream=7)
     assert np.abs(np.angle(g * np.conj(g[0]))).max() > 1.0      # a LoS Doppler does turn it
 
 
-def test_clarke_autocorrelation():
+def test_clarke_autocorrelation(O):
     from scipy import special
     fd = 0.01
     lags = np.rint(np.array([0.5, 1.0, 2.405, 3.8]) / (2 * np.pi * fd)).astype(int)
-    H = np.array([_h(200, doppler=fd, seed=2, stream=s) for s in range(4000)]).astype(np.complex128)
+    H = np.array([_h(O, 200, doppler=fd, seed=2, stream=s) for s in range(4000)]).astype(np.complex128)
     for L in lags:
         r = np.mean(H[:, :200 - L] * np.conj(H[:, L:]))
         assert abs(r.real - special.j0(2 * np.pi * fd * L)) < 0.08 and abs(r.imag) < 0.08, (L, r)
@@ -84,11 +83,11 @@ def test_no_frequency_beyond_the_doppler(O):
         assert f.max() > 0.9 * fd * 2 ** 32 and f.min() < -0.9 * fd * 2 ** 32
 
 
-def test_taps_follow_the_power_delay_profile_and_are_uncorrelated():
+def test_taps_follow_the_power_delay_profile_and_are_uncorrelated(O):
     pdp = ((0, 0.6), (2, 0.3), (5, 0.1))
     x = np.zeros(8, np.complex64)
     x[0] = 1
-    H = np.array([F.channel(x, fading=dict(taps=pdp, n_sin=4, seed=3, stream=s))[[0, 2, 5]] for s in range(4000)]).astype(np.complex128)
+    H = np.array([O.channel(x, fading=dict(taps=pdp, n_sin=4, seed=3, stream=s))[[0, 2, 5]] for s in range(4000)]).astype(np.complex128)
     N = H.shape[0]
     for k, (_, p) in enumerate(pdp):
         assert abs(np.mean(np.abs(H[:, k]) ** 2) - p) < 5 * p / np.sqrt(N), k
@@ -97,26 +96,26 @@ def test_taps_follow_the_power_delay_profile_and_are_uncorrelated():
             assert abs(np.mean(H[:, a] * np.conj(H[:, b]))) / np.sqrt(pdp[a][1] * pdp[b][1]) < 5 / np.sqrt(N), (a, b)
 
 
-def test_determinism_streams_and_split_segments():
+def test_determinism_streams_and_split_segments(O):
     rng = np.random.default_rng(8)
     x = (rng.standard_normal(3000) + 1j * rng.standard_normal(3000)).astype(np.complex64)
     fad = dict(taps=((0, 1.0),), k_factor=2.0, doppler=1e-3, los_doppler=-3e-4, seed=11, stream=4)
     kw = dict(gain=0.8, noise_sigma=0.05, seed=99, stream=2)
-    a = F.channel(x, fading=fad, **kw)
-    assert np.array_equal(a, F.channel(x, fading=fad, **kw))
-    assert not np.array_equal(a, F.channel(x, fading=dict(fad, stream=5), **kw))
+    a = O.channel(x, fading=fad, **kw)
+    assert np.array_equal(a, O.channel(x, fading=fad, **kw))
+    assert not np.array_equal(a, O.channel(x, fading=dict(fad, stream=5), **kw))
     N = 1234
-    first = F.channel(x[:N], fading=fad, **kw)
-    second = F.channel(x[N:], n0=N, fading=dict(fad, t0=N), **kw)
+    first = O.channel(x[:N], fading=fad, **kw)
+    second = O.channel(x[N:], n0=N, fading=dict(fad, t0=N), **kw)
     assert np.array_equal(np.concatenate([first, second]), a)
 
 
-def test_out_of_range_parameters_are_refused_by_the_oracle():
+def test_out_of_range_parameters_are_refused_by_the_oracle(O):
     x = np.ones(4, np.complex64)
     for bad in (dict(taps=()), dict(n_sin=0), dict(n_sin=17), dict(k_factor=-1.0), dict(doppler=0.3), dict(doppler=-1e-3),
                 dict(los_doppler=0.26), dict(taps=((-1, 1.0),)), dict(taps=((0, -1.0),))):
         with pytest.raises(ValueError):
-            F.channel(x, fading=dict(dict(taps=((0, 1.0),)), **bad))
+            O.channel(x, fading=dict(dict(taps=((0, 1.0),)), **bad))
 
 
 # ------------------------------------------------------------------------------------------------------------------- GPU
@@ -126,8 +125,8 @@ def _seg_pair(W, n, seg, fad):
     return w.chan_seg(in_len=n, n=n, taps=(), **seg), w.fading(**fad)
 
 
-def _oracle_seg(x, s, f):
-    return F.channel(x, f, n0=int(s["n0"][0]), gain=float(s["gain"][0]), cfo=float(s["cfo"][0]), phase0=float(s["phase0"][0]),
+def _oracle_seg(O, x, s, f):
+    return O.channel(x, fading=f, n0=int(s["n0"][0]), gain=float(s["gain"][0]), cfo=float(s["cfo"][0]), phase0=float(s["phase0"][0]),
                      noise_sigma=float(s["noise_sigma"][0]), seed=int(s["seed"][0]), stream=int(s["stream"][0]))
 
 
@@ -143,7 +142,7 @@ CASES = {
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", sorted(CASES))
-def test_kernel_equals_oracle(W, case):
+def test_kernel_equals_oracle(O, W, case):
     import torch
     kw = dict(CASES[case])
     segkw = kw.pop("seg", {})
@@ -155,14 +154,14 @@ def test_kernel_equals_oracle(W, case):
         ty = torch.zeros_like(tx)
         h.channel_fading_dev(tx.data_ptr(), ty.data_ptr(), s, f)
         got = ty.cpu().numpy().view(np.complex64)
-        assert np.array_equal(got, _oracle_seg(x, s, f))
+        assert np.array_equal(got, _oracle_seg(O, x, s, f))
         assert np.array_equal(h.channel(x, fading=f, **segkw), got)    # host-buffer twin
     finally:
         h.close()
 
 
 @pytest.mark.gpu
-def test_many_segments_over_several_launches(W):
+def test_many_segments_over_several_launches(O, W):
     """70000 segments: more than one launch of 65535 grid rows, every one its own stream, t0 and n0."""
     import torch
     w = W.wifi_b200
@@ -191,7 +190,7 @@ def test_many_segments_over_several_launches(W):
     finally:
         h.close()
     for i in list(range(0, 600)) + list(range(65400, 65700)) + list(range(n_seg - 300, n_seg)):
-        want = _oracle_seg(x[i * L:(i + 1) * L], segs[i:i + 1], fades[i:i + 1])
+        want = _oracle_seg(O, x[i * L:(i + 1) * L], segs[i:i + 1], fades[i:i + 1])
         assert np.array_equal(got[i], want), i
     assert len({got[i, 0] for i in range(0, n_seg, 97)}) > 700      # distinct streams, distinct realisations
 
@@ -313,6 +312,31 @@ def test_out_of_range_fading_is_refused_and_writes_nothing(W):
             rc = h._L.wifi_b200_channel_fading(h._h, w._p(np.ones(256, np.complex64)), 256, w._p(out), 256, w._p(s), w._p(f), s.size)
             assert rc == w.E_ARG and np.all(out == 7 + 7j)
         assert h._L.wifi_b200_channel_fading_dev(h._h, x.data_ptr(), y.data_ptr(), w._p(good_s), None, 1) == w.E_ARG
+    finally:
+        h.close()
+
+
+@pytest.mark.gpu
+def test_out_of_range_fixed_channel_is_refused_and_writes_nothing(W):
+    """The fixed-tap host form checks its segments as the fading one does, before anything is allocated or written."""
+    w = W.wifi_b200
+    h = W.Handle(max_samples=1 << 16)
+    try:
+        x = np.ones(256, np.complex64)
+        good = w.chan_seg(in_len=256, n=256)
+        out = np.full(256, 7 + 7j, np.complex64)
+        assert h._L.wifi_b200_channel(h._h, w._p(x), 256, w._p(out), 256, w._p(good), 1) == 0
+        assert not np.all(out == 7 + 7j)
+        cases = [(None, 1), (good, 0)]
+        for field, v in (("in_off", 1), ("in_off", -1), ("out_off", 1), ("out_off", -1), ("n", 257), ("in_len", 257),
+                         ("in_len", -1), ("n_taps", 9)):
+            s = good.copy()
+            s[field] = v
+            cases.append((s, 1))
+        for s, n_segs in cases:
+            out = np.full(256, 7 + 7j, np.complex64)
+            rc = h._L.wifi_b200_channel(h._h, w._p(x), 256, w._p(out), 256, w._p(s), n_segs)
+            assert rc == w.E_ARG and np.all(out == 7 + 7j), (s, n_segs)
     finally:
         h.close()
 

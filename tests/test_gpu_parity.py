@@ -228,6 +228,7 @@ def test_channel_matches_oracle(H, O, W):
     H.channel_dev(tx.data_ptr(), ty.data_ptr(), seg)
     got = ty.cpu().numpy().view(np.complex64)
     assert np.array_equal(got, ref), np.abs(got - ref).max()
+    assert np.array_equal(H.channel(x, n0=1234, gain=0.7, cfo=0.013, phase0=0.5, noise_sigma=0.2, taps=taps, seed=77, stream=3), got)
 
 
 def test_full_size_roundtrip_property(O, W):
