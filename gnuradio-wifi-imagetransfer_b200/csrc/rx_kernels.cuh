@@ -643,7 +643,8 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
     __shared__ float s_h2[SOFT ? 4 : 1][SOFT ? 64 : 2];
     __shared__ cf s_hu[4][64];
     __shared__ double s_md[4][64], s_ms[4][64];
-    __shared__ uint16_t s_lut[4][432];
+    // trellis-word LUT: slots k..k+3 of word w are one uint4 at [k / 4][w], so four offsets come with one load
+    __shared__ __align__(16) uint32_t s_lut[4][432];
     // decisions as bit planes: byte (carrier << 3 | bit) = that coded bit (0 / 1), so a LUT entry is the byte
     // offset itself; carrier 48 is a zero slot that the erasure entries point at
     __shared__ __align__(8) uint8_t s_bits[4][49 * 8];
@@ -682,7 +683,7 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
     const bool dcA = (iA == 32);
     const int carA = c_tab.carrier_of[iA], carB = c_tab.carrier_of[iB];
     const float ltsA = c_tab.lts[iA], ltsB = c_tab.lts[iB];
-    const int q0 = 2 * dev_bitrev5(lane);
+    const int q0 = warp_fft_in(lane);
     const WarpTw tw = warp_tw(lane, false);
 
     cf HA = {0.f, 0.f}, HB = {0.f, 0.f};
@@ -723,7 +724,7 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
     if (wps) {
         for (int i = lane; i < 2 * ndbps; i += 32) {
             uint16_t e = depunct_lut[enc * 432 + i];
-            s_lut[wib][(i & 15) * 27 + (i >> 4)] = (e == 0xffffu) ? (uint16_t)(48 << 3) : e;   // [k][word]: conflict-free reads
+            s_lut[wib][((i & 15) >> 2) * 108 + (i >> 4) * 4 + (i & 3)] = (e == 0xffffu) ? 48u << 3 : e;   // conflict-free reads
         }
         if (lane < wps)
             for (int k = 0; k < 16; ++k)
@@ -837,9 +838,10 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
                 if (u) b = cdiv(b, G); else a = cdiv(a, G);
             }
         }
-        if (n == 0) {
+        // (PHASE == 0 spelt out: on the n >= 3 assumption alone the compiler keeps the LTS blocks in the data loop)
+        if (PHASE == 0 && n == 0) {
             HA = a; HB = b;
-        } else if (n == 1) {
+        } else if (PHASE == 0 && n == 1) {
             {
                 cf d = csub(HA, a), s = cadd(HA, a);
                 float md = sqrtf(d.re * d.re + d.im * d.im), ms = sqrtf(s.re * s.re + s.im * s.im);
@@ -874,35 +876,29 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
             }
             __syncwarp();
         } else {
-            cf symA = {0.f, 0.f}, symB = {0.f, 0.f};
-            int bitsA = 0, bitsB = 0;
+            // Straight-line carrier path: every lane equalizes and decides both of its bins, and the results of a
+            // bin that is no data carrier (pilot, DC, guard) are never stored or selected into H.  Branching per
+            // carrier instead made the warp run both sides of every test.
+            cf ptA, ptB;
+            int bitsA, bitsB;
+            const cf symA = cdiv(a, HA), symB = cdiv(b, HB);
+            dev_decide_point(nb, symA, bitsA, ptA);
+            dev_decide_point(nb, symB, bitsB, ptB);
+            SoftQ sqA = {}, sqB = {};
+            if (SOFT && soft_on) { sqA = dev_soft_demap(nb, symA, w0A); sqB = dev_soft_demap(nb, symB, w0B); }
+            if (ALGO == WIFI_EQ_LMS) {
+                const cf qA = cdiv(a, ptA), qB = cdiv(b, ptB);
+                const cf nA = cadd(cscale(HA, 0.5f), cscale(qA, 0.5f)), nB = cadd(cscale(HB, 0.5f), cscale(qB, 0.5f));
+                HA = carA >= 0 ? nA : HA;
+                HB = carB >= 0 ? nB : HB;
+            }
             cf huA = {0.f, 0.f}, huB = {0.f, 0.f};
-            SoftQ sqA, sqB;
-#pragma unroll
-            for (int u = 0; u < 2; ++u)
-#pragma unroll
-                for (int t = 0; t < 3; ++t) { sqA.q[u][t] = 0; sqB.q[u][t] = 0; }
-            if (carA >= 0) {
-                cf ptA;
-                symA = cdiv(a, HA);
-                dev_decide_point(nb, symA, bitsA, ptA);
-                if (SOFT && soft_on) sqA = dev_soft_demap(nb, symA, w0A);
-                if (ALGO == WIFI_EQ_LMS) {
-                    cf q = cdiv(a, ptA);
-                    HA = cadd(cscale(HA, 0.5f), cscale(q, 0.5f));
-                } else if (ALGO == WIFI_EQ_STA) huA = cdiv(a, ptA);
-            } else if (iA == 39) huA = cscale(a, p);
-            else if (iA == 53) huA = cscale(a, -p);
-            if (carB >= 0) {
-                cf ptB;
-                symB = cdiv(b, HB);
-                dev_decide_point(nb, symB, bitsB, ptB);
-                if (SOFT && soft_on) sqB = dev_soft_demap(nb, symB, w0B);
-                if (ALGO == WIFI_EQ_LMS) {
-                    cf q = cdiv(b, ptB);
-                    HB = cadd(cscale(HB, 0.5f), cscale(q, 0.5f));
-                } else if (ALGO == WIFI_EQ_STA) huB = cdiv(b, ptB);
-            } else if (iB == 11 || iB == 25) huB = cscale(b, p);
+            if (ALGO == WIFI_EQ_STA) {
+                const cf dA = cdiv(a, ptA), dB = cdiv(b, ptB);
+                const cf pA = cscale(a, iA == 53 ? -p : p), pB = cscale(b, p);
+                huA = carA >= 0 ? dA : (iA == 39 || iA == 53) ? pA : huA;
+                huB = carB >= 0 ? dB : (iB == 11 || iB == 25) ? pB : huB;
+            }
             if (ALGO == WIFI_EQ_STA) {
                 s_hu[wib][iA] = huA; s_hu[wib][iB] = huB;
                 __syncwarp();
@@ -923,7 +919,7 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
                 }
                 __syncwarp();
             }
-            if (n == 2) {
+            if (PHASE == 0) {   // n == 2: SIGNAL
                 if (carA >= 0) st->sig_bits[carA] = (uint8_t)bitsA;
                 if (carB >= 0) st->sig_bits[carB] = (uint8_t)bitsB;
             } else {
@@ -946,9 +942,11 @@ __global__ void __launch_bounds__(128, DEMOD_MINB) k_demod(const cf *__restrict_
                     if (lane < wps) {
                         uint32_t word = era_word;
 #pragma unroll
-                        for (int k = 0; k < 16; ++k) {
-                            const uint32_t e = s_lut[wib][k * 27 + lane];
-                            word += (uint32_t)s_bits[wib][e] << (2 * k);          // disjoint bit positions: + is |
+                        for (int j = 0; j < 4; ++j) {
+                            const uint4 e = reinterpret_cast<const uint4 *>(s_lut[wib])[j * 27 + lane];
+                            // disjoint bit positions: + is |
+                            word += ((uint32_t)s_bits[wib][e.x] << (8 * j)) + ((uint32_t)s_bits[wib][e.y] << (8 * j + 2)) +
+                                    ((uint32_t)s_bits[wib][e.z] << (8 * j + 4)) + ((uint32_t)s_bits[wib][e.w] << (8 * j + 6));
                         }
                         vw[(n - 3) * wps + lane] = word;
                     }

@@ -71,7 +71,7 @@ __global__ void __launch_bounds__(128) k_tx(const uint8_t *__restrict__ psdu_blo
     __syncthreads();
     const int total_syms = 5 + n_sym;
     cf *o = out + D.burst_off;
-    const int q0 = 2 * dev_bitrev5(lane);
+    const int q0 = warp_fft_in(lane);
     const WarpTw tw = warp_tw(lane, true);
     for (int s = wib; s < total_syms; s += 4) {
         cf v[2];

@@ -187,25 +187,42 @@ __device__ __forceinline__ WarpTw warp_tw(int lane, bool inverse)
     return t;
 }
 
-// 64-point FFT across one warp.  On entry lane l holds in[2*bitrev5(l)] (a) and
-// in[2*bitrev5(l)+1] (b) -- i.e. DIT positions l and l+32 after bit reversal.  On
-// exit a = X[l], b = X[l+32].  Same butterfly network and rounding as oracle fft64().
+// Input index of a in warp_fft64 on lane l: 2*bitrev5(r) with r = l rotated left by one bit (5 bits);
+// b is the input right after it.
+__device__ __forceinline__ int warp_fft_in(int lane)
+{
+    return 2 * dev_bitrev5(((lane << 1) | (lane >> 4)) & 31);
+}
+
+// Lanes l and l^m trade one value: afterwards the lane with (l & m) == 0 holds its lo and the partner's lo,
+// the other one the partner's hi and its own hi.  This turns span-2^k butterfly pairs into span-2^k' pairs.
+__device__ __forceinline__ void warp_fft_trade(cf &lo, cf &hi, int lane, int m)
+{
+    const bool up = (lane & m) != 0;
+    const cf r = cshfl_xor(up ? lo : hi, m);
+    lo = up ? r : lo;
+    hi = up ? hi : r;
+}
+
+// 64-point FFT across one warp, one butterfly per lane and stage.  On entry lane l holds in[warp_fft_in(l)] (a)
+// and the input after it (b): DIT positions r and r+32 after bit reversal, r = l rotated left by one bit.
+// Before the stage of span 2^s (s < 5) the lane holds a span-2^s pair; one trade with lane l^m re-pairs the
+// values for the next stage.  The trade masks 16, 1, 2, 4, 8, 16 rotate the lane-to-position map back by one bit,
+// so that on exit a = X[l], b = X[l+32], and at every stage s the pair's twiddle is tw.w[s] of warp_tw.
+// Each butterfly is t = w*hi, lo + t, lo - t: the operations, operands and rounding of oracle fft64().
 __device__ __forceinline__ void warp_fft64(cf &a, cf &b, int lane, const WarpTw &tw)
 {
+    warp_fft_trade(a, b, lane, 16);
 #pragma unroll
     for (int s = 0; s < 5; ++s) {
-        const int half = 1 << s;
-        const cf w = tw.w[s];
-        const bool hi = (lane & half) != 0;
-        cf ta = hi ? cmul(w, a) : a;
-        cf tb = hi ? cmul(w, b) : b;
-        cf ra = cshfl_xor(ta, half);
-        cf rb = cshfl_xor(tb, half);
-        a = hi ? csub(ra, ta) : cadd(a, ra);
-        b = hi ? csub(rb, tb) : cadd(b, rb);
+        const cf t = cmul(tw.w[s], b);
+        const cf u = a;
+        a = cadd(u, t);
+        b = csub(u, t);
+        warp_fft_trade(a, b, lane, 1 << s);
     }
-    cf t = cmul(tw.w[5], b);
-    cf u = a;
+    const cf t = cmul(tw.w[5], b);
+    const cf u = a;
     a = cadd(u, t);
     b = csub(u, t);
 }
