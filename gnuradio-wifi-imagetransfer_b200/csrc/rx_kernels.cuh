@@ -996,8 +996,10 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_signal(wifi_b200_frame *frames, i
 {
     __shared__ uint32_t ring[5 * 16 * VIT_BLOCK];
     __shared__ uint4 s_bm[8 * 4 * 16];
+    __shared__ uint32_t s_hop[VIT_HOP_ENTRIES];
     const int tid = threadIdx.x;
     for (int i = tid; i < 512; i += VIT_BLOCK) s_bm[i] = VitCoreH::table_entry(i >> 6, (i >> 4) & 3, (uint32_t)(i & 15));
+    for (int i = tid; i < VIT_HOP_ENTRIES; i += VIT_BLOCK) s_hop[i] = vit_h_hop_entry(i);
     __syncthreads();
     int f = f0 + blockIdx.x * VIT_BLOCK + tid;
     if (f >= n_frames) return;
@@ -1019,7 +1021,9 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_signal(wifi_b200_frame *frames, i
     const uint32_t first = (uint32_t)lo;
     v.step4<0>(s_bm, 0xau, 0xau, first & 0xfu, (first >> 4) & 0xfu);
     v.step4<4>(s_bm, (first >> 8) & 0xfu, (first >> 12) & 0xfu, (first >> 16) & 0xfu, (first >> 20) & 0xfu);
-    v.trace_begin(ring, 1, 5, tid, true, 0xfcu);
+    uint8_t *rbt = reinterpret_cast<uint8_t *>(ring) + 4 * tid;   // the thread's column of slot 0
+    const uint32_t rbt_sh = (uint32_t)__cvta_generic_to_shared(rbt), hop_sh = (uint32_t)__cvta_generic_to_shared(s_hop);
+    v.trace_begin(rbt + VIT_SLOT_BYTES, rbt_sh + VIT_SLOT_BYTES, s_hop, true, 0xfcu);
     uint32_t dec = 0;   // decoded bit i at bit i
 #pragma unroll 1
     for (int chunk = 1; chunk < 8; ++chunk) {
@@ -1028,11 +1032,17 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_signal(wifi_b200_frame *frames, i
         hi >>= 32;
         v.step4<0>(s_bm, bits & 0xfu, (bits >> 4) & 0xfu, (bits >> 8) & 0xfu, (bits >> 12) & 0xfu);
         v.step4<4>(s_bm, (bits >> 16) & 0xfu, (bits >> 20) & 0xfu, (bits >> 24) & 0xfu, bits >> 28);
-        VitTrace tr = v.trace_begin(ring, (chunk + 1) % 5, 5, tid, (chunk & 3) == 0);
+        int sl = (chunk + 1) % 5;
+        uint32_t c = v.trace_begin(rbt + sl * VIT_SLOT_BYTES, rbt_sh + sl * VIT_SLOT_BYTES, s_hop, (chunk & 3) == 0);
         if (chunk >= 5) {
-            // the ring byte holds the decisions in ascending bit order, as dec does
-            VitCoreH::trace_hops<4>(tr, ring, 5, tid);
-            dec |= vit_ring_byte(ring, tr.sl, tr.bs, tid) << (8 * (chunk - 5));
+            // four hops back through slots sl - 1 .. sl - 4 (mod 5); the ring byte holds the decisions in ascending
+            // bit order, as dec does.  The first hop reads the snapshot just stored: keep the stores ahead of it.
+            asm volatile("" ::: "memory");
+            for (int i = 0; i < 4; ++i) {
+                sl = sl == 0 ? 4 : sl - 1;
+                c = VitCoreH::hop(c, hop_sh, rbt_sh + sl * VIT_SLOT_BYTES);
+            }
+            dec |= VitCoreH::ring_byte(c) << (8 * (chunk - 5));
         }
     }
     int r = 0, len = 0;
@@ -1262,17 +1272,24 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict
     uint32_t *s_crc = vsm + VIT_NTB_MAX * 16 * VIT_BLOCK;   // 256
     uint16_t *s_scr = (uint16_t *)(s_crc + 256);            // 128
     uint4 *s_bm = (uint4 *)(s_crc + 256 + 64);              // branch-word table [8 steps][4 selectors][16 symbol pairs] (VitCoreH::table_entry)
+    uint4 *s_rows = s_bm + 512;                             // traceback rows [VIT_ROWS][3] (vit_h_row_entry)
+    uint32_t *s_hop = (uint32_t *)(s_rows + 3 * VIT_ROWS);  // hop table (vit_h_hop_entry)
     const int tid = threadIdx.x;
     for (int i = tid; i < 256; i += VIT_BLOCK) s_crc[i] = c_tab.crc_tab[i];
     for (int i = tid; i < 128; i += VIT_BLOCK) s_scr[i] = c_tab.scr_tab[i];
     for (int i = tid; i < 512; i += VIT_BLOCK) s_bm[i] = VitCoreH::table_entry(i >> 6, (i >> 4) & 3, (uint32_t)(i & 15));
+    for (int i = tid; i < 12 * VIT_ROWS; i += VIT_BLOCK) ((uint32_t *)s_rows)[i] = vit_h_row_entry(i / 12, i % 12);
+    for (int i = tid; i < VIT_HOP_ENTRIES; i += VIT_BLOCK) s_hop[i] = vit_h_hop_entry(i);
+    // the identity slot, in every thread's column (a frame with ntb = 10 overwrites it with snapshots and never reads it
+    // as such)
+    for (int w = 0; w < 16; ++w) ring[(VIT_ID_SLOT * 16 + w) * VIT_BLOCK + tid] = vit_h_identity_word(w);
     __syncthreads();
     const int job = f0 + blockIdx.x * VIT_BLOCK + tid;
     if (job >= n_frames) return;
     const JobDesc J = jobs[job];
     if (J.n_sym == 0) return;
     const int punct = c_tab.mcs[J.enc].punct;
-    const int ntb = punct == 0 ? 5 : (punct == 1 ? 9 : 10);
+    const int ntb = punct == 0 ? 5 : (punct == 1 ? 9 : 10);   // the three depths the traceback rows know (vit_h_row_entry)
     const int nw = (J.n_sym * c_tab.mcs[J.enc].n_dbps + 7) >> 3;
     const uint32_t *in = vit_in + (int64_t)job * VIT_MAXW;
     uint32_t *out = psdu + (int64_t)job * (PSDU_STRIDE / 4);
@@ -1285,33 +1302,45 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict
     // every path byte, which trace_begin masks off (keep = 0xfc)
     v.step4<0>(s_bm, 0xau, 0xau, prev & 0xfu, (prev >> 4) & 0xfu);
     v.step4<4>(s_bm, (prev >> 8) & 0xfu, (prev >> 12) & 0xfu, (prev >> 16) & 0xfu, (prev >> 20) & 0xfu);
-    int slot = 1 % ntb;
-    v.trace_begin(ring, slot, ntb, tid, true, 0xfcu);
+    // the traceback of chunk j - 1 (snapshot slot s = j mod ntb, row `row`) runs interleaved with the trellis steps of
+    // chunk j, three hops before each step4 and three before the output byte; the cursor `c` is a ring byte offset
+    // (VitCoreH), the hops' slots come from the row
+    uint8_t *rbt = reinterpret_cast<uint8_t *>(ring) + 4 * tid;   // the thread's column of slot 0
+    const uint32_t rbt_sh = (uint32_t)__cvta_generic_to_shared(rbt), hop_sh = (uint32_t)__cvta_generic_to_shared(s_hop);
+    int row = 3 * (vit_h_row0(ntb) + 1);
+    uint4 r0 = s_rows[row];
+    uint32_t c = v.trace_begin(rbt + r0.x, rbt_sh + r0.y, s_hop, true, 0xfcu);
     PsduSink sink;
     sink.init(out, L, s_crc, s_scr);
     uint32_t next = 1 < nw ? in[1] : 0u;
-    // software pipeline: the traceback of chunk j-1 runs interleaved with the trellis steps of chunk j
-    VitTrace tr;
-    tr.bs = 0; tr.sl = slot; tr.left = 0;
-    bool pending = false;
 #pragma unroll 1
     for (int chunk = 1; chunk <= last_chunk; ++chunk) {
         uint32_t bits = __funnelshift_r(prev, next, 24);
         prev = next;
         next = (chunk + 1 < nw) ? in[chunk + 1] : 0u;
-        VitCoreH::trace_hops<3>(tr, ring, ntb, tid);
+        const uint4 r1 = s_rows[row + 1], r2 = s_rows[row + 2];
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r0.z);
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r0.w);
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.x);
         v.step4<0>(s_bm, bits & 0xfu, (bits >> 4) & 0xfu, (bits >> 8) & 0xfu, (bits >> 12) & 0xfu);
-        VitCoreH::trace_hops<3>(tr, ring, ntb, tid);
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.y);
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.z);
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.w);
         v.step4<4>(s_bm, (bits >> 16) & 0xfu, (bits >> 20) & 0xfu, (bits >> 24) & 0xfu, bits >> 28);
-        VitCoreH::trace_hops<3>(tr, ring, ntb, tid);
-        if (pending && chunk - 1 >= ntb) sink.push(VitCoreH::trace_finish(tr, ring, tid), chunk - 1 - ntb);
-        slot = (slot + 1 == ntb) ? 0 : slot + 1;
-        tr = v.trace_begin(ring, slot, ntb, tid, (chunk & 3) == 0);
-        pending = true;
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r2.x);
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r2.y);
+        c = VitCoreH::hop(c, hop_sh, rbt_sh + r2.z);
+        if (chunk - 1 >= ntb) sink.push(VitCoreH::trace_finish(c), chunk - 1 - ntb);
+        row = (int)r2.w;
+        r0 = s_rows[row];
+        c = v.trace_begin(rbt + r0.x, rbt_sh + r0.y, s_hop, (chunk & 3) == 0);
     }
-    if (pending && last_chunk >= ntb) {
-        VitCoreH::trace_hops<9>(tr, ring, ntb, tid);
-        sink.push(VitCoreH::trace_finish(tr, ring, tid), last_chunk - ntb);
+    if (last_chunk >= ntb) {
+        const uint4 r1 = s_rows[row + 1], r2 = s_rows[row + 2];
+        const uint32_t base[9] = {r0.z, r0.w, r1.x, r1.y, r1.z, r1.w, r2.x, r2.y, r2.z};
+#pragma unroll
+        for (int i = 0; i < 9; ++i) c = VitCoreH::hop(c, hop_sh, rbt_sh + base[i]);
+        sink.push(VitCoreH::trace_finish(c), last_chunk - ntb);
     }
     frames[J.frame].crc_ok = sink.crc_ok();
 }

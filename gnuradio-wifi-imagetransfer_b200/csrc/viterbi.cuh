@@ -18,7 +18,8 @@
 // A butterfly leaves its survivors split into "new even states" and "new odd states" words; instead of interleaving
 // them back to natural order after every step, the next steps pair the split words directly -- the state stride inside
 // a word doubles each step: 1 (natural) -> 2 -> 4 -> 8 -> 16 -- and one transpose restores natural order after the
-// fourth step.  Chunks are 8 steps, so snapshots and the best-state search always see the natural layout.  The path
+// fourth step.  Chunks are 8 steps, so the best-state search always sees the natural layout, and so do the snapshots
+// of VitQuad and VitCoreSoft (VitCoreH snapshots the split layout in front of the transpose).  The path
 // bytes are never shifted: step s of a chunk sets its own decision bit.  Chunk 0 has 6 steps; it runs as two erased
 // steps + 6, whose two extra decision bits are masked off before the snapshot (see the kernels).
 // Path snapshots of the per-thread forms go to shared memory, word-interleaved across the block's threads (bank =
@@ -51,11 +52,10 @@ __host__ __device__ constexpr uint32_t vit_sel2(int k0, int k1)
 }
 
 // The traceback of one chunk is a chain of dependent shared-memory reads.  trace_begin() stores the snapshot and finds
-// the first best state; trace_hops() advances a few hops (branch-free, so the scheduler can interleave the chain with
-// the next chunk's add-compare-select work; measured: a variant without the three selects, for warps whose frames all
-// trace back nine snapshots, is slower -- the kernel is bound by its schedule, not by these few ops); then the output
-// byte is read.  That read must come before the next snapshot is stored: the byte lives in the slot it overwrites.
-// VitTrace is the cursor: state, ring slot, hops left.
+// the first best state; the hops follow (branch-free, so the scheduler can interleave the chain with the next chunk's
+// add-compare-select work); then the output byte is read.  That read must come before the next snapshot is stored:
+// the byte lives in the slot it overwrites.  VitQuad and VitCoreSoft keep the cursor as VitTrace (state, ring slot,
+// hops left) and step it with trace_hops(); VitCoreH's cursor is a byte address (see there).
 struct VitTrace { int bs, sl, left; };
 // byte (slot, state) of this thread's ring: the ring is word-interleaved across the block's threads,
 // word (slot * 16 + state / 4) * VIT_BLOCK + tid, so the path byte is a single byte load
@@ -76,10 +76,74 @@ __device__ __forceinline__ uint32_t vit_ring_byte(const uint32_t *ring, int sl, 
 // byte-packed form of VitQuad::bfly (compare word, sign-replicating permute, two selects per output word), for the
 // same 32 registers of state a whole trellis takes in bytes (16 metric words + 16 path words).
 // Path bytes are therefore bit-reversed with respect to upstream's shift register (decision of step s at bit 7 - s):
-// the traceback reverses the byte it follows (one BREV per hop), and the output byte is reversed once.
-// Metrics stay below 12 + 4 * 16 = 76 between renormalisations (every fourth chunk), so 8 bits hold them.
+// the traceback follows them through a table (vit_h_hop_entry), and the output byte is reversed once.
+// Metrics stay below 12 + 4 * 16 = 76 between renormalisations (every fourth chunk), so 8 bits hold them; their bytes
+// never have bit 7 set, which the chunk-final transpose uses to clear the path bytes (trace_begin).
+//
+// Ring layout and traceback cursor.  The snapshot is taken from the split layout the chunk's last step leaves (Q), so
+// a slot's byte order is a fixed permutation of the states: word w = 8j + i (i < 8, m = 2i) holds states 32j + m,
+// 32j + 16 + m, 32j + m + 1, 32j + m + 17 in bytes 0..3 (vit_h_off).  The traceback cursor points at the byte; a hop is
+//     cursor = hop_base + table[*cursor]
+// where table[b] is the in-slot offset of the predecessor state that path byte b names, and hop_base is the thread's
+// column of the slot the hop lands in: one byte load, one table load and one add, where following the state and slot
+// took ten alu instructions.  Which slot that is does not depend on the data, so the kernels take the bases
+// from per-slot rows (k_viterbi) or count them (k_signal).  A hop that must not move (the traceback is shorter than
+// the hop slots the schedule has) runs through the identity slot: its byte for state x names x, so a hop whose base
+// is the identity slot's lands on the same state there.
+__host__ __device__ constexpr uint32_t vit_h_off(uint32_t x)   // in-slot byte offset of state x (thread column 0)
+{
+    return (8 * (x >> 5) + ((x & 15) >> 1)) * (VIT_BLOCK * 4) + ((x >> 4) & 1) + 2 * (x & 1);
+}
+#define VIT_SLOT_BYTES (16 * VIT_BLOCK * 4)
+#define VIT_HOP_ENTRIES (256 + 64)
+// the hop table: entries 0..255 map a path byte to the offset of the state its decisions of steps 0..5 name (the state
+// eight steps back: the six bits, reversed); entries 256 + l map a best-state label l = 63 - state to its offset
+__device__ __forceinline__ uint32_t vit_h_hop_entry(int i)
+{
+    return vit_h_off(i < 256 ? __brev((uint32_t)i) >> 26 : 63u - (uint32_t)(i - 256));
+}
+// word w of the identity slot: byte k holds the path byte whose predecessor is the state stored there
+__device__ __forceinline__ uint32_t vit_h_identity_word(int w)
+{
+    const uint32_t j = (uint32_t)w >> 3, m = 2u * ((uint32_t)w & 7u);
+    const uint32_t x[4] = {32 * j + m, 32 * j + 16 + m, 32 * j + m + 1, 32 * j + m + 17};
+    uint32_t v = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) v |= (__brev(x[k]) >> 26) << (8 * k);
+    return v;
+}
+
+// k_viterbi's traceback rows: one per (traceback depth ntb, snapshot slot s), 24 in all (ntb 5: rows 0..4, ntb 9:
+// 5..13, ntb 10: 14..23), 12 words each, no thread column:
+//   0     the snapshot's slot s
+//   1     where the cursor starts: slot s, or the identity slot (9, unused at ntb 5 and 9) for the hops that stand still
+//   2..10 the slot each of the chunk's nine hops lands in.  At ntb < 10 the first 10 - ntb hops stand still: they land
+//         in the identity slot, the last of them in slot s.  The others land in s - 1, s - 2, ... (mod ntb), the last
+//         in slot s - (ntb - 1) = s + 1, the next snapshot's
+//   11    the next row (slot s + 1 mod ntb), as its uint4 index
+#define VIT_ROWS 24
+#define VIT_ID_SLOT 9
+// the rows know exactly the traceback depths of the 802.11a/g code rates (1/2: 5, 2/3: 9, 3/4: 10, k_viterbi) and a
+// ring of ten slots, the last of which only ntb = 10 writes; another depth or ring size needs new rows
+static_assert(VIT_NTB_MAX == 10 && VIT_ID_SLOT == VIT_NTB_MAX - 1, "traceback rows assume ntb in {5, 9, 10}, ten ring slots");
+__host__ __device__ constexpr int vit_h_row0(int ntb) { return ntb == 5 ? 0 : (ntb == 9 ? 5 : 14); }
+__device__ __forceinline__ uint32_t vit_h_row_entry(int r, int e)
+{
+    const int ntb = r < 5 ? 5 : (r < 14 ? 9 : 10);
+    const int s = r - vit_h_row0(ntb);
+    int slot;
+    if (e == 0) slot = s;
+    else if (e == 1) slot = ntb == 10 ? s : VIT_ID_SLOT;
+    else if (e <= 10) {
+        const int still = 10 - ntb, i = e - 2;    // hop i; the first `still` hops leave the cursor where it is
+        slot = i < still - 1 ? VIT_ID_SLOT : (s - (i - still + 1) + ntb) % ntb;
+    } else return (uint32_t)(3 * (vit_h_row0(ntb) + (s + 1) % ntb));
+    return (uint32_t)(slot * VIT_SLOT_BYTES);
+}
+
 struct VitCoreH {
     uint32_t X[32];                      // natural order: word j = states 2j (low halfword), 2j + 1 (high)
+    uint32_t Q[32];                      // after step4<4>: the split layout, Q[16j + m] = states 32j + m (low), 32j + 16 + m
 
     __device__ __forceinline__ void init()
     {
@@ -131,11 +195,12 @@ struct VitCoreH {
         v1 = __viaddmax_u16x2(lo, e.x, fadd(hi, e.w));
     }
     static __host__ __device__ constexpr int selc(uint32_t sel) { return (int)((sel & 0xfu) >> 1); }
-    // bt: the table, uint4 [8][4][16]
+    // bt: the table, uint4 [8][4][16].  step4<0> ends in natural order (X); step4<4>, the chunk's last four steps,
+    // leaves the split layout Q for trace_begin, which snapshots it and transposes it.
     template <int S0>
     __device__ __forceinline__ void step4(const uint4 *bt, uint32_t n0, uint32_t n1, uint32_t n2, uint32_t n3)
     {
-        uint32_t S[32], Q[32];
+        uint32_t S[32];
         uint4 e[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) e[c] = bt[((S0 + 0) * 4 + c) * 16 + n0];
@@ -162,39 +227,48 @@ struct VitCoreH {
 #pragma unroll
             for (int o = 0; o < 8; ++o)
                 bflyt(e[selc(vit_sel2(16 * j + o, 16 * j + 8 + o))], S[8 * j + o], S[8 * (j + 2) + o], Q[16 * j + 2 * o], Q[16 * j + 2 * o + 1]);
+        if (S0 == 0) {
+#pragma unroll
+            for (int j = 0; j < 2; ++j)
+#pragma unroll
+                for (int e2 = 0; e2 < 16; e2 += 2) {
+                    X[(32 * j + e2) >> 1] = prmt(Q[16 * j + e2], Q[16 * j + e2 + 1], 0x5410u);
+                    X[(32 * j + 16 + e2) >> 1] = prmt(Q[16 * j + e2], Q[16 * j + e2 + 1], 0x7632u);
+                }
+        }
+    }
+    // end of a chunk, after step4<4>: snapshot the path bytes (at byte offset `snap` of the ring, the thread's column of
+    // the slot; layout see vit_h_off), transpose to natural order with the path bytes cleared, first best state,
+    // optional renormalisation.  Returns the traceback cursor: the best state's byte in the slot whose thread column
+    // starts at c0_base (the snapshot's, or the identity slot's).  keep: mask applied to the path bytes first (0xff;
+    // 0xfc after the 6-step first chunk, which runs as two erased steps + 6).
+    __device__ __forceinline__ uint32_t trace_begin(uint8_t *snap, uint32_t c0_base, const uint32_t *hop_tab, bool renorm,
+                                                    uint32_t keep = 0xffu)
+    {
+        const uint32_t keepw = 0xff00ff00u | keep | (keep << 16);
+#pragma unroll
+        for (int w = 0; w < 16; ++w)
+            *reinterpret_cast<uint32_t *>(snap + w * (VIT_BLOCK * 4)) = prmt(Q[2 * w] & keepw, Q[2 * w + 1] & keepw, 0x6420u);
+        // the transpose of step4<0>, with selector nibbles 8 | i (replicate the sign bit of byte i) for the path bytes:
+        // byte i is the state's metric byte, below 0x80, so the path bytes come out cleared
 #pragma unroll
         for (int j = 0; j < 2; ++j)
 #pragma unroll
             for (int e2 = 0; e2 < 16; e2 += 2) {
-                X[(32 * j + e2) >> 1] = prmt(Q[16 * j + e2], Q[16 * j + e2 + 1], 0x5410u);
-                X[(32 * j + 16 + e2) >> 1] = prmt(Q[16 * j + e2], Q[16 * j + e2 + 1], 0x7632u);
+                X[(32 * j + e2) >> 1] = prmt(Q[16 * j + e2], Q[16 * j + e2 + 1], 0x5d19u);
+                X[(32 * j + 16 + e2) >> 1] = prmt(Q[16 * j + e2], Q[16 * j + e2 + 1], 0x7f3bu);
             }
-    }
-    // end of a chunk: snapshot the path bytes (ring slot `slot`, one byte per state, see vit_ring_byte), first best
-    // state, optional renormalisation, path bytes cleared.  keep: mask applied to the path bytes first (0xff; 0xfc after
-    // the 6-step first chunk, which runs as two erased steps + 6).
-    __device__ __forceinline__ VitTrace trace_begin(uint32_t *ring, int slot, int ntb, int tid, bool renorm, uint32_t keep = 0xffu)
-    {
-        const uint32_t keepw = 0xff00ff00u | keep | (keep << 16);
-#pragma unroll
-        for (int w = 0; w < 16; ++w) ring[(slot * 16 + w) * VIT_BLOCK + tid] = prmt(X[2 * w] & keepw, X[2 * w + 1] & keepw, 0x6420u);
-        // path bytes cleared; keys (metric << 8) | (63 - state) -- the largest key is the largest metric at the smallest
-        // state -- are the cleared words plus the state labels (an add: fma pipe, where a permute would be alu)
+        // keys (metric << 8) | (63 - state) -- the largest key is the largest metric at the smallest state -- are the
+        // cleared words plus the state labels (an add: fma pipe, where a permute would be alu)
         uint32_t key[32];
 #pragma unroll
-        for (int j = 0; j < 32; ++j) {
-            X[j] &= 0xff00ff00u;
-            key[j] = fadd(X[j], (uint32_t)(63 - 2 * j) | ((uint32_t)(62 - 2 * j) << 16));
-        }
+        for (int j = 0; j < 32; ++j) key[j] = fadd(X[j], (uint32_t)(63 - 2 * j) | ((uint32_t)(62 - 2 * j) << 16));
 #pragma unroll
         for (int n = 16; n >= 1; n >>= 1)
 #pragma unroll
             for (int i = 0; i < n; ++i) key[i] = __vmaxu2(key[i], key[i + n]);
         const uint32_t kbest = max(key[0] & 0xffffu, key[0] >> 16);
-        VitTrace t;
-        t.bs = 63 - (int)(kbest & 0xffu);
-        t.sl = slot;
-        t.left = ntb - 1;
+        const uint32_t c = c0_base + hop_tab[256 + (kbest & 0xffu)];
         if (renorm) {
             // Only metric differences matter (upstream subtracts the minimum after every chunk).  Any state is reached
             // from any other in K - 1 = 6 steps of at most 2 agreements each, so min >= max - 12: subtracting max - 12
@@ -204,27 +278,31 @@ struct VitCoreH {
 #pragma unroll
             for (int i = 0; i < 32; ++i) X[i] = fadd(X[i], nminw);
         }
-        return t;
+        return c;
     }
-    // ring bytes hold the decisions in ascending bit order: the state eight steps back is the byte reversed, >> 2
-    template <int N>
-    static __device__ __forceinline__ void trace_hops(VitTrace &t, const uint32_t *ring, int ntb, int tid)
+    // Cursors and bases are shared-window addresses, read with explicit ld.shared: as C++ pointers, the compiler
+    // re-associates base + table entry into ring + (thread column + slot + entry) and spends a second add per hop.
+    // One traceback hop (see the top of VitCoreH): to the byte of the predecessor state in the slot column at `base`.
+    // hop_tab: the shared-window address of the hop table.  The first hop after trace_begin reads a byte of the
+    // snapshot trace_begin has just stored with plain C++ stores; a caller that does so in straight-line code (k_signal)
+    // puts a compiler memory barrier between them.  (In k_viterbi the snapshot is stored at the end of one loop trip and
+    // read in the next.)
+    static __device__ __forceinline__ uint32_t hop(uint32_t c, uint32_t hop_tab, uint32_t base)
     {
-#pragma unroll
-        for (int i = 0; i < N; ++i) {
-            const bool go = t.left > 0;
-            const int nb = (int)(__brev(vit_ring_byte(ring, t.sl, t.bs, tid)) >> 26);
-            const int ns = (t.sl == 0) ? ntb - 1 : t.sl - 1;
-            t.bs = go ? nb : t.bs;
-            t.sl = go ? ns : t.sl;
-            t.left -= go ? 1 : 0;
-        }
+        uint32_t b, t;
+        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(b) : "r"(c));
+        asm("ld.shared.u32 %0, [%1];" : "=r"(t) : "r"(hop_tab + 4u * b));
+        return base + t;
+    }
+    // the byte at the cursor; the "memory" clobber keeps it ahead of the snapshot that overwrites its slot
+    static __device__ __forceinline__ uint32_t ring_byte(uint32_t c)
+    {
+        uint32_t b;
+        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(b) : "r"(c) : "memory");
+        return b;
     }
     // the chunk's output byte in upstream's bit order (MSB = earliest decision)
-    static __device__ __forceinline__ uint32_t trace_finish(const VitTrace &t, const uint32_t *ring, int tid)
-    {
-        return __brev(vit_ring_byte(ring, t.sl, t.bs, tid)) >> 24;
-    }
+    static __device__ __forceinline__ uint32_t trace_finish(uint32_t c) { return __brev(ring_byte(c)) >> 24; }
 };
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -161,8 +161,9 @@ const char *STAGE_NAMES[ST_COUNT] = {"h2d", "detect", "select", "sync_long", "de
 #endif
 #define VQ_SPLIT_MAX 4736        // frames beyond a step of the per-thread kernel's staircase that get their own launch (run_rx)
 #define DET_SMEM DET_SMEM_BYTES
-// k_viterbi: ring, CRC table, descrambler table, branch-word table (8 x 4 x 16 entries of 16 bytes): 50432 bytes, 4 blocks per SM
-#define VIT_SMEM_BYTES ((VIT_NTB_MAX * 16 * VIT_BLOCK + 256) * 4 + 256 + 8192)
+// k_viterbi: ring, CRC table, descrambler table, branch-word table (8 x 4 x 16 entries of 16 bytes), traceback rows
+// (24 x 48 bytes), hop table (320 words): 52864 bytes, 4 blocks per SM
+#define VIT_SMEM_BYTES ((VIT_NTB_MAX * 16 * VIT_BLOCK + 256) * 4 + 256 + 8192 + VIT_ROWS * 48 + VIT_HOP_ENTRIES * 4)
 
 } // namespace
 
