@@ -1263,21 +1263,94 @@ __global__ void __launch_bounds__(256) k_pack(const JobDesc *__restrict__ jobs, 
 
 // ------------------------------------------------------------------ R6a-c Viterbi + descramble + CRC
 // One thread per frame slot; jobs[frame].n_sym == 0 means nothing to decode.  Trellis words of the
-// frame are contiguous (vit_in[frame][w]); words past the coded data read as 0 (oracle note 2).
-__global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict__ jobs, int f0, int n_frames, const uint32_t *__restrict__ vit_in,
-                                                        uint32_t *__restrict__ psdu, wifi_b200_frame *frames)
+// frame are contiguous (in[frame][w]); words past the coded data read as 0 (oracle note 2).
+// viterbi_body is the kernel of both one-trellis-per-thread decoders: k_viterbi (hard decisions, VitCoreH) and
+// k_viterbi_soft (soft decisions, VitCoreS).  A reader, VitHardIn or VitSoftIn, names the core and feeds it its
+// input: chunk 0 (6 steps, run as two erased steps + 6) in first(), then the eight steps of each further chunk as
+// fetch() and two four-step halves; prefetch() runs once between them.
+
+// hard decisions (k_pack, k_demod): one word of eight steps x two 2-bit symbols (2 = erased) per word; chunk j >= 1 is
+// the last two steps of word j - 1 and the first six of word j.  VitCoreH reads its branch words from the table.
+struct VitHardIn {
+    using Core = VitCoreH;
+    static constexpr int MAXW = VIT_MAXW, BM = 512;   // words per job; entries of the branch-word table
+    static __device__ __forceinline__ uint4 table_entry(int i) { return VitCoreH::table_entry(i >> 6, (i >> 4) & 3, (uint32_t)(i & 15)); }
+    static __device__ __forceinline__ int words(const JobDesc &J) { return (J.n_sym * c_tab.mcs[J.enc].n_dbps + 7) >> 3; }
+    const uint32_t *in;
+    int nw;
+    const uint4 *bm;
+    uint32_t prev, next, bits;
+    __device__ __forceinline__ void first(VitCoreH &v)
+    {
+        prev = in[0];
+        v.step4<0>(bm, 0xau, 0xau, prev & 0xfu, (prev >> 4) & 0xfu);
+        v.step4<4>(bm, (prev >> 8) & 0xfu, (prev >> 12) & 0xfu, (prev >> 16) & 0xfu, (prev >> 20) & 0xfu);
+    }
+    // word 1, read ahead for chunk 1.  Loaded here, after chunk 0's snapshot, rather than in first(): the earlier load
+    // changes ptxas's register allocation of the whole kernel
+    __device__ __forceinline__ void prefetch() { next = 1 < nw ? in[1] : 0u; }
+    __device__ __forceinline__ void fetch(int chunk)
+    {
+        bits = __funnelshift_r(prev, next, 24);
+        prev = next;
+        next = (chunk + 1 < nw) ? in[chunk + 1] : 0u;
+    }
+    template <int H>
+    __device__ __forceinline__ void half(VitCoreH &v)
+    {
+        const uint32_t b = bits >> (16 * H);
+        v.step4<4 * H>(bm, b & 0xfu, (b >> 4) & 0xfu, (b >> 8) & 0xfu, (b >> 12) & 0xfu);
+    }
+};
+
+// soft decisions (k_pack_soft, k_demod): one word of two steps x two int8 soft values (0 = erased); chunk j >= 1 is
+// words 4j - 1 .. 4j + 2.  No branch-word table.
+struct VitSoftIn {
+    using Core = VitCoreS;
+    static constexpr int MAXW = SOFT_MAXW, BM = 0;
+    static __device__ __forceinline__ int words(const JobDesc &J) { return J.n_sym * (c_tab.mcs[J.enc].n_dbps >> 1); }
+    const uint32_t *in;
+    int nw;
+    const uint4 *bm;                      // unused: no branch-word table
+    uint32_t w[4];
+    __device__ __forceinline__ uint32_t at(int i) const { return i < nw ? in[i] : 0u; }
+    __device__ __forceinline__ void first(VitCoreS &v)
+    {
+        v.step4<0>(0u, at(0));            // soft value 0: every branch value is 254, every candidate ties
+        v.step4<4>(at(1), at(2));
+    }
+    __device__ __forceinline__ void prefetch() {}   // fetch() reads a chunk's words itself
+    __device__ __forceinline__ void fetch(int chunk)
+    {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) w[k] = at(4 * chunk - 1 + k);
+    }
+    template <int H>
+    __device__ __forceinline__ void half(VitCoreS &v) { v.step4<4 * H>(w[2 * H], w[2 * H + 1]); }
+};
+
+// dynamic shared memory of viterbi_body: ring, CRC table, descrambler table, the reader's branch-word table (16 bytes an
+// entry), traceback rows (24 x 48 bytes), hop table (320 words): 52864 bytes for k_viterbi (4 blocks per SM), 44672
+// for k_viterbi_soft
+template <class In>
+constexpr int vit_smem_bytes() { return (VIT_NTB_MAX * 16 * VIT_BLOCK + 256) * 4 + 256 + In::BM * 16 + VIT_ROWS * 48 + VIT_HOP_ENTRIES * 4; }
+
+// tid: threadIdx.x as the kernel reads it, where __launch_bounds__ tells the compiler that it is below VIT_BLOCK
+template <class In>
+__device__ __forceinline__ void viterbi_body(int tid, const JobDesc *__restrict__ jobs, int f0, int n_frames, const uint32_t *__restrict__ vin,
+                                             uint32_t *__restrict__ psdu, wifi_b200_frame *frames)
 {
     extern __shared__ uint32_t vsm[];
     uint32_t *ring = vsm;                                   // VIT_NTB_MAX*16*VIT_BLOCK words
     uint32_t *s_crc = vsm + VIT_NTB_MAX * 16 * VIT_BLOCK;   // 256
     uint16_t *s_scr = (uint16_t *)(s_crc + 256);            // 128
-    uint4 *s_bm = (uint4 *)(s_crc + 256 + 64);              // branch-word table [8 steps][4 selectors][16 symbol pairs] (VitCoreH::table_entry)
-    uint4 *s_rows = s_bm + 512;                             // traceback rows [VIT_ROWS][3] (vit_h_row_entry)
+    uint4 *s_bm = (uint4 *)(s_crc + 256 + 64);              // branch-word table, In::BM entries (VitCoreH::table_entry)
+    uint4 *s_rows = s_bm + In::BM;                          // traceback rows [VIT_ROWS][3] (vit_h_row_entry)
     uint32_t *s_hop = (uint32_t *)(s_rows + 3 * VIT_ROWS);  // hop table (vit_h_hop_entry)
-    const int tid = threadIdx.x;
     for (int i = tid; i < 256; i += VIT_BLOCK) s_crc[i] = c_tab.crc_tab[i];
     for (int i = tid; i < 128; i += VIT_BLOCK) s_scr[i] = c_tab.scr_tab[i];
-    for (int i = tid; i < 512; i += VIT_BLOCK) s_bm[i] = VitCoreH::table_entry(i >> 6, (i >> 4) & 3, (uint32_t)(i & 15));
+    if constexpr (In::BM > 0)
+        for (int i = tid; i < In::BM; i += VIT_BLOCK) s_bm[i] = In::table_entry(i);
     for (int i = tid; i < 12 * VIT_ROWS; i += VIT_BLOCK) ((uint32_t *)s_rows)[i] = vit_h_row_entry(i / 12, i % 12);
     for (int i = tid; i < VIT_HOP_ENTRIES; i += VIT_BLOCK) s_hop[i] = vit_h_hop_entry(i);
     // the identity slot, in every thread's column (a frame with ntb = 10 overwrites it with snapshots and never reads it
@@ -1290,20 +1363,17 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict
     if (J.n_sym == 0) return;
     const int punct = c_tab.mcs[J.enc].punct;
     const int ntb = punct == 0 ? 5 : (punct == 1 ? 9 : 10);   // the three depths the traceback rows know (vit_h_row_entry)
-    const int nw = (J.n_sym * c_tab.mcs[J.enc].n_dbps + 7) >> 3;
-    const uint32_t *in = vit_in + (int64_t)job * VIT_MAXW;
+    In f{vin + (int64_t)job * In::MAXW, In::words(J), s_bm};
     uint32_t *out = psdu + (int64_t)job * (PSDU_STRIDE / 4);
     const int L = J.len;
     const int last_chunk = L + 1 + ntb;   // chunk whose traceback yields PSDU byte L-1
-    VitCoreH v;
+    typename In::Core v;
     v.init();
-    uint32_t prev = in[0];
-    // chunk 0 has 6 steps: two erased steps in front of them leave the all-zero metrics as they are and set bits 0, 1 of
-    // every path byte, which trace_begin masks off (keep = 0xfc)
-    v.step4<0>(s_bm, 0xau, 0xau, prev & 0xfu, (prev >> 4) & 0xfu);
-    v.step4<4>(s_bm, (prev >> 8) & 0xfu, (prev >> 12) & 0xfu, (prev >> 16) & 0xfu, (prev >> 20) & 0xfu);
+    // chunk 0 has 6 steps: two erased steps in front of them leave all metrics equal and set bits 0, 1 of every path
+    // byte, which trace_begin masks off (keep = 0xfc)
+    f.first(v);
     // the traceback of chunk j - 1 (snapshot slot s = j mod ntb, row `row`) runs interleaved with the trellis steps of
-    // chunk j, three hops before each step4 and three before the output byte; the cursor `c` is a ring byte offset
+    // chunk j, three hops before each half and three before the output byte; the cursor `c` is a ring byte offset
     // (VitCoreH), the hops' slots come from the row
     uint8_t *rbt = reinterpret_cast<uint8_t *>(ring) + 4 * tid;   // the thread's column of slot 0
     const uint32_t rbt_sh = (uint32_t)__cvta_generic_to_shared(rbt), hop_sh = (uint32_t)__cvta_generic_to_shared(s_hop);
@@ -1312,21 +1382,19 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict
     uint32_t c = v.trace_begin(rbt + r0.x, rbt_sh + r0.y, s_hop, true, 0xfcu);
     PsduSink sink;
     sink.init(out, L, s_crc, s_scr);
-    uint32_t next = 1 < nw ? in[1] : 0u;
+    f.prefetch();
 #pragma unroll 1
     for (int chunk = 1; chunk <= last_chunk; ++chunk) {
-        uint32_t bits = __funnelshift_r(prev, next, 24);
-        prev = next;
-        next = (chunk + 1 < nw) ? in[chunk + 1] : 0u;
+        f.fetch(chunk);
         const uint4 r1 = s_rows[row + 1], r2 = s_rows[row + 2];
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r0.z);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r0.w);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.x);
-        v.step4<0>(s_bm, bits & 0xfu, (bits >> 4) & 0xfu, (bits >> 8) & 0xfu, (bits >> 12) & 0xfu);
+        f.template half<0>(v);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.y);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.z);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r1.w);
-        v.step4<4>(s_bm, (bits >> 16) & 0xfu, (bits >> 20) & 0xfu, (bits >> 24) & 0xfu, bits >> 28);
+        f.template half<1>(v);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r2.x);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r2.y);
         c = VitCoreH::hop(c, hop_sh, rbt_sh + r2.z);
@@ -1343,6 +1411,19 @@ __global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict
         sink.push(VitCoreH::trace_finish(c), last_chunk - ntb);
     }
     frames[J.frame].crc_ok = sink.crc_ok();
+}
+
+__global__ void __launch_bounds__(VIT_BLOCK) k_viterbi(const JobDesc *__restrict__ jobs, int f0, int n_frames, const uint32_t *__restrict__ vit_in,
+                                                        uint32_t *__restrict__ psdu, wifi_b200_frame *frames)
+{
+    viterbi_body<VitHardIn>(threadIdx.x, jobs, f0, n_frames, vit_in, psdu, frames);
+}
+
+// soft-decision mode (DESIGN.md 9)
+__global__ void __launch_bounds__(VIT_BLOCK) k_viterbi_soft(const JobDesc *__restrict__ jobs, int f0, int n_frames, const uint32_t *__restrict__ vit_soft_in,
+                                                             uint32_t *__restrict__ psdu, wifi_b200_frame *frames)
+{
+    viterbi_body<VitSoftIn>(threadIdx.x, jobs, f0, n_frames, vit_soft_in, psdu, frames);
 }
 
 // ------------------------------------------------------------------ R6a-c, four lanes per trellis (middle-sized calls)
@@ -1394,7 +1475,7 @@ __global__ void __launch_bounds__(VQ_BLOCK) k_viterbi_quad(const JobDesc *__rest
     sink.init(psdu + (int64_t)(active ? job : f0) * (PSDU_STRIDE / 4), L, s_crc, s_scr);
     sink.writer = active && (tid & 3) == 0;
     uint32_t next = 1 < nw ? in[1] : 0u;
-    VitTrace tr;
+    VitQuad::Trace tr;
     tr.bs = 0; tr.sl = slot; tr.left = 0;
 #pragma unroll 1
     for (int chunk = 1; chunk <= trips; ++chunk) {
@@ -1549,65 +1630,4 @@ __global__ void __launch_bounds__(256) k_pack_soft(const JobDesc *__restrict__ j
             vw[w] = word;
         }
     }
-}
-
-__global__ void __launch_bounds__(VIT_BLOCK) k_viterbi_soft(const JobDesc *__restrict__ jobs, int f0, int n_frames, const uint32_t *__restrict__ vit_soft_in,
-                                                             uint32_t *__restrict__ psdu, wifi_b200_frame *frames)
-{
-    extern __shared__ uint32_t vsm[];
-    uint32_t *ring = vsm;
-    uint32_t *s_crc = vsm + VIT_NTB_MAX * 16 * VIT_BLOCK;
-    uint16_t *s_scr = (uint16_t *)(s_crc + 256);
-    const int tid = threadIdx.x;
-    for (int i = tid; i < 256; i += VIT_BLOCK) s_crc[i] = c_tab.crc_tab[i];
-    for (int i = tid; i < 128; i += VIT_BLOCK) s_scr[i] = c_tab.scr_tab[i];
-    __syncthreads();
-    const int job = f0 + blockIdx.x * VIT_BLOCK + tid;
-    if (job >= n_frames) return;
-    const JobDesc J = jobs[job];
-    if (J.n_sym == 0) return;
-    const int punct = c_tab.mcs[J.enc].punct;
-    const int ntb = punct == 0 ? 5 : (punct == 1 ? 9 : 10);
-    const int nw = J.n_sym * (c_tab.mcs[J.enc].n_dbps >> 1);     // data words, 2 steps each; later words read 0
-    const uint32_t *in = vit_soft_in + (int64_t)job * SOFT_MAXW;
-    const int L = J.len;
-    const int last_chunk = L + 1 + ntb;
-    VitCoreSoft v;
-    v.init();
-    PsduSink sink;
-    sink.init(psdu + (int64_t)job * (PSDU_STRIDE / 4), L, s_crc, s_scr);
-    // chunk 0 has 6 steps: two erased steps (soft value 0: every branch metric 254, so every candidate ties) in front of
-    // them leave every metric equal and set bits 7, 6 of every path byte, which are masked off; the renormalisation
-    // removes the uniform +508
-    v.step4<0>(0u, 0 < nw ? in[0] : 0u);
-    v.step4<4>(1 < nw ? in[1] : 0u, 2 < nw ? in[2] : 0u);
-#pragma unroll
-    for (int i = 0; i < 32; ++i) v.P[i] &= 0x003f003fu;
-    int slot = 1 % ntb;
-    v.trace_begin(ring, slot, ntb, tid, true);
-    int wi = 3;
-    VitTrace tr;
-    tr.bs = 0; tr.sl = slot; tr.left = 0;
-    bool pending = false;
-#pragma unroll 1
-    for (int chunk = 1; chunk <= last_chunk; ++chunk) {
-        uint32_t w4[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) w4[k] = (wi + k < nw) ? in[wi + k] : 0u;
-        wi += 4;
-        VitCoreSoft::trace_hops<3>(tr, ring, ntb, tid);
-        v.step4<0>(w4[0], w4[1]);
-        VitCoreSoft::trace_hops<3>(tr, ring, ntb, tid);
-        v.step4<4>(w4[2], w4[3]);
-        VitCoreSoft::trace_hops<3>(tr, ring, ntb, tid);
-        if (pending && chunk - 1 >= ntb) sink.push(vit_ring_byte(ring, tr.sl, tr.bs, tid), chunk - 1 - ntb);
-        slot = (slot + 1 == ntb) ? 0 : slot + 1;
-        tr = v.trace_begin(ring, slot, ntb, tid, (chunk & 1) == 0);
-        pending = true;
-    }
-    if (pending && last_chunk >= ntb) {
-        VitCoreSoft::trace_hops<9>(tr, ring, ntb, tid);
-        sink.push(vit_ring_byte(ring, tr.sl, tr.bs, tid), last_chunk - ntb);
-    }
-    frames[J.frame].crc_ok = sink.crc_ok();
 }

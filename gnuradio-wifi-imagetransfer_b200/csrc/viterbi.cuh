@@ -12,16 +12,18 @@
 //   VitQuad   one trellis per FOUR lanes (k_viterbi_quad), byte-packed metrics and path bytes (4 states per register),
 //             two quad exchanges per 4 steps;
 //   (k_viterbi_warp, rx_kernels.cuh: one trellis per warp.)
-// VitCoreSoft is the soft-decision decoder (k_viterbi_soft): 16-bit metrics and path halfwords, two states per register.
+// VitCoreS is the soft-decision decoder (k_viterbi_soft): one trellis per thread, VitCoreH's survivor words with 16-bit
+// metrics, one state per register, and VitCoreH's traceback.
 //
-// VitCoreH, VitQuad and VitCoreSoft run the trellis four steps at a time (step4) with one re-layout instead of four.
+// VitCoreH and VitQuad run the trellis four steps at a time (step4) with one re-layout instead of four.
 // A butterfly leaves its survivors split into "new even states" and "new odd states" words; instead of interleaving
 // them back to natural order after every step, the next steps pair the split words directly -- the state stride inside
 // a word doubles each step: 1 (natural) -> 2 -> 4 -> 8 -> 16 -- and one transpose restores natural order after the
-// fourth step.  Chunks are 8 steps, so the best-state search always sees the natural layout, and so do the snapshots
-// of VitQuad and VitCoreSoft (VitCoreH snapshots the split layout in front of the transpose).  The path
-// bytes are never shifted: step s of a chunk sets its own decision bit.  Chunk 0 has 6 steps; it runs as two erased
-// steps + 6, whose two extra decision bits are masked off before the snapshot (see the kernels).
+// fourth step.  Chunks are 8 steps, so the best-state search always sees the natural layout, and so does the snapshot
+// of VitQuad (VitCoreH snapshots the split layout in front of the transpose).  VitCoreS needs no re-layout: with one
+// state per register a step only renames registers.  The path bytes are never shifted: step s of a chunk sets its own
+// decision bit.  Chunk 0 has 6 steps; it runs as two erased steps + 6, whose two extra decision bits are masked off
+// before the snapshot (see the kernels).
 // Path snapshots of the per-thread forms go to shared memory, word-interleaved across the block's threads (bank =
 // thread id, conflict free).
 #pragma once
@@ -54,16 +56,8 @@ __host__ __device__ constexpr uint32_t vit_sel2(int k0, int k1)
 // The traceback of one chunk is a chain of dependent shared-memory reads.  trace_begin() stores the snapshot and finds
 // the first best state; the hops follow (branch-free, so the scheduler can interleave the chain with the next chunk's
 // add-compare-select work); then the output byte is read.  That read must come before the next snapshot is stored:
-// the byte lives in the slot it overwrites.  VitQuad and VitCoreSoft keep the cursor as VitTrace (state, ring slot,
-// hops left) and step it with trace_hops(); VitCoreH's cursor is a byte address (see there).
-struct VitTrace { int bs, sl, left; };
-// byte (slot, state) of this thread's ring: the ring is word-interleaved across the block's threads,
-// word (slot * 16 + state / 4) * VIT_BLOCK + tid, so the path byte is a single byte load
-__device__ __forceinline__ uint32_t vit_ring_byte(const uint32_t *ring, int sl, int bs, int tid)
-{
-    const uint8_t *rb = reinterpret_cast<const uint8_t *>(ring) + tid * 4;
-    return rb[sl * (16 * VIT_BLOCK * 4) + (bs >> 2) * (VIT_BLOCK * 4) + (bs & 3)];
-}
+// the byte lives in the slot it overwrites.  VitCoreH's (and VitCoreS's) cursor is a byte address (see VitCoreH);
+// VitQuad keeps it as VitQuad::Trace (state, ring slot, hops left) and steps it with trace_hops().
 
 // ---------------------------------------------------------------------------------------------------------------
 // VitCoreH: the per-thread decoder with metric and path byte of a state in ONE halfword, two states per register:
@@ -170,8 +164,8 @@ struct VitCoreH {
         return d;
     }
     // ---- branch words from a table ----
-    // Every stage of the four-step schedule (the one of VitCoreSoft::step4: stride inside a word 1 -> 2 -> 4 -> 8 -> 16,
-    // then a halfword transpose per word pair) uses exactly four selectors (two complementary pairs), distinguished by the
+    // Every stage of the four-step schedule (stride inside a word 1 -> 2 -> 4 -> 8 -> 16, then a halfword transpose per
+    // word pair) uses exactly four selectors (two complementary pairs), distinguished by the
     // expected pair of their low-halfword butterfly (c = 2A + B of k0); the high halfword's is c ^ 1 in stage A, 3 - c in
     // stages B and C, c in stage D.  table[s][c][nibble] = (svm, sv, svm + BIT_s, sv + BIT_s) for step s of a chunk:
     // one LDS.128 replaces the permute and the three adds per selector and step (the lsu pipe is idle, the alu pipe is
@@ -336,6 +330,7 @@ struct VitCoreH {
 #define VQ_RSTRIDE (VIT_NTB_MAX * 16 + 4) // ring words per frame; 164 = 4 (mod 32): the 8 quads x 4 lanes of a warp hit 32 banks
 
 struct VitQuad {
+    struct Trace { int bs, sl, left; };  // traceback cursor: state, ring slot, hops left
     uint32_t m[4], p[4];
     uint32_t selA0, selA1, selB0, selB1, selC0, selC1, selD0, selD1;
     uint32_t keyc[4];                    // state labels (63 - state) of local word i, for the best-state keys
@@ -454,7 +449,7 @@ struct VitQuad {
 
     // ring: this frame's VIT_NTB_MAX x 16 words (natural order).  All four lanes follow the traceback (same addresses:
     // broadcast reads), so no lane waits for another's result.
-    __device__ __forceinline__ VitTrace trace_begin(uint32_t *ring, int slot, int ntb, bool renorm)
+    __device__ __forceinline__ Trace trace_begin(uint32_t *ring, int slot, int ntb, bool renorm)
     {
         __syncwarp();                                        // the quad is done reading the slot this snapshot replaces
 #pragma unroll
@@ -473,7 +468,7 @@ struct VitQuad {
         kbest = max(kbest, __shfl_xor_sync(0xffffffffu, kbest, 1));
         kbest = max(kbest, __shfl_xor_sync(0xffffffffu, kbest, 2));  // (also orders the snapshot stores before the quad's reads)
         __syncwarp();
-        VitTrace t;
+        Trace t;
         t.bs = 63 - (int)(kbest & 0xffu);
         t.sl = slot;
         t.left = ntb - 1;
@@ -492,7 +487,7 @@ struct VitQuad {
         return reinterpret_cast<const uint8_t *>(ring)[sl * 64 + bs];
     }
     template <int N>
-    static __device__ __forceinline__ void trace_hops(VitTrace &t, const uint32_t *ring, int ntb)
+    static __device__ __forceinline__ void trace_hops(Trace &t, const uint32_t *ring, int ntb)
     {
 #pragma unroll
         for (int i = 0; i < N; ++i) {
@@ -542,143 +537,82 @@ struct PsduSink {
     __device__ __forceinline__ int crc_ok() const { return ((crc ^ 0xffffffffu) == 558161692u) ? 1 : 0; }
 };
 
-// Soft-decision variant (oracle viterbi_soft): 16-bit path metrics, two states per register, branch
-// metric = correlation of the expected output bits with int8 soft inputs, offset +254 per step.
-struct VitCoreSoft {
-    uint32_t M[32], P[32];
+// ---------------------------------------------------------------------------------------------------------------
+// VitCoreS: the soft-decision decoder (k_viterbi_soft; oracle viterbi_soft) in VitCoreH's idiom, one state per register:
+//     word = metric << 16 | path byte,   the decision of step s of a chunk at bit s of the path byte (ascending).
+// The branch value is the correlation of the expected code bits (A, B) with the step's two int8 soft values, + 254:
+//     x = (A ? q0 : -q0) + (B ? q1 : -q1) + 254,   y = 508 - x
+//     new[2k] = max(old[k] + x, old[k + 32] + y),   new[2k + 1] = max(old[k] + y, old[k + 32] + x).
+// The candidate from state k + 32 also carries the step's decision bit, and every later bit of both candidates' path
+// bytes is still zero, so among equal metrics it is the larger word: one unsigned maximum (VIADDMNMX.U32, which also adds
+// one candidate's branch value) and one add per new state are the compare, upstream's tie rule (-> k + 32) and the
+// selection of metric and path.  With one state per register a step is a renaming of registers, so there is no
+// re-layout.  The snapshot goes to the ring in vit_h_off's order, so VitCoreH's hop table, traceback rows, identity
+// slot, hop() and trace_finish() serve this core unchanged.
+// Metric bound: k_demod's soft values lie within +-32 (any int8 but -128 keeps a branch value in 0 .. 508), so a
+// branch value is at most 510; any state reaches any other in K - 1 = 6 steps, so min >= max - 6 * 510.
+#define VIT_S_SPREAD (6 * 510)
+// renormalised by max - VIT_S_SPREAD every fourth chunk, metrics stay below VIT_S_SPREAD + 4 * 8 * 510 = 19380
+static_assert(VIT_S_SPREAD + 4 * 8 * 510 < 65536, "soft metrics must fit 16 bits between renormalisations");
+struct VitCoreS {
+    uint32_t X[64];                      // X[x]: the survivor word of state x
 
     __device__ __forceinline__ void init()
     {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) { M[i] = 0; P[i] = 0; }
+        for (int i = 0; i < 64; ++i) X[i] = 0;
     }
-    // BIT: position of this step's decision in the path halfword (never shifted, see VitQuad::bfly)
-    template <uint32_t BIT>
-    static __device__ __forceinline__ void bfly(uint32_t Tlo, uint32_t Thi, uint32_t sel, uint32_t lo, uint32_t hi, uint32_t plo, uint32_t phi,
-                                                uint32_t &v0, uint32_t &v1, uint32_t &p0, uint32_t &p1)
-    {
-        const uint32_t x = prmt(Tlo, Thi, sel), y = 0x01fc01fcu - x;
-        const uint32_t m0 = lo + x, m1 = hi + y, m2 = lo + y, m3 = hi + x;
-        const uint32_t k0 = prmt(m0 + 0x7fff7fffu - m1, 0u, 0xbb99u);
-        const uint32_t k1 = prmt(m2 + 0x7fff7fffu - m3, 0u, 0xbb99u);
-        v0 = (m0 & k0) | (m1 & ~k0);
-        v1 = (m2 & k1) | (m3 & ~k1);
-        const uint32_t pb = phi + BIT;
-        p0 = (plo & k0) | (pb & ~k0);
-        p1 = (plo & k1) | (pb & ~k1);
-    }
-    static __device__ __forceinline__ void branch(int q0, int q1, uint32_t &Tlo, uint32_t &Thi)
-    {
-        const uint32_t t11 = (uint32_t)(q0 + q1 + 254), t00 = 508u - t11;
-        const uint32_t t10 = (uint32_t)(q0 - q1 + 254), t01 = 508u - t10;
-        Tlo = t00 | (t01 << 16);
-        Thi = t10 | (t11 << 16);
-    }
-    // Four steps with one re-layout (see the top of this file): with two states per word the stride inside a
-    // word goes 1 -> 2 -> 4 -> 8 -> 16 and one halfword transpose per word pair restores natural order.
-    // w0 / w1: the two input words (2 steps x 2 int8 each).
+    // steps S0 .. S0 + 3 of a chunk; w0, w1: two input words of two steps x (q0, q1) int8 each (k_pack_soft)
     template <int S0>
     __device__ __forceinline__ void step4(uint32_t w0, uint32_t w1)
     {
-        constexpr uint32_t B0 = 0x00010001u << (7 - S0), B1 = B0 >> 1, B2 = B0 >> 2, B3 = B0 >> 3;
-        uint32_t Tlo, Thi;
-        uint32_t S[32], SP[32], Q[32], QP[32];
-        // A: natural, pair j: k = 2j + b -> S[j] = {4j, 4j+2}, S[16+j] = {4j+1, 4j+3}
-        branch((int)(int8_t)(w0 & 0xffu), (int)(int8_t)((w0 >> 8) & 0xffu), Tlo, Thi);
 #pragma unroll
-        for (int j = 0; j < 16; ++j) bfly<B0>(Tlo, Thi, vit_sel2(2 * j, 2 * j + 1), M[j], M[j + 16], P[j], P[j + 16], S[j], S[16 + j], SP[j], SP[16 + j]);
-        // B: stride 2.  even pair j: k = 4j + 2b ; odd pair j: k = 4j + 2b + 1 -> Q[4j + o] = {8j + o, 8j + 4 + o}
-        branch((int)(int8_t)((w0 >> 16) & 0xffu), (int)(int8_t)(w0 >> 24), Tlo, Thi);
+        for (int s = 0; s < 4; ++s) {
+            const uint32_t h = (s < 2 ? w0 : w1) >> (16 * (s & 1));
+            const int q0 = (int8_t)h, q1 = (int8_t)(h >> 8);
+            // t[p]: branch value of expected pair p = 2A + B, << 16; that of 3 - p is y.  tb: the same + the decision bit
+            uint32_t t[4], tb[4];
+            t[3] = (uint32_t)(q0 + q1 + 254) << 16;
+            t[2] = (uint32_t)(q0 - q1 + 254) << 16;
+            t[1] = (508u << 16) - t[2];
+            t[0] = (508u << 16) - t[3];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            bfly<B1>(Tlo, Thi, vit_sel2(4 * j, 4 * j + 2), S[j], S[j + 8], SP[j], SP[j + 8], Q[4 * j], Q[4 * j + 1], QP[4 * j], QP[4 * j + 1]);
-            bfly<B1>(Tlo, Thi, vit_sel2(4 * j + 1, 4 * j + 3), S[16 + j], S[24 + j], SP[16 + j], SP[24 + j], Q[4 * j + 2], Q[4 * j + 3], QP[4 * j + 2], QP[4 * j + 3]);
-        }
-        // C: stride 4.  pair (j, o): k = 8j + 4b + o -> S[8j + o'] = {16j + o', 16j + 8 + o'}, o' = 2o, 2o+1
-        branch((int)(int8_t)(w1 & 0xffu), (int)(int8_t)((w1 >> 8) & 0xffu), Tlo, Thi);
+            for (int p = 0; p < 4; ++p) tb[p] = t[p] + (1u << (S0 + s));
+            uint32_t N[64];
 #pragma unroll
-        for (int j = 0; j < 4; ++j)
-#pragma unroll
-            for (int o = 0; o < 4; ++o)
-                bfly<B2>(Tlo, Thi, vit_sel2(8 * j + o, 8 * j + 4 + o), Q[4 * j + o], Q[4 * (j + 4) + o], QP[4 * j + o], QP[4 * (j + 4) + o],
-                     S[8 * j + 2 * o], S[8 * j + 2 * o + 1], SP[8 * j + 2 * o], SP[8 * j + 2 * o + 1]);
-        // D: stride 8.  pair (j, o'): k = 16j + 8b + o' -> Q[16j + o''] = {32j + o'', 32j + 16 + o''}, o'' = 2o', 2o'+1
-        branch((int)(int8_t)((w1 >> 16) & 0xffu), (int)(int8_t)(w1 >> 24), Tlo, Thi);
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int o = 0; o < 8; ++o)
-                bfly<B3>(Tlo, Thi, vit_sel2(16 * j + o, 16 * j + 8 + o), S[8 * j + o], S[8 * (j + 2) + o], SP[8 * j + o], SP[8 * (j + 2) + o],
-                     Q[16 * j + 2 * o], Q[16 * j + 2 * o + 1], QP[16 * j + 2 * o], QP[16 * j + 2 * o + 1]);
-        // stride 16 -> natural: natural word w = {2w, 2w+1}; Q[16j + e], Q[16j + e + 1] (e even) hold them in the same lane
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int e = 0; e < 16; e += 2) {
-                M[(32 * j + e) >> 1] = prmt(Q[16 * j + e], Q[16 * j + e + 1], 0x5410u);
-                M[(32 * j + 16 + e) >> 1] = prmt(Q[16 * j + e], Q[16 * j + e + 1], 0x7632u);
-                P[(32 * j + e) >> 1] = prmt(QP[16 * j + e], QP[16 * j + e + 1], 0x5410u);
-                P[(32 * j + 16 + e) >> 1] = prmt(QP[16 * j + e], QP[16 * j + e + 1], 0x7632u);
+            for (int k = 0; k < 32; ++k) {
+                const int p = 2 * vit_par((2 * k) & 0x6d) + vit_par((2 * k) & 0x4f);
+                N[2 * k] = __viaddmax_u32(X[k], t[p], VitCoreH::fadd(X[k + 32], tb[3 - p]));
+                N[2 * k + 1] = __viaddmax_u32(X[k], t[3 - p], VitCoreH::fadd(X[k + 32], tb[p]));
             }
+#pragma unroll
+            for (int i = 0; i < 64; ++i) X[i] = N[i];
+        }
     }
-    // snapshot + first best state (index-carrying tournament over adjacent words) + optional renormalisation
-    __device__ __forceinline__ VitTrace trace_begin(uint32_t *ring, int slot, int ntb, int tid, bool renorm)
+    // end of a chunk: as VitCoreH::trace_begin (same arguments and cursor), the path bytes cleared by a mask
+    __device__ __forceinline__ uint32_t trace_begin(uint8_t *snap, uint32_t c0_base, const uint32_t *hop_tab, bool renorm,
+                                                    uint32_t keep = 0xffu)
     {
+        // keys (metric << 16) | (63 - state): the largest key is the largest metric at the smallest state
+        uint32_t key[64];
 #pragma unroll
-        for (int w = 0; w < 16; ++w) ring[(slot * 16 + w) * VIT_BLOCK + tid] = prmt(P[2 * w], P[2 * w + 1], 0x6420u);
-        uint32_t tv[16], ti[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const uint32_t a = M[2 * i], b = M[2 * i + 1];
-            const uint32_t k = prmt((a | 0x80008000u) - b, 0u, 0xbb99u);          // 0xffff where a >= b
-            tv[i] = (a & k) | (b & ~k);
-            ti[i] = ((uint32_t)(2 * i) * 0x00010001u & k) | ((uint32_t)(2 * i + 1) * 0x00010001u & ~k);
+        for (int x = 0; x < 64; ++x) {
+            snap[vit_h_off(x)] = (uint8_t)(X[x] & keep);
+            X[x] &= 0xffff0000u;
+            key[x] = VitCoreH::fadd(X[x], 63u - x);
         }
 #pragma unroll
-        for (int n = 8; n >= 1; n >>= 1)
+        for (int n = 32; n >= 1; n >>= 1)
 #pragma unroll
-            for (int i = 0; i < n; ++i) {
-                const uint32_t a = tv[2 * i], b = tv[2 * i + 1];
-                const uint32_t k = prmt((a | 0x80008000u) - b, 0u, 0xbb99u);
-                tv[i] = (a & k) | (b & ~k);
-                ti[i] = (ti[2 * i] & k) | (ti[2 * i + 1] & ~k);
-            }
-        const int v0 = (int)(tv[0] & 0xffffu), s0 = (int)(ti[0] & 0xffffu) * 2;
-        const int v1 = (int)(tv[0] >> 16), s1 = (int)(ti[0] >> 16) * 2 + 1;
-        VitTrace t;
-        t.bs = (v1 > v0 || (v1 == v0 && s1 < s0)) ? s1 : s0;
-        t.sl = slot;
-        t.left = ntb - 1;
+            for (int i = 0; i < n; ++i) key[i] = max(key[i], key[i + n]);
+        const uint32_t c = c0_base + hop_tab[256 + (key[0] & 0xffffu)];
         if (renorm) {
-            uint32_t mn = M[0];
+            // only metric differences matter: subtracting max - VIT_S_SPREAD keeps every metric non-negative
+            const uint32_t mx = key[0] >> 16;
+            const uint32_t nmin = 0u - (mx > VIT_S_SPREAD ? (mx - VIT_S_SPREAD) << 16 : 0u);
 #pragma unroll
-            for (int i = 1; i < 32; ++i) mn = vmin2(mn, M[i]);
-            mn = vmin2(mn, mn >> 16);
-            const uint32_t minw = (mn & 0xffffu) * 0x00010001u;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) M[i] -= minw;
+            for (int x = 0; x < 64; ++x) X[x] = VitCoreH::fadd(X[x], nmin);
         }
-#pragma unroll
-        for (int i = 0; i < 32; ++i) P[i] = 0;
-        return t;
-    }
-    static __device__ __forceinline__ uint32_t vmin2(uint32_t a, uint32_t b)
-    {
-        uint32_t k = prmt((a | 0x80008000u) - b, 0u, 0xbb99u);
-        return (b & k) | (a & ~k);
-    }
-    // ring bytes hold the decisions MSB first (upstream's order): the state eight steps back is the byte >> 2
-    template <int N>
-    static __device__ __forceinline__ void trace_hops(VitTrace &t, const uint32_t *ring, int ntb, int tid)
-    {
-#pragma unroll
-        for (int i = 0; i < N; ++i) {
-            const bool go = t.left > 0;
-            const int nb = (int)(vit_ring_byte(ring, t.sl, t.bs, tid) >> 2);
-            const int ns = (t.sl == 0) ? ntb - 1 : t.sl - 1;
-            t.bs = go ? nb : t.bs;
-            t.sl = go ? ns : t.sl;
-            t.left -= go ? 1 : 0;
-        }
+        return c;
     }
 };

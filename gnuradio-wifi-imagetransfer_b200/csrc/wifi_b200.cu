@@ -161,9 +161,6 @@ const char *STAGE_NAMES[ST_COUNT] = {"h2d", "detect", "select", "sync_long", "de
 #endif
 #define VQ_SPLIT_MAX 4736        // frames beyond a step of the per-thread kernel's staircase that get their own launch (run_rx)
 #define DET_SMEM DET_SMEM_BYTES
-// k_viterbi: ring, CRC table, descrambler table, branch-word table (8 x 4 x 16 entries of 16 bytes), traceback rows
-// (24 x 48 bytes), hop table (320 words): 52864 bytes, 4 blocks per SM
-#define VIT_SMEM_BYTES ((VIT_NTB_MAX * 16 * VIT_BLOCK + 256) * 4 + 256 + 8192 + VIT_ROWS * 48 + VIT_HOP_ENTRIES * 4)
 
 } // namespace
 
@@ -554,8 +551,7 @@ int run_rx(wifi_b200 *h, const cf *iq, bool mirror, const H2dPlan *plan = nullpt
     static const demod_fn demod_tab[2][2][4] = {{DEMOD_ROW(false, 0), DEMOD_ROW(false, 1)}, {DEMOD_ROW(true, 0), DEMOD_ROW(true, 1)}};
 #undef DEMOD_ROW
     const demod_fn demod_head = demod_tab[soft][0][prm.algo & 3], demod_data = demod_tab[soft][1][prm.algo & 3];
-    const size_t vit_smem_soft = (size_t)(VIT_NTB_MAX * 16 * VIT_BLOCK + 256) * 4 + 256 + 256;   // ring, CRC table, descrambler table, branch words
-    const size_t vit_smem = (size_t)VIT_SMEM_BYTES;
+    const size_t vit_smem = (size_t)vit_smem_bytes<VitHardIn>(), vit_smem_soft = (size_t)vit_smem_bytes<VitSoftIn>();
     const bool timed = n_groups == 1;              // per-stage events only make sense for a single pass
     int64_t frame_base = 0, row_base = 0, tile_base = 0;
     for (int g = 0; g < n_groups; ++g) {
@@ -821,7 +817,7 @@ int wifi_b200_create(const wifi_b200_cfg *cfg_in, wifi_b200_t **out)
     for (int i = 0; i <= ST_COUNT; ++i) if (cudaEventCreate(&h->ev[i]) != cudaSuccess) return fail(WIFI_E_CUDA);
     if (upload_tables(h) != WIFI_OK) return fail(WIFI_E_CUDA);
     if (cudaFuncSetAttribute(k_detect, cudaFuncAttributeMaxDynamicSharedMemorySize, DET_SMEM) != cudaSuccess) return fail(WIFI_E_CUDA);
-    if (VIT_SMEM_BYTES > 48 * 1024 && cudaFuncSetAttribute(k_viterbi, cudaFuncAttributeMaxDynamicSharedMemorySize, VIT_SMEM_BYTES) != cudaSuccess) return fail(WIFI_E_CUDA);
+    if (vit_smem_bytes<VitHardIn>() > 48 * 1024 && cudaFuncSetAttribute(k_viterbi, cudaFuncAttributeMaxDynamicSharedMemorySize, vit_smem_bytes<VitHardIn>()) != cudaSuccess) return fail(WIFI_E_CUDA);
     {
         // CUDA loads a kernel on its first launch (milliseconds): do it here, not inside the first live run
         const void *kernels[] = {(const void *)k_detect, (const void *)k_select_spec, (const void *)k_select_fix, (const void *)k_select, (const void *)k_reserve,
