@@ -53,6 +53,20 @@ __device__ __forceinline__ int find_link(const LinkDesc *links, int n_links, int
 #define DET_SMEM_BYTES (DET_ROWS * DET_STRIDE * (int)sizeof(cf) + 32)   // + one mbarrier per warp
 
 __device__ __forceinline__ uint32_t det_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// bit 0 / bit 1: the first / second sample of the pair at p (shared memory) is not an exact zero (-0 is a zero, NaN is not).
+// Volatile loads, here and below: the compiler must not keep the walk's samples alive in registers to reuse them here.
+__device__ __forceinline__ uint32_t det_nonzero_pair(const cf *p)
+{
+    uint32_t a, b, c, d;
+    asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(a), "=r"(b), "=r"(c), "=r"(d) : "r"(det_smem_u32(p)));
+    return (((a | b) << 1) != 0u ? 1u : 0u) | (((c | d) << 1) != 0u ? 2u : 0u);
+}
+__device__ __forceinline__ bool det_nonzero_one(const cf *p)
+{
+    uint32_t a, b;
+    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(a), "=r"(b) : "r"(det_smem_u32(p)));
+    return ((a | b) << 1) != 0u;
+}
 
 __global__ void __launch_bounds__(DET_BLOCK, 384 / DET_BLOCK) k_detect(const cf *__restrict__ iq, const LinkDesc *__restrict__ links, int n_links,
                                                          int64_t tile_base, int64_t total_tiles, float thr_f, uint32_t *__restrict__ flags,
@@ -146,6 +160,23 @@ __global__ void __launch_bounds__(DET_BLOCK, 384 / DET_BLOCK) k_detect(const cf 
                 if (n < 32) w0 |= 1u << n; else w1 |= 1u << (n - 32);
             }
             ring[n] = xn;                            // replaces sample n - 64
+        }
+        // silence is silence (oracle FrontEnd): no flag where the 64-sample window n-63 .. n holds only exact zeros (the
+        // running sums may keep a rounding residue there).  If the first flagged sample is nonzero, every flagged window
+        // holds it or a later own sample: one load settles the chunk.  Otherwise, bit k of nzh / nzo: sample k - 64 /
+        // sample k is nonzero; the window holds one iff n is at or after the first nonzero own sample, or before the last
+        // nonzero history sample (k in 1 .. 63, k > n).
+        if ((w0 | w1) != 0u && !det_nonzero_one(sx + (tid + 2) * DET_STRIDE + (w0 ? __ffs((int)w0) - 1 : 31 + __ffs((int)w1)))) {
+            uint64_t nzh = 0ull, nzo = 0ull;
+#pragma unroll 8
+            for (int m = 0; m < 32; ++m) {
+                nzh |= (uint64_t)det_nonzero_pair(sx + (tid + 1) * DET_STRIDE + 2 * m) << (2 * m);
+                nzo |= (uint64_t)det_nonzero_pair(sx + (tid + 2) * DET_STRIDE + 2 * m) << (2 * m);
+            }
+            nzh &= ~1ull;                            // sample -64 is outside every window of the chunk
+            const uint64_t occ = (0ull - (nzo & (0ull - nzo))) | (nzh ? (~0ull >> __clzll((long long)nzh)) >> 1 : 0ull);
+            w0 &= (uint32_t)occ;
+            w1 &= (uint32_t)(occ >> 32);
         }
     }
     const int64_t chunk = tile * DET_THREADS + half * DET_BLOCK + tid;

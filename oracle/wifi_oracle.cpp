@@ -584,22 +584,29 @@ struct FrontEnd {
     int64_t hist = 0; /* valid samples stored before x[0] (a stream resumed in the middle); older ones read as 0 */
     cf sa = {0.f, 0.f};
     float sp = 0;
+    int nz = 0;       /* exact count of the nonzero samples among the last 63 (the p window without the newest) */
     /* samples before the start of the stream are zeros (GNU Radio history) */
     inline cf at(int64_t j) const { return j < -hist ? cf{0.f, 0.f} : x[j]; }
+    static inline int nonzero(cf v) { return v.re != 0.f || v.im != 0.f; }
     void seed(int64_t i0)
     {
         sa = {0.f, 0.f};
         sp = 0.f;
+        nz = 0;
         if (i0 >= 64) {
             for (int64_t j = i0 - 47; j < i0; ++j) sa = wdm_cmacc(sa, x[j], x[j - 16]);
             for (int64_t j = i0 - 63; j < i0; ++j) sp = wdm_norm_add(sp, x[j]);
+            for (int64_t j = i0 - 63; j < i0; ++j) nz += nonzero(x[j]);
             return;
         }
         for (int64_t j = i0 - 47; j < i0; ++j) sa = wdm_cmacc(sa, at(j), at(j - 16));
         for (int64_t j = i0 - 63; j < i0; ++j) sp = wdm_norm_add(sp, at(j));
+        for (int64_t j = i0 - 63; j < i0; ++j) nz += nonzero(at(j));
     }
     /* running sums as fused multiply-add chains: a[i] = sum of x[j] conj(x[j-16]) over the last 48 lags, p[i] = sum of
-     * |x[j]|^2 over the last 64 samples; the term leaving the window is subtracted after the output is taken */
+     * |x[j]|^2 over the last 64 samples; the term leaving the window is subtracted after the output is taken.
+     * Silence is silence (DESIGN.md, choice 7): where all 64 samples of the p window are exact zeros, a[i] and p[i] are
+     * exactly 0 (the 48 lags of a lie inside that window), whatever rounding residue the running sums still hold. */
     float m2 = 0; /* |a[i]|^2 of the last step */
     inline void step(int64_t i, cf &a, float &p, float &c)
     {
@@ -611,6 +618,9 @@ struct FrontEnd {
             sp = wdm_norm_add(sp, x[i]);
             p = sp;
             sp = wdm_norm_sub(sp, x[i - 63]);
+            nz += nonzero(x[i]);
+            if (nz == 0) { a = {0.f, 0.f}; p = 0.f; }
+            nz -= nonzero(x[i - 63]);
         } else {
             sa = wdm_cmacc(sa, at(i), at(i - 16));
             a = sa;
@@ -618,6 +628,9 @@ struct FrontEnd {
             sp = wdm_norm_add(sp, at(i));
             p = sp;
             sp = wdm_norm_sub(sp, at(i - 63));
+            nz += nonzero(at(i));
+            if (nz == 0) { a = {0.f, 0.f}; p = 0.f; }
+            nz -= nonzero(at(i - 63));
         }
         m2 = wdm_norm(a);
         c = sqrtf(m2) / p;
@@ -799,7 +812,7 @@ static void rx_link(const cf *x, int64_t n, int link, const orc_rx_cfg &cfg, Res
         /* sync_short compares c = |a| / p with the threshold; the contract compares the squares,
          * |a|^2 > thr^2 p^2 with thr the largest float not above the threshold: the same test up to one rounding of c
          * (threshold jitter of a few 1e-8 relative), no square root and no division per sample (DESIGN.md, choice 7).
-         * p = 0 (silence) and NaN give "not over", as c = 0/0 does upstream. */
+         * p = 0 and NaN give "not over", as c = 0/0 does upstream; a window of exact zeros has a = p = 0 (FrontEnd). */
         float thr_f = (float)cfg.threshold;
         if ((double)thr_f > cfg.threshold) thr_f = nextafterf(thr_f, -INFINITY);
         const float thr2 = thr_f * thr_f;

@@ -236,3 +236,263 @@ def rx_frame(samples, frame_start, enc=None):
             break
     plain = bits ^ scrambler_seq(seed, bits.size)
     return enc_, length, np.packbits(plain[16:16 + 8 * length], bitorder="little").tobytes()
+
+
+# ---------------------------------------------------------------- receiver stages in float64
+# The receive chain of wifi_phy_hier (gr-ieee802-11's sync_short, sync_long and frame_equalizer, as SURVEY.md 8a and
+# Appendix A restate them), computed in float64 from the formulas: exact window sums, numpy's FFT, exp() rotations,
+# each upstream rotation applied on its own.  Every stage takes its inputs explicitly, so a test can feed it either
+# the previous model stage or what the device under test reported.
+SS_MIN_GAP, SS_MAX_SAMPLES, SYNC_LENGTH = 480, 540 * 80, 320
+LEVEL = {1: np.sqrt(0.5), 2: np.sqrt(0.1), 3: np.sqrt(1 / 42)}       # per-axis unit of QPSK / 16-QAM / 64-QAM
+USED = np.array([i for i in range(6, 59) if i != 32])                  # the 52 used carriers, shifted order (index = k + 32)
+PILOT_IDX = np.array([11, 25, 39, 53])
+DATA_IDX = np.array([i for i in USED if i not in PILOT_IDX])
+
+
+def lts_shifted():
+    L = np.zeros(64)
+    L[6:59] = LTS
+    return L
+
+
+def long_taps():
+    """sync_long's matched filter LONG[63 - n] = conj(lts_t[n]) rounded to 4 decimals, lts_t the LTS time symbol."""
+    L = np.zeros(64, complex)
+    for i, k in enumerate(range(-26, 27)):
+        L[k % 64] = LTS[i]
+    lt = time_symbol(L)
+    return np.round(np.conj(lt[::-1]).real, 4) + 1j * np.round(np.conj(lt[::-1]).imag, 4)
+
+
+def constellation(enc):
+    """Point of every carrier index v (bit k of v = coded bit b_k, b_0 first on air)."""
+    nb = N_BPSC[enc]
+    return map_bits([(v >> k) & 1 for v in range(1 << nb) for k in range(nb)], enc)
+
+
+def frontend(x, thr=0.56):
+    """Exact window sums of the autocorrelation front end; samples before index 0 are zeros.
+    a[i] = sum of x[j] conj(x[j-16]) over j = i-47 .. i, p[i] = sum of |x[j]|^2 over j = i-63 .. i.
+    Returns (a, p, flags, margin, E): flags = p > 0 and |a| > thr p, margin = ||a| - thr p|, E[i] = sum of |x|^2 over the
+    last 128 samples (the scale of the margin)."""
+    from numpy.lib.stride_tricks import sliding_window_view as win
+    x = np.asarray(x, np.complex128)
+    n = x.size
+    xz = np.concatenate([np.zeros(127, complex), x])
+    pw = xz.real ** 2 + xz.imag ** 2
+    prod = np.zeros(xz.size, complex)
+    prod[16:] = xz[16:] * np.conj(xz[:-16])
+    a = win(prod[80:], 48).sum(axis=1)[:n]
+    p = win(pw[64:], 64).sum(axis=1)[:n]
+    cs = np.concatenate([[0.0], np.cumsum(pw)])
+    E = np.maximum(cs[128:128 + n] - cs[:n], 0.0)
+    flags = (p > 0) & (np.abs(a) > thr * p)
+    return a, p, flags, np.abs(np.abs(a) - thr * p), E
+
+
+def sync_short(flags, a, n=None, min_plateau=2, min_pos=0):
+    """sync_short's SEARCH / COPY state machine on a flag array (the port of its per-sample loop, stepped from flag to
+    flag: an unflagged sample only resets the plateau counter).  Returns (triggers, burst_len, freq_short) with
+    freq_short = angle(a[t]) / 16."""
+    n = len(flags) if n is None else n
+    trig = []
+    search, plateau, c0, last = True, 0, 0, -2
+    for i in np.flatnonzero(flags):
+        i = int(i)
+        if i != last + 1:
+            plateau = 0
+        last = i
+        if not search and i >= c0 + SS_MAX_SAMPLES:
+            search = True                     # the copy ended on sample c0 + MAX_SAMPLES - 1
+        if search:
+            if plateau < min_plateau:
+                plateau += 1
+                continue
+            if i < min_pos:
+                continue
+            search, plateau, c0 = False, 0, i
+            trig.append(i)                    # falls through to COPY with the same sample
+        if plateau < min_plateau:
+            plateau += 1
+        elif i - c0 > SS_MIN_GAP:
+            trig.append(i)
+            c0, plateau = i, 1
+    t = np.array(trig, np.int64)
+    nxt = np.concatenate([t[1:], [n]])
+    blen = np.minimum(np.minimum(nxt, t + SS_MAX_SAMPLES), n) - t
+    fs = np.angle(a[t]) / 16 if t.size else np.zeros(0)
+    return t, blen, fs
+
+
+def _burst(x, t, j, hist=0):
+    src = t + np.asarray(j) - 16
+    ok = src >= -hist
+    out = np.zeros(src.shape, complex)
+    out[ok] = np.asarray(x, np.complex128)[src[ok] + hist]
+    return out
+
+
+def sync_long(x, t, burst_len, freq_short, fo_carry=0.0, hist=0, taps=None):
+    """The LTS matched filter over 320 lags of sync_short's derotated burst, the top four |corr|^2 (stable order) and the
+    63/64/65 pair rule preferring 64.  x[hist] is the stream's sample 0.  Returns a dict: frame_start, found, freq_long
+    (fo_carry where no pair is found: sync_long keeps its offset across bursts), tie (relative gap between the fourth and
+    fifth largest magnitudes, and between equal-rank neighbours: a tie below 1e-6 makes the ranking fragile)."""
+    r = {"frame_start": SYNC_LENGTH, "found": 0, "freq_long": float(fo_carry), "tie": np.inf}
+    if burst_len < SYNC_LENGTH + 63:
+        return r
+    taps = long_taps() if taps is None else taps
+    j = np.arange(SYNC_LENGTH + 63)
+    b = _burst(x, t, j, hist) * np.exp(-1j * float(freq_short) * j)
+    from numpy.lib.stride_tricks import sliding_window_view as win
+    corr = win(b, 64)[:SYNC_LENGTH] @ taps[::-1]          # corr[i] = sum_m LONG[63 - m] b[i + m]
+    mag = np.abs(corr) ** 2
+    order = np.argsort(-mag, kind="stable")
+    top = order[:4]
+    srt = mag[order[:5]]
+    r["tie"] = float(np.min(np.abs(np.diff(srt)) / srt[0])) if srt[0] > 0 else 0.0
+    done = False
+    for i in range(3):
+        if done:
+            break
+        for k in range(i + 1, 4):
+            lo, hi = min(top[i], top[k]), max(top[i], top[k])
+            d = hi - lo
+            if d in (63, 64, 65):
+                r.update(frame_start=int(lo), found=int(d), freq_long=float(np.angle(corr[lo] * np.conj(corr[hi])) / d))
+                if d == 64:
+                    done = True
+                    break
+    return r
+
+
+def symbols(x, t, burst_len, freq_short, freq_long, frame_start, n_syms, hist=0, final=True, last=False):
+    """sync_long's COPY output cut into 64-sample symbols (CP dropped): LTS1, LTS2, SIGNAL, data ...  Each sample gets
+    sync_short's exp(-j fs j) and sync_long's exp(+j fl j), j its burst position; a partial symbol is zero-padded."""
+    avail = burst_len - SYNC_LENGTH
+    R = avail - frame_start
+    E = 0 if R <= 0 else (R if R <= 128 else 128 + 64 * ((R - 128) // 80) + max(0, ((R - 128) % 80) - 16))
+    k = np.arange(n_syms * 64)
+    nn, m = k // 64, k % 64
+    j = frame_start + np.where(nn < 2, 64 * nn + m, 128 + 80 * (nn - 2) + 16 + m)
+    s = _burst(x, t, j, hist) * np.exp(-1j * float(freq_short) * j) * np.exp(1j * float(freq_long) * j)
+    s[k >= E] = 0
+    return s.reshape(n_syms, 64)
+
+
+def decide_nearest(enc, z):
+    """Index of the nearest constellation point of every z, and its distance to the closest decision boundary."""
+    z = np.asarray(z, complex)
+    pts = constellation(enc)
+    idx = np.argmin(np.abs(z[..., None] - pts), axis=-1)
+    h = N_BPSC[enc] // 2
+    if N_BPSC[enc] == 1:
+        return idx, np.abs(z.real)
+    lv = LEVEL[h]
+    bnd = lv * np.arange(-(2 ** h) + 2, 2 ** h - 1, 2)     # midpoints between adjacent levels
+    dist = np.minimum(np.abs(z.real[..., None] - bnd).min(-1), np.abs(z.imag[..., None] - bnd).min(-1))
+    return idx, dist
+
+
+def llr(enc, z):
+    """Max-log LLR per coded bit in units of the axis level (positive = bit 1), 48 * N_BPSC values per symbol in the
+    order of the carrier index bits."""
+    nb = N_BPSC[enc]
+    if nb == 1:
+        return z.real[:, None]
+    h = nb // 2
+    out = []
+    for a in (z.real / LEVEL[h], z.imag / LEVEL[h]):
+        m = np.abs(a)
+        out.append(a)
+        if h == 2:
+            out.append(2 - m)
+        if h == 3:
+            out += [4 - m, 2 - np.abs(m - 4)]
+    return np.stack(out, axis=-1)
+
+
+def equalize(sy, enc, algo, freq_short, freq_long, rows=None, bw=10e6, freq=5.89e9):
+    """frame_equalizer on the symbols of one frame (sy: LTS1, LTS2, SIGNAL, data ...): FFT and +-32 shift, the
+    sampling-offset ramp 2 pi n 80 (eps0 + d_er)(i - 32) / 64 with eps0 from the frequency offset sync_long tagged,
+    the pilot phase beta, the pilot phase-drift term er through the 0.1 IIR, then LS / LMS / COMB / STA.
+    rows: the data decisions (carrier indices) the decision-directed updates use, one row per data symbol; None = the
+    model's own nearest points.  SIGNAL is decided by the model (BPSK).
+    Returns dict: snr (dB, from the LTS pair), points (n_data x 48), w (soft weight per data carrier), soft (16 l w)."""
+    n_syms = sy.shape[0]
+    pol = PILOT_POLARITY.astype(float)
+    lts = lts_shifted()
+    eps0 = (float(freq_short) - float(freq_long)) * bw / (2 * np.pi * freq)
+    d_er, prev = 0.0, None
+    H = np.zeros(64, complex)
+    snr, w0 = np.nan, np.ones(64)
+    pts, soft = [], []
+    ph_i = np.arange(64) - 32
+    for nn in range(n_syms):
+        cur = np.fft.fft(sy[nn])[(np.arange(64) + 32) & 63]
+        cur = cur * np.exp(1j * 2 * np.pi * nn * 80 * (eps0 + d_er) * ph_i / 64)
+        if nn < 2:
+            pil = cur[PILOT_IDX] * np.array([1, -1, 1, 1])
+        else:
+            p = pol[(nn - 2) % 127]
+            pil = cur[PILOT_IDX] * np.array([p, p, p, -p])
+        beta = np.angle(pil.sum())
+        er = 0.0
+        if nn >= 2:
+            er = np.angle(np.sum(pil * np.conj(prev))) * bw / (2 * np.pi * freq * 80)
+        prev = pil
+        cur = cur * np.exp(-1j * beta)
+        if nn >= 2:
+            d_er = 0.9 * d_er + 0.1 * er
+        e = 0 if nn == 2 else enc
+        if algo == 2:                                       # comb: divide by the pilot-interpolated gain first
+            if nn < 2:
+                cp = cur[PILOT_IDX] * np.array([1, -1, 1, 1])
+            else:
+                p = pol[(nn - 2) % 127]
+                cp = cur[PILOT_IDX] * np.array([p, p, p, -p])
+            knots_x = [0, 11, 25, 39, 53, 64]
+            knots_y = [cp.mean(), cp[0], cp[1], cp[2], cp[3], cp.mean()]
+            G = np.zeros(64, complex)
+            for s in range(5):
+                x0, x1 = knots_x[s], knots_x[s + 1]
+                i = np.arange(x0 + (s > 0), x1 + 1) if s < 4 else np.arange(54, 64)
+                G[i] = (knots_y[s] * (x1 - i) + knots_y[s + 1] * (i - x0)) / (x1 - x0)
+            cur = cur / G
+        if nn == 0:
+            H = cur.copy()
+            continue
+        if nn == 1:
+            d, s = H[USED] - cur[USED], H[USED] + cur[USED]
+            snr = 10 * np.log10(np.sum(np.abs(s) ** 2) / np.sum(np.abs(d) ** 2) / 2)
+            H = H.copy()
+            H[USED] = s / (2 * lts[USED])
+            w0 = np.abs(H) ** 2 / np.mean(np.abs(H[USED]) ** 2)
+            continue
+        z = cur[DATA_IDX] / H[DATA_IDX]
+        if nn == 2 or rows is None:
+            dec = decide_nearest(e, z)[0]
+        else:
+            dec = np.asarray(rows[nn - 3], int)
+        if nn > 2:
+            pts.append(z)
+            soft.append(16 * llr(e, z) * w0[DATA_IDX][:, None])
+        q = cur[DATA_IDX] / constellation(e)[dec]
+        if algo == 1:                                       # lms, alpha 0.5
+            H[DATA_IDX] = 0.5 * H[DATA_IDX] + 0.5 * q
+        elif algo == 3:                                     # sta, alpha 0.5, beta 2
+            p = pol[(nn - 2) % 127]
+            Hu = np.zeros(64, complex)
+            Hu[DATA_IDX] = q
+            Hu[PILOT_IDX] = cur[PILOT_IDX] * np.array([p, p, p, -p])
+            used = np.zeros(64, bool)
+            used[USED] = True
+            Hn = H.copy()
+            for i in USED:
+                k = np.arange(i - 2, i + 3)
+                k = k[used[k]]
+                Hn[i] = 0.5 * H[i] + 0.5 * Hu[k].mean()
+            H = Hn
+    nd = len(pts)
+    return {"snr": snr, "points": np.array(pts).reshape(nd, 48), "w": w0[DATA_IDX],
+            "soft": np.array(soft).reshape(nd, 48 * N_BPSC[enc]) if nd else np.zeros((0, 48 * N_BPSC[enc]))}

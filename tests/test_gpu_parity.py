@@ -1008,14 +1008,14 @@ def test_ota_runners_record_and_replay(O, W, fmt, tmp_path):
     path.write_bytes(raw)
     a = W.ota_runners.IrsAp(("127.0.0.1", out.getsockname()[1]), chan_est=0, fmt=fmt, chunk=20000)
     st = a.run(str(path))
-    # what the reference receiver makes of this recording (sync_short re-triggers inside one of the noise-free
-    # frames and truncates it, in the oracle as on the GPU): the replay forwards exactly the oracle's PDUs
+    # the zeros between the noise-free frames are silence (no trigger in them cuts a frame short, DESIGN.md choice 7):
+    # the replay forwards exactly the oracle's PDUs, every payload once
     played = want if fmt == "fc32" else (q.astype(np.float32) * np.float32(1.0 / 16384.0)).view(np.complex64)
     ref = O.rx(played, algo=0)
-    assert st["samples_in"] == want.size and st["pdus_out"] == len(ref.pdus()) >= 6
+    assert st["samples_in"] == want.size and st["pdus_out"] == len(ref.pdus()) == 7
     got = [out.recvfrom(4096)[0] for _ in range(st["pdus_out"])]
     assert got == [p[24:][4:] for p in ref.pdus()]                   # "Extract Pics" strips the MAC header and 4 more bytes
-    assert set(got) <= {p[4:] for p in payloads}
+    assert got == [p[4:] for p in payloads]
     a.close()
 
 
